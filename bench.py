@@ -2,7 +2,7 @@
 """Benchmark of the EIP-4844 hot path (BASELINE.json metric: blobs/sec commit+proof at 1/2/4/8 B200; G1 MSM
 points/sec vs CPU reference).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One step = one pass of the hot path over one batch: for each of 1024 synthetic blobs per GPU (SURVEY §8d generator),
 commitment = blob_to_kzg_commitment(blob) and proof = compute_blob_kzg_proof(blob, commitment), through the library's
@@ -28,6 +28,9 @@ The JSON line (rank 0):
 
 --impl reference times that CPU restatement alone (the reference's own Rust code cannot be built here: no cargo,
 un-vendored git dependencies); it never loads the product library.
+
+--dump-outputs DIR writes what the last timed step returned to its caller -- commitments, proofs and status words --
+as DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for output on the same inputs.
 """
 import argparse
 import ctypes
@@ -55,6 +58,7 @@ CELL_BLOBS = 888          # PeerDAS block: blobs per compute_cells_and_kzg_proof
 # dram__bytes_read.sum + dram__bytes_write.sum of ONE 1024-blob launch of msm_gather_ba_kernel from the ncu --set full
 # capture committed as profiles/r02_ncu_ba_1024blob_end_of_round_raw.csv
 NCU_DRAM_BYTES_PER_BLOB = (35.41e9 + 9.30e9) / 1024
+DUMP_LIMIT_BYTES = 64_000_000   # --dump-outputs: all ranks' files together
 
 
 def workload_name(n, wb):
@@ -173,6 +177,25 @@ def var_msm_work_mac32(n):
     return (min((255 // c + 1) * (10 * n + 14 * (1 << c)) for c in range(4, 24)) + 256 * 9) * 300.0
 
 
+def dump_outputs(out_dir, first_blob, coms, proofs, status, ranks=1, suffix=""):
+    """Write one step's outputs of a rank as DIR/<name><suffix>.npy, one row per blob: commitments.npy and proofs.npy
+    (float32, n x 48, the byte values of the compressed G1 points), status.npy (float32, the C_KZG_RET of each blob)
+    and blob_index.npy (float64, the synthetic blob number).  When the files of all ranks would exceed
+    DUMP_LIMIT_BYTES, the same seeded sample of blobs is kept on every run."""
+    import numpy as np
+
+    n = len(status)
+    rows = min(n, (DUMP_LIMIT_BYTES // ranks - 4096) // (4 * (48 + 48 + 1) + 8))   # 4096: room for the four .npy headers
+    keep = np.arange(n) if rows == n else np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+    arrays = {"commitments": np.frombuffer(coms, dtype=np.uint8).reshape(n, 48)[keep].astype(np.float32),
+              "proofs": np.frombuffer(proofs, dtype=np.uint8).reshape(n, 48)[keep].astype(np.float32),
+              "status": np.asarray(status)[keep].astype(np.float32),
+              "blob_index": (first_blob + keep).astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -182,7 +205,12 @@ def main():
     ap.add_argument("--blobs", type=int, default=BLOBS_PER_GPU)
     ap.add_argument("--window-bits", type=int, default=16, help="fixed-base window c (16 -> 100 GiB table, the library default; shrinks automatically if HBM is short)")
     ap.add_argument("--no-extras", action="store_true", help="skip the verify / msm_sweep / latency blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's commitments, proofs and status words to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to --impl native")
     # Exactly ONE line on stdout (the JSON): native libraries (NCCL's version banner, CUDA warnings) write to fd 1
     # behind Python's back, so fd 1 is pointed at stderr for the whole run and the JSON goes to the saved descriptor.
     sys.stdout.flush()
@@ -200,9 +228,8 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps = max(1, min(args.steps, 3))
-        base, dt = cpu_reference_run(steps, args.warmup)
-        line = {"impl": "reference", "metric": METRIC, "value": base["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
+        base, dt = cpu_reference_run(args.steps, args.warmup)
+        line = {"impl": "reference", "metric": METRIC, "value": base["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
                 "warmup": min(args.warmup, 1), "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                 "dtype": "u64 (6x64-bit Montgomery limbs)", "data": "synthetic",
                 "config": {"workload": workload_name(n, args.window_bits) + "; CPU arm: bounded sample per step, see cpu_baseline.sample"},
@@ -270,6 +297,8 @@ def main():
     ms_per_step = max_over_ranks(ms) / args.steps
     value = world * n / (ms_per_step * 1e-3)
     dev_coms, dev_proofs = bytes(coms.cpu().numpy().tobytes()), bytes(proofs.cpu().numpy().tobytes())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank * n, dev_coms, dev_proofs, status.cpu().numpy(), world, "" if world == 1 else "_rank%d" % rank)
 
     # ---- end to end through the host-buffer C ABI call
     def e2e_run(h_blobs, h_coms, h_proofs):
