@@ -1888,7 +1888,11 @@ static C_KZG_RET phase1_impl(uint8_t* tuples_out, bool out_on_device, const Blob
   if (!first_bad_status(c, n_local, bad)) return C_KZG_ERROR;
   if (bad) { set_err("invalid commitment, proof or field element bytes"); return bad_code(bad); }
   if (!c->srs_valid || !c->g2_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
-  if (cudaMemcpy(tuples_out, c->vb_tuples.p, n_local * 160, out_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost) != cudaSuccess) {
+  // on the context's stream and waited for: a plain cudaMemcpy between device buffers may still be running when it
+  // returns, on the legacy stream, which the library's non-blocking streams (phase 2 reads these tuples) do not wait for
+  cudaStream_t s0 = c->slot[0].st;
+  if (cudaMemcpyAsync(tuples_out, c->vb_tuples.p, n_local * 160, out_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s0) != cudaSuccess ||
+      cudaStreamSynchronize(s0) != cudaSuccess) {
     set_err("tuple copy failed");
     return C_KZG_ERROR;
   }

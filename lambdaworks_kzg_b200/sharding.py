@@ -140,10 +140,15 @@ def verify_blob_kzg_proof_batch_distributed_device(blobs_ptr: int, commitments_p
     device = torch.device("cuda", torch.cuda.current_device())
     first, n_local = shard_range(n_total, world, rank)
     n_max = shard_range(n_total, world, 0)[1]   # rank 0 holds a largest shard
+    # The library works on streams of its own that do not order after torch's: every tensor it reads or writes is
+    # finished on torch's stream (allocated, zero-filled, gathered, concatenated) before the call.  A zero-fill that
+    # landed after phase 2 would erase this rank's partial sums and drop its items from the pairing check.
+    sync = torch.cuda.current_stream().synchronize
     mine = torch.zeros(n_max * 160, dtype=torch.uint8, device=device)
     err = 0
     try:
         if n_local:
+            sync()
             api.verify_batch_phase1_device(mine.data_ptr(), blobs_ptr, commitments_ptr, proofs_ptr, n_local, settings, inputs_on_device)
     except api.KzgError as e:
         err = e.code
@@ -153,7 +158,6 @@ def verify_blob_kzg_proof_batch_distributed_device(blobs_ptr: int, commitments_p
         raise api.KzgError(int(flag[0]), "verify_blob_kzg_proof_batch_distributed_device", "invalid item on some rank")
     gathered = torch.empty(world * n_max * 160, dtype=torch.uint8, device=device)
     dist.all_gather_into_tensor(gathered, mine)                       # exchange A
-    torch.cuda.current_stream().synchronize()                         # the library's streams do not order after torch's
     if n_total == world * n_max:
         all_tuples = gathered
     else:                                                             # uneven shards: drop the padding
@@ -161,8 +165,9 @@ def verify_blob_kzg_proof_batch_distributed_device(blobs_ptr: int, commitments_p
         all_tuples = torch.cat(parts)
     partial = torch.zeros(288, dtype=torch.uint8, device=device)
     if n_local:
+        sync()
         api.verify_batch_phase2_device(partial.data_ptr(), all_tuples.data_ptr(), n_total, first, n_local, settings)
     partials = torch.empty(world * 288, dtype=torch.uint8, device=device)
     dist.all_gather_into_tensor(partials, partial)                    # exchange B
-    torch.cuda.current_stream().synchronize()
+    sync()
     return api.verify_batch_phase3_device(partials.data_ptr(), world, settings)
