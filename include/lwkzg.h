@@ -221,7 +221,9 @@ int lwkzg_get_devices(int *ids, int cap);
  * evaluation form and cells 0..63 of its extension are the blob itself; in MODE_REFERENCE a blob is 4096 big-endian
  * coefficients reduced mod r (src/utils.rs:27-41) and all 128 cells are computed.  Field elements inside a Cell use
  * the mode's byte order (big-endian except in MODE_CKZG_LE).  The settings must come from load_trusted_setup[_file]
- * (the Lagrange modes keep the monomial points the loader saw); hand-built Lagrange settings get C_KZG_ERROR. */
+ * (the Lagrange modes keep the monomial points the loader saw); hand-built Lagrange settings get C_KZG_ERROR.
+ * Parity is unpinned: the known answers of these calls (tests/golden/cell_kats.json) come from the repository's own
+ * oracle, not from external c-kzg / consensus-spec vectors. */
 #define FIELD_ELEMENTS_PER_EXT_BLOB (2 * FIELD_ELEMENTS_PER_BLOB)
 #define FIELD_ELEMENTS_PER_CELL 64
 #define BYTES_PER_CELL (FIELD_ELEMENTS_PER_CELL * BYTES_PER_FIELD_ELEMENT)
@@ -246,6 +248,26 @@ C_KZG_RET lwkzg_compute_cells_and_kzg_proofs_batch(Cell *cells, KZGProof *proofs
  * are zeroed; d_status (n ints) may be NULL */
 C_KZG_RET lwkzg_compute_cells_and_kzg_proofs_batch_device(void *d_cells, void *d_proofs, const void *d_blobs, size_t n,
                                                           const KZGSettings *s, void *stream, void *d_status);
+/* additive: recover_cells_and_kzg_proofs over n blobs, each given by num_cells (64..128) of its cells.  cell_indices
+ * and cells are n x num_cells, blob-major; the indices of each blob are strictly ascending and < 128 (blobs may use
+ * different index sets of the same size).  recovered_cells: n x 128 cells or NULL; recovered_proofs: n x 128 proofs or
+ * NULL (not both NULL).  status[n] (may be NULL) gets the code recover_cells_and_kzg_proofs would return for that blob;
+ * a failed blob's output slots are left untouched.  Bytes of good blobs are identical to n single calls.  One call
+ * recovers up to "cell_chunk_blobs" blobs per pass: one block per blob for the recovery proper, then the batched FK20
+ * pipeline of lwkzg_compute_cells_and_kzg_proofs_batch; after lwkzg_set_devices the blobs are sharded over the GPUs.
+ * Whole-call errors: n == 0 returns C_KZG_OK and writes nothing; a NULL required pointer returns C_KZG_BADARGS;
+ * num_cells outside [64, 128] returns C_KZG_BADARGS (C_KZG_ERROR in MODE_REFERENCE); with status == NULL the first
+ * failing blob's code is returned.  Per-blob failures (unsorted, repeated or out-of-range indices, a cell word >= r,
+ * cells that fit no polynomial of degree < 4096) are C_KZG_BADARGS in modes 1 and 2, C_KZG_ERROR in mode 0. */
+C_KZG_RET lwkzg_recover_cells_and_kzg_proofs_batch(Cell *recovered_cells, KZGProof *recovered_proofs,
+                                                   const uint64_t *cell_indices, const Cell *cells, size_t num_cells,
+                                                   size_t n, const KZGSettings *s, int *status);
+/* the same on device buffers (16-byte aligned), ordered after / before work on `stream`, asynchronous; outputs of
+ * failed blobs are zeroed; d_status (n ints, C_KZG_RET values) may be NULL */
+C_KZG_RET lwkzg_recover_cells_and_kzg_proofs_batch_device(void *d_cells_out, void *d_proofs_out,
+                                                          const void *d_cell_indices, const void *d_cells,
+                                                          size_t num_cells, size_t n, const KZGSettings *s,
+                                                          void *stream, void *d_status);
 /* Test hook: intermediate values of the FK20 pipeline for one blob, so a parity test can name the stage that deviates:
  * scalars = the 8192 MSM scalars DFT_128(circulant column b)_j / 128 as 32-byte little-endian integers, at index
  * (j / 64) * 4096 + b * 64 + j % 64 (the order of the two half tables);

@@ -64,6 +64,8 @@ from .api import (  # noqa: F401
     compute_cells_and_kzg_proofs_batch,
     compute_cells_and_kzg_proofs_batch_device,
     recover_cells_and_kzg_proofs,
+    recover_cells_and_kzg_proofs_batch,
+    recover_cells_and_kzg_proofs_batch_device,
     verify_cell_kzg_proof_batch,
     cell_window_bits,
     table_share,

@@ -82,6 +82,8 @@ def load_library() -> ctypes.CDLL:
         "verify_cell_kzg_proof_batch": [bp, vp, vp, vp, vp, sz, sp],
         "lwkzg_compute_cells_and_kzg_proofs_batch": [vp, vp, vp, sz, sp, ip],
         "lwkzg_compute_cells_and_kzg_proofs_batch_device": [vp, vp, vp, sz, sp, vp, vp],
+        "lwkzg_recover_cells_and_kzg_proofs_batch": [vp, vp, vp, vp, sz, sz, sp, ip],
+        "lwkzg_recover_cells_and_kzg_proofs_batch_device": [vp, vp, vp, vp, sz, sz, sp, vp, vp],
         "lwkzg_cell_window_bits": [sp],
         "lwkzg_table_share": [sp],
         "lwkzg_debug_cell_stages": [vp, vp, vp, vp, vp, sp],
@@ -504,6 +506,29 @@ def recover_cells_and_kzg_proofs(cell_indices: Sequence[int], cells: Sequence[by
     cl = [rc.raw[i * BYTES_PER_CELL: (i + 1) * BYTES_PER_CELL] for i in range(CELLS_PER_EXT_BLOB)] if want_cells else []
     pl = [rp.raw[i * 48: (i + 1) * 48] for i in range(CELLS_PER_EXT_BLOB)] if want_proofs else []
     return cl, pl
+
+
+def recover_cells_and_kzg_proofs_batch(cell_indices: Sequence[int], cells: bytes, num_cells: int, n: int, s, want_cells: bool = True,
+                                       want_proofs: bool = True):
+    """n blobs from num_cells cells each (indices and cells n x num_cells, blob-major)
+    -> (cells bytes n x 128 x 2048 or b"", proofs bytes n x 128 x 48 or b"", status list)."""
+    assert len(cell_indices) == n * num_cells and len(cells) == n * num_cells * BYTES_PER_CELL
+    idx = (ctypes.c_uint64 * max(1, n * num_cells))(*cell_indices)
+    rc = ctypes.create_string_buffer(max(1, n * CELLS_PER_EXT_BLOB * BYTES_PER_CELL)) if want_cells else None
+    rp = ctypes.create_string_buffer(max(1, n * CELLS_PER_EXT_BLOB * 48)) if want_proofs else None
+    st = (ctypes.c_int * max(1, n))()
+    _check(load_library().lwkzg_recover_cells_and_kzg_proofs_batch(rc, rp, idx, cells or b"\0", num_cells, n, _sp(s), st),
+           "lwkzg_recover_cells_and_kzg_proofs_batch")
+    return (rc.raw[: n * CELLS_PER_EXT_BLOB * BYTES_PER_CELL] if want_cells else b"", rp.raw[: n * CELLS_PER_EXT_BLOB * 48] if want_proofs else b"",
+            list(st)[:n])
+
+
+def recover_cells_and_kzg_proofs_batch_device(d_cells_out: int, d_proofs_out: int, d_cell_indices: int, d_cells: int, num_cells: int, n: int, s,
+                                              stream: int = 0, d_status: int = 0):
+    """Device-pointer variant: raw device addresses (0 = not wanted), asynchronous with respect to the host."""
+    _check(load_library().lwkzg_recover_cells_and_kzg_proofs_batch_device(d_cells_out or None, d_proofs_out or None, d_cell_indices or None,
+                                                                          d_cells or None, num_cells, n, _sp(s), stream or None, d_status or None),
+           "lwkzg_recover_cells_and_kzg_proofs_batch_device")
 
 
 def verify_cell_kzg_proof_batch(commitments: Sequence[bytes], cell_indices: Sequence[int], cells: Sequence[bytes], proofs: Sequence[bytes], s) -> bool:

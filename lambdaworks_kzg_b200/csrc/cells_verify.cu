@@ -218,7 +218,7 @@ __global__ void __launch_bounds__(128) cell_verify_finish_kernel(uint32_t* __res
 }
 
 // ------------------------------------------------------------------ recovery
-// One block, 512 threads.  Global scratch `ws` holds 3 x 8192 field elements; an 8192-point transform is one
+// One block of 512 threads per blob.  Its global scratch holds 3 x 8192 field elements; an 8192-point transform is one
 // radix-2 pass through global memory plus two 4096-point transforms in shared memory.
 constexpr int REC_THREADS = 512;
 constexpr int REC_SMEM = 4096 * 32;
@@ -239,18 +239,39 @@ __device__ void fft8192(Fr* __restrict__ out, const Fr* __restrict__ in, uint32_
   }
 }
 
+// Block b recovers blob b from its n_cells cells: indices, parsed evaluations and per-cell parse status at
+// b * n_cells; it writes 4096 coefficients at coef_out + b * 4096 and status[b] (0, or 1 / 2 = C_KZG_BADARGS /
+// C_KZG_ERROR by mode, as cell_parse_kernel).  The indices live on the device, so they are validated here: a blob
+// with an index >= 128, indices not strictly ascending or a word >= r gets a zero coefficient row, so that the later
+// stages of the pass read initialised memory.
 __global__ void __launch_bounds__(REC_THREADS) cell_recover_kernel(Fr* __restrict__ coef_out, int* __restrict__ status, Fr* __restrict__ ws,
-                                                                  const uint32_t* __restrict__ evals, const uint64_t* __restrict__ cell_indices, int n_cells,
+                                                                  const uint32_t* __restrict__ evals, const int* __restrict__ cell_status,
+                                                                  const uint64_t* __restrict__ cell_indices, int n_cells, int mode,
                                                                   const Fr* __restrict__ tw) {
   extern __shared__ uint32_t sm[];
   __shared__ uint32_t present[128];
   __shared__ uint32_t small[3][8 * 128];   // short vanishing polynomial, its DFT on <nu>, its DFT on 7^64 <nu>
+  const int blob = blockIdx.x, tid = threadIdx.x;
+  const int fail = mode == 0 ? 2 : 1;
+  coef_out += (size_t)blob * 4096;
+  ws += (size_t)blob * 3 * 8192;
+  evals += (size_t)blob * n_cells * CELL_ELEMS * 8;
+  cell_status += (size_t)blob * n_cells;
+  cell_indices += (size_t)blob * n_cells;
   Fr* ext = ws;              // E in natural order, later E * Z, later the quotient
   Fr* tmp = ws + 8192;
   Fr* tmp2 = ws + 16384;
-  const int tid = threadIdx.x;
   if (tid < 128) present[tid] = 0;
-  __syncthreads();
+  bool malformed = false;
+  if (tid < n_cells) {
+    const uint64_t ix = cell_indices[tid];
+    malformed = ix >= N_CELLS || (tid > 0 && ix <= cell_indices[tid - 1]) || cell_status[tid] != 0;
+  }
+  if (__syncthreads_or(malformed)) {
+    for (int i = tid; i < 4096; i += blockDim.x) coef_out[i] = fr_zero();
+    if (tid == 0) status[blob] = fail;
+    return;
+  }
   if (tid < n_cells) present[cell_indices[tid] & 127u] = 1;
   __syncthreads();
   // ---- short vanishing polynomial prod (X - nu^brp7(i)) over the missing cells i (degree <= 64), by one thread
@@ -341,7 +362,9 @@ __global__ void __launch_bounds__(REC_THREADS) cell_recover_kernel(Fr* __restric
       else if (!fr_is_zero(v)) bad = true;
       p = fr_mul(p, sinv);
     }
-    if (bad) atomicOr(status, 1);   // inconsistent cells: no polynomial of degree < 4096 matches them (BADARGS)
+    // inconsistent cells: no polynomial of degree < 4096 matches them
+    bad = __syncthreads_or(bad);
+    if (tid == 0) status[blob] = bad ? fail : 0;
   }
 }
 
@@ -393,17 +416,18 @@ void launch_cell_verify_scalars(void* d_wcoef, void* d_rpow, void* d_scalars_b, 
   count_launch(2);
 }
 
-void launch_cell_recover(void* d_coef, int* d_status, const void* d_evals, const uint64_t* d_cell_indices, int n_cells, const void* d_tw8192, cudaStream_t st) {
-  // workspace: 3 x 8192 field elements behind the coefficient output (the caller allocates 4096 + 3 * 8192 elements)
-  static bool attr_set[64] = {};
+void launch_cell_recover(void* d_coef, int* d_status, void* d_ws, const void* d_evals, const int* d_cell_status, const uint64_t* d_cell_indices,
+                         int n_blobs, int n_cells, int mode, const void* d_tw8192, cudaStream_t st) {
+  if (n_blobs <= 0) return;
+  static bool attr_set[64] = {};   // function attributes are per device
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 64 && !attr_set[dev]) {
     cudaFuncSetAttribute(cell_recover_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, REC_SMEM);
     attr_set[dev] = true;
   }
-  Fr* coef = (Fr*)d_coef;
-  cell_recover_kernel<<<1, REC_THREADS, REC_SMEM, st>>>(coef, d_status, coef + 4096, (const uint32_t*)d_evals, d_cell_indices, n_cells, (const Fr*)d_tw8192);
+  cell_recover_kernel<<<n_blobs, REC_THREADS, REC_SMEM, st>>>((Fr*)d_coef, d_status, (Fr*)d_ws, (const uint32_t*)d_evals, d_cell_status, d_cell_indices,
+                                                             n_cells, mode, (const Fr*)d_tw8192);
   count_launch();
 }
 

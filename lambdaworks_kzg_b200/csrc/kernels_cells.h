@@ -62,9 +62,14 @@ void launch_cell_verify_scalars(void* d_wcoef, void* d_rpow, void* d_scalars_b, 
 // r = H(domain || 4096 || 64 || n_commitments || n_cells || commitments || (commitment_index || cell_index || cell || proof)...)
 void launch_cell_batch_challenge(void* d_r, const void* d_commitments48, int n_commitments, const uint32_t* d_commitment_indices, const uint64_t* d_cell_indices,
                                  const void* d_cells, const void* d_proofs48, int n_cells, int mode, cudaStream_t st);
-// recovery (one blob): evaluations of >= 64 cells -> coefficient form (Montgomery).  d_coef must hold 4096 + 3 * 8192 field
-// elements (the tail is workspace); *d_status |= 1 if the cells are inconsistent with a polynomial of degree < 4096
-void launch_cell_recover(void* d_coef, int* d_status, const void* d_evals, const uint64_t* d_cell_indices, int n_cells, const void* d_tw8192, cudaStream_t st);
+// recovery of n_blobs blobs, one block each: n_cells (64..128) cells per blob -> coefficient form (Montgomery,
+// d_coef: n_blobs x 4096 x 32 B).  Inputs are blob-major, n_blobs x n_cells: cell indices, evaluations and the per-cell
+// status of launch_cell_parse.  d_status[blob] = 0, or 1 / 2 (C_KZG_BADARGS / C_KZG_ERROR: mode 0 -> 2) when an index
+// is >= 128 or not strictly ascending, a word is >= r or no polynomial of degree < 4096 matches the cells; the
+// coefficient row of a malformed blob is zeroed.  d_ws: n_blobs x CELL_RECOVER_WS_BYTES of workspace
+constexpr size_t CELL_RECOVER_WS_BYTES = size_t(3) * EXT_POINTS * 32;
+void launch_cell_recover(void* d_coef, int* d_status, void* d_ws, const void* d_evals, const int* d_cell_status, const uint64_t* d_cell_indices,
+                         int n_blobs, int n_cells, int mode, const void* d_tw8192, cudaStream_t st);
 // coefficient form (Montgomery) -> cells (both halves computed by FFT) -- the tail of launch_cell_poly for callers that already hold coefficients
 void launch_cell_coef_to_cells(void* d_cells, const void* d_coef, int n, int mode, const void* d_tw8192, cudaStream_t st);
 

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
-"""lwkzg_set_devices for the PeerDAS calls: ONE process, one C call, every visible GPU.  The sharded cell batch must
-return the bytes of the single-device call (MODE_DENEB: the replicas get the monomial SRS from the primary context).
-Prints MULTI_DEVICE_CELLS_OK on success."""
+"""lwkzg_set_devices for the PeerDAS calls: ONE process, one C call, every visible GPU.  The sharded cell batch and the
+sharded recovery batch must return the bytes of the single-device calls (MODE_DENEB: the replicas get the monomial SRS
+from the primary context).  Prints MULTI_DEVICE_CELLS_OK on success."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -26,11 +26,27 @@ def run(tag):
     return cells, proofs
 
 
+def recover(tag, idx, sel):
+    t0 = time.perf_counter()
+    cells, proofs, st = lw.recover_cells_and_kzg_proofs_batch(idx, sel, 64, n, s)
+    dt = time.perf_counter() - t0
+    assert not any(st)
+    print("%s: recovered %d blobs from 64 cells each in %.1f ms" % (tag, n, dt * 1e3), flush=True)
+    return cells, proofs
+
+
 run("1 device (first call builds the FK20 tables)")
 c1, p1 = run("1 device ")
+keep = list(range(1, 128, 2))
+idx = keep * n
+sel = b"".join(c1[(b * 128 + i) * 2048: (b * 128 + i + 1) * 2048] for b in range(n) for i in keep)
+rc1, rp1 = recover("1 device ", idx, sel)
+assert rc1 == c1 and rp1 == p1, "recovered outputs differ from the computed ones"
 lw.set_devices(list(range(g)))
 run("%d devices (first call builds the replicas)" % g)
 c2, p2 = run("%d devices" % g)
 assert c1 == c2 and p1 == p2, "multi-device cell outputs differ from the single-device outputs"
+rc2, rp2 = recover("%d devices" % g, idx, sel)
+assert rc2 == rc1 and rp2 == rp1, "multi-device recovery outputs differ from the single-device outputs"
 lw.set_devices([])
 print("MULTI_DEVICE_CELLS_OK", flush=True)
