@@ -92,9 +92,16 @@ Options& opts() {
 }
 std::mutex g_mu;  // guards the options
 
+// Device buffer that grows on demand and is freed with its owner.  The owner synchronises the streams that use it first.
 struct DevBuf {
   void* p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() {
+    if (p) cudaFree(p);
+  }
   bool ensure(size_t bytes) {
     if (bytes <= cap) return true;
     if (p) cudaFree(p);
@@ -104,12 +111,21 @@ struct DevBuf {
     cap = bytes;
     return true;
   }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
-  }
 };
+
+// Every device buffer of a workspace with the bytes one request needs, listed once per workspace: both "reserve" and
+// "already fits" are answered from that list.
+using BufList = std::vector<std::pair<DevBuf*, size_t>>;
+bool reserve(const BufList& bufs) {
+  for (const auto& b : bufs)
+    if (!b.first->ensure(b.second)) return false;
+  return true;
+}
+bool fits(const BufList& bufs) {
+  for (const auto& b : bufs)
+    if (b.first->cap < b.second) return false;
+  return true;
+}
 
 // ------------------------------------------------------------------ pageable host buffers
 // A c-kzg caller passes ordinary (pageable) memory.  cudaMemcpyAsync from pageable memory is a synchronous, single-
@@ -362,7 +378,6 @@ void destroy_ctx(Ctx* c) {
   for (auto& s : c->slot) {
     if (s.st) cudaStreamSynchronize(s.st);
     if (s.aux) cudaStreamSynchronize(s.aux);
-    for (DevBuf* b : {&s.ba_scratch, &s.blobs, &s.q, &s.partials, &s.states, &s.z, &s.y, &s.ybe, &s.c48, &s.cin48, &s.p48, &s.caff, &s.status, &s.status2, &s.zbe}) b->release();
     if (s.ev_in) cudaEventDestroy(s.ev_in);
     if (s.ev_aux) cudaEventDestroy(s.ev_aux);
     if (s.ev_done) cudaEventDestroy(s.ev_done);
@@ -371,9 +386,6 @@ void destroy_ctx(Ctx* c) {
     if (s.aux) cudaStreamDestroy(s.aux);
   }
   if (c->hash_st) cudaStreamSynchronize(c->hash_st);
-  for (DevBuf* b : {&c->vb_cin, &c->vb_pin, &c->vb_caff, &c->vb_piaff, &c->vb_c48r, &c->vb_p48r, &c->vb_z, &c->vb_y, &c->vb_tuples, &c->vb_status,
-                    &c->vb_r, &c->vb_partial, &c->vb_scratch, &c->vb_ok, &c->vb_zy_in, &c->vb_hstate, &c->vb_blobs, &c->vb_states, &c->vb_status2, &c->vb_sub})
-    b->release();
   if (c->ev_hash) cudaEventDestroy(c->ev_hash);
   for (cudaEvent_t e : c->ev_pool) cudaEventDestroy(e);
   if (c->copy_st) { cudaStreamSynchronize(c->copy_st); cudaStreamDestroy(c->copy_st); }
@@ -747,23 +759,16 @@ int auto_bpb(int n) {
 
 void run_msm(Slot& s, const Ctx* c, const void* d_scalars, bool be_input, int n, int bpb, cudaStream_t st);
 
-bool slot_reserve(Slot& s, int n, int bpb, bool need_blobs) {
-  if (use_batch_affine(n) && !s.ba_scratch.ensure(msm_ba_scratch_bytes(n * bpb))) return false;
-  if (need_blobs && !s.blobs.ensure((size_t)n * BLOB_BYTES)) return false;
-  return s.q.ensure((size_t)n * BLOB_BYTES) && s.partials.ensure((size_t)n * bpb * XYZZ_BYTES) && s.states.ensure((size_t)n * 32) &&
-         s.z.ensure((size_t)n * 32) && s.y.ensure((size_t)n * 32) && s.ybe.ensure((size_t)n * 32) && s.c48.ensure((size_t)n * 48) &&
-         s.cin48.ensure((size_t)n * 48) && s.p48.ensure((size_t)n * 48) && s.caff.ensure((size_t)n * AFFINE_BYTES) &&
-         s.status.ensure((size_t)n * sizeof(int)) && s.status2.ensure((size_t)n * sizeof(int)) && s.zbe.ensure((size_t)n * 32);
-}
-
-// true when slot_reserve(s, n, bpb, need_blobs) would not have to reallocate anything
-bool slot_fits(const Slot& s, int n, int bpb, bool need_blobs) {
+// the buffers of a pipeline slot for a chunk of n blobs split bpb ways (need_blobs: the blobs are copied in)
+BufList slot_buffers(Slot& s, int n, int bpb, bool need_blobs) {
   const size_t m = (size_t)n;
-  if (use_batch_affine(n) && s.ba_scratch.cap < msm_ba_scratch_bytes(n * bpb)) return false;
-  if (need_blobs && s.blobs.cap < m * BLOB_BYTES) return false;
-  return s.q.cap >= m * BLOB_BYTES && s.partials.cap >= m * bpb * XYZZ_BYTES && s.states.cap >= m * 32 && s.z.cap >= m * 32 &&
-         s.y.cap >= m * 32 && s.ybe.cap >= m * 32 && s.c48.cap >= m * 48 && s.cin48.cap >= m * 48 && s.p48.cap >= m * 48 &&
-         s.caff.cap >= m * AFFINE_BYTES && s.status.cap >= m * sizeof(int) && s.status2.cap >= m * sizeof(int) && s.zbe.cap >= m * 32;
+  BufList bufs;
+  if (use_batch_affine(n)) bufs.push_back({&s.ba_scratch, msm_ba_scratch_bytes(n * bpb)});
+  if (need_blobs) bufs.push_back({&s.blobs, m * BLOB_BYTES});
+  bufs.insert(bufs.end(), {{&s.q, m * BLOB_BYTES}, {&s.partials, m * bpb * XYZZ_BYTES}, {&s.states, m * 32}, {&s.z, m * 32}, {&s.y, m * 32},
+                           {&s.ybe, m * 32}, {&s.c48, m * 48}, {&s.cin48, m * 48}, {&s.p48, m * 48}, {&s.caff, m * AFFINE_BYTES},
+                           {&s.status, m * sizeof(int)}, {&s.status2, m * sizeof(int)}, {&s.zbe, m * 32}});
+  return bufs;
 }
 
 void run_msm(Slot& s, const Ctx* c, const void* d_scalars, bool be_input, int n, int bpb, cudaStream_t st) {
@@ -866,28 +871,41 @@ bool enqueue_chunk(Ctx* c, Slot& s, Mode mode, const void* d_blobs, int n, void*
   return true;
 }
 
-C_KZG_RET first_bad(const std::vector<int>& st) {
-  for (int v : st)
-    if (v) return (C_KZG_RET)v;
-  return C_KZG_OK;
-}
-
 // ------------------------------------------------------------------ devices (lwkzg_set_devices)
 std::vector<int>& device_list() {   // guarded by g_mu; empty = whatever device the settings were loaded on
   static std::vector<int> d;
   return d;
 }
 
-// The contexts a multi-device call runs on: the primary one plus a replica per other device of lwkzg_set_devices
-// (same SRS, same window, same mode), built side by side on first use.
-std::vector<Ctx*> ctxs_for(Ctx* c) {
+// Replica of c on the current device: same SRS, same window, same mode.  The host arrays hold the Lagrange points in
+// the Lagrange modes, so the replica also gets a copy of the monomial points the primary context kept (FK20, cell
+// verification).  NULL when any of it fails.
+Ctx* build_replica(const Ctx* c) {
+  Ctx* r = build_ctx(c->g1_host, c->g2_host, c->mode, c->c);
+  if (!r || r->d_mono || !c->d_mono) return r;
+  const size_t bytes = (size_t)N_POINTS * AFFINE_BYTES;
+  cudaStream_t st = r->slot[0].st;
+  if (cudaMalloc(&r->d_mono, bytes) != cudaSuccess) { destroy_ctx(r); return nullptr; }
+  r->mono_owned = true;
+  if (cudaMemcpyPeerAsync(r->d_mono, r->device, c->d_mono, c->device, bytes, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) {
+    destroy_ctx(r);
+    return nullptr;
+  }
+  return r;
+}
+
+// The contexts a call over n items runs on: the primary one plus a replica per other device of lwkzg_set_devices,
+// built side by side on first use.  The call shards only when every context gets at least two items; otherwise it
+// runs on the primary context alone and no replica is built for it.
+std::vector<Ctx*> ctxs_for(Ctx* c, size_t n) {
   std::vector<int> devs;
   {
     std::lock_guard<std::mutex> lk(g_mu);
     devs = device_list();
   }
   std::vector<Ctx*> out{c};
-  if (devs.size() <= 1 || !c->srs_valid) return out;
+  const size_t g = 1 + devs.size() - std::count(devs.begin(), devs.end(), c->device);
+  if (devs.size() <= 1 || !c->srs_valid || n < 2 * g) return out;
   std::lock_guard<std::mutex> lk(c->replicas_mu);
   std::vector<int> missing;
   for (int d : devs) {
@@ -902,7 +920,7 @@ std::vector<Ctx*> ctxs_for(Ctx* c) {
     for (size_t k = 0; k < missing.size(); k++)
       th.emplace_back([&, k]() {
         if (cudaSetDevice(missing[k]) != cudaSuccess) return;
-        built[k] = build_ctx(c->g1_host, c->g2_host, c->mode, c->c);
+        built[k] = build_replica(c);
       });
     for (auto& t : th) t.join();
     for (Ctx* b : built)
@@ -921,6 +939,56 @@ void shard_of(size_t n, size_t g, size_t k, size_t& first, size_t& count) {
   const size_t base = n / g, rem = n % g;
   count = base + (k < rem ? 1 : 0);
   first = k * base + std::min(k, rem);
+}
+
+// fn(k, ctxs[k], first, count) for every shard of n items over the contexts, with that context's device current: one
+// host thread per context, or inline on the calling thread when there is only one.  Returns the first failing code
+// and its shard's error message.
+template <class Fn>
+C_KZG_RET for_shards(const std::vector<Ctx*>& ctxs, size_t n, const Fn& fn) {
+  const size_t g = ctxs.size();
+  std::vector<C_KZG_RET> rcs(g, C_KZG_OK);
+  std::vector<std::string> errs(g);
+  auto shard = [&](size_t k) {
+    size_t first, count;
+    shard_of(n, g, k, first, count);
+    DeviceGuard dg(ctxs[k]->device);
+    rcs[k] = fn(k, ctxs[k], first, count);
+    if (rcs[k] != C_KZG_OK) errs[k] = tl_err;
+  };
+  if (g == 1) {
+    shard(0);
+  } else {
+    std::vector<std::thread> th;
+    for (size_t k = 0; k < g; k++) th.emplace_back(shard, k);
+    for (auto& t : th) t.join();
+  }
+  for (size_t k = 0; k < g; k++)
+    if (rcs[k] != C_KZG_OK) { set_err(errs[k]); return rcs[k]; }
+  return C_KZG_OK;
+}
+
+// Host-buffer batches of independent items (commitments, proofs, cells, recovery: no exchange between shards) over
+// the devices of lwkzg_set_devices.  run(ctx, first, count, status + first) does one shard on one device and fills
+// one status code per item.  An unusable SRS fails every item.  With status == NULL the first failing item's code is
+// returned, with `what` as the error message.
+template <class Run>
+C_KZG_RET sharded_batch(Ctx* c, size_t n, int* status, const char* what, const Run& run) {
+  if (!c->srs_valid) {
+    set_err("SRS re-hydration failed: g1_values holds a point that is not on the curve");
+    if (status) for (size_t i = 0; i < n; i++) status[i] = C_KZG_ERROR;
+    return C_KZG_ERROR;
+  }
+  std::vector<int> st_own;
+  int* st = status;
+  if (!st) { st_own.assign(n, 0); st = st_own.data(); }
+  C_KZG_RET rc = for_shards(ctxs_for(c, n), n, [&](size_t, Ctx* x, size_t first, size_t count) { return run(x, first, count, st + first); });
+  if (rc != C_KZG_OK) return rc;
+  if (!status) {
+    for (size_t i = 0; i < n; i++)
+      if (st[i]) { set_err(what); return (C_KZG_RET)st[i]; }
+  }
+  return C_KZG_OK;
 }
 
 // Host-buffer batch driver on ONE device: chunked, double-buffered over the stream slots so
@@ -962,7 +1030,7 @@ C_KZG_RET host_batch_on(Ctx* c, Mode mode, size_t n, const Blob* blobs, const By
     int m = (int)m_sz;
     Slot& sl = c->slot[k % NSLOT];
     if (cudaStreamSynchronize(sl.st) != cudaSuccess) { set_err("stream sync failed"); return fail(); }
-    if (!slot_reserve(sl, m, auto_bpb(m), true)) return fail();
+    if (!reserve(slot_buffers(sl, m, auto_bpb(m), true))) return fail();
     if (pageable) {
       if (!c->ring.h2d(sl.blobs.p, blobs + off, (size_t)m * BLOB_BYTES, c->ring_seq++, sl.st)) return fail();
     } else if (cudaMemcpyAsync(sl.blobs.p, blobs + off, (size_t)m * BLOB_BYTES, cudaMemcpyHostToDevice, sl.st) != cudaSuccess) { set_err("H2D failed"); return fail(); }
@@ -1002,42 +1070,10 @@ C_KZG_RET host_batch(Mode mode, const KZGSettings* s, size_t n, const Blob* blob
   if (n == 0) return C_KZG_OK;
   Ctx* c = ctx_of(s);
   if (!c) return C_KZG_ERROR;
-  if (!c->srs_valid) {
-    set_err("SRS re-hydration failed: g1_values holds a point that is not on the curve");
-    if (status) for (size_t i = 0; i < n; i++) status[i] = C_KZG_ERROR;
-    return C_KZG_ERROR;
-  }
-  std::vector<int> st_own;
-  int* st = status;
-  if (!st) { st_own.assign(n, 0); st = st_own.data(); }
-  C_KZG_RET rc = C_KZG_OK;
-  std::vector<Ctx*> ctxs = n >= 2 ? ctxs_for(c) : std::vector<Ctx*>{c};
-  if (ctxs.size() <= 1 || n < 2 * ctxs.size()) {
-    rc = host_batch_on(c, mode, n, blobs, commit_in, z_in, c_out, p_out, y_out, st);
-  } else {
-    const size_t g = ctxs.size();
-    std::vector<C_KZG_RET> rcs(g, C_KZG_OK);
-    std::vector<std::string> errs(g);
-    std::vector<std::thread> th;
-    for (size_t k = 0; k < g; k++)
-      th.emplace_back([&, k]() {
-        size_t first, cnt;
-        shard_of(n, g, k, first, cnt);
-        if (!cnt) return;
-        rcs[k] = host_batch_on(ctxs[k], mode, cnt, blobs + first, commit_in ? commit_in + first : nullptr, z_in ? z_in + first : nullptr,
-                               c_out ? c_out + first : nullptr, p_out ? p_out + first : nullptr, y_out ? y_out + first : nullptr, st + first);
-        if (rcs[k] != C_KZG_OK) errs[k] = tl_err;
-      });
-    for (auto& t : th) t.join();
-    for (size_t k = 0; k < g; k++)
-      if (rcs[k] != C_KZG_OK && rc == C_KZG_OK) { rc = rcs[k]; set_err(errs[k]); }
-  }
-  if (rc != C_KZG_OK) return rc;
-  if (!status) {
-    for (size_t i = 0; i < n; i++)
-      if (st[i]) { set_err("invalid input item"); return (C_KZG_RET)st[i]; }
-  }
-  return C_KZG_OK;
+  return sharded_batch(c, n, status, "invalid input item", [&](Ctx* x, size_t first, size_t count, int* st) {
+    return host_batch_on(x, mode, count, blobs + first, commit_in ? commit_in + first : nullptr, z_in ? z_in + first : nullptr,
+                         c_out ? c_out + first : nullptr, p_out ? p_out + first : nullptr, y_out ? y_out + first : nullptr, st);
+  });
 }
 
 // Device-buffer batch driver, asynchronous with respect to the host: forks from
@@ -1068,13 +1104,16 @@ C_KZG_RET device_batch(Mode mode, const KZGSettings* s, size_t n, const void* d_
   // The host only waits for earlier work when a buffer really has to grow: back-to-back calls (also from
   // different user streams) then queue behind each other on the slot streams and the tail of one batch
   // overlaps the head of the next.
-  bool fits = true;
-  for (size_t k = 0; k < plan.size() && fits; k++)
-    fits = slot_fits(c->slot[k % NSLOT], (int)plan[k].second, auto_bpb((int)plan[k].second), false);
-  if (!fits) {
+  std::vector<BufList> bufs;
+  bool all_fit = true;
+  for (size_t k = 0; k < plan.size(); k++) {
+    bufs.push_back(slot_buffers(c->slot[k % NSLOT], (int)plan[k].second, auto_bpb((int)plan[k].second), false));
+    all_fit = all_fit && fits(bufs.back());
+  }
+  if (!all_fit) {
     for (auto& sl : c->slot) { cudaStreamSynchronize(sl.st); cudaStreamSynchronize(sl.aux); }
-    for (size_t k = 0; k < plan.size(); k++)
-      if (!slot_reserve(c->slot[k % NSLOT], (int)plan[k].second, auto_bpb((int)plan[k].second), false)) return C_KZG_ERROR;
+    for (const BufList& b : bufs)
+      if (!reserve(b)) return C_KZG_ERROR;
   }
   cudaEvent_t ev_user;
   if (cudaEventCreateWithFlags(&ev_user, cudaEventDisableTiming) != cudaSuccess) { set_err("event"); return C_KZG_ERROR; }
@@ -1204,7 +1243,7 @@ C_KZG_RET settings_from_compressed(KZGSettings* out, const uint8_t* g1_bytes, si
       void *d_rows = nullptr, *d_aff = nullptr, *d_canon = nullptr;
       Slot& sl = tmp->slot[0];
       const int bpb = 1;
-      if (!slot_reserve(sl, N_POINTS, bpb, false)) return false;
+      if (!reserve(slot_buffers(sl, N_POINTS, bpb, false))) return false;
       CU_TRY(cudaMalloc(&d_rows, (size_t)N_POINTS * BLOB_BYTES));
       CU_TRY(cudaMalloc(&d_aff, (size_t)N_POINTS * AFFINE_BYTES));
       CU_TRY(cudaMalloc(&d_canon, (size_t)N_POINTS * 96));
@@ -1729,92 +1768,103 @@ static C_KZG_RET verify_blob_single(bool* ok, const Blob* blob, const Bytes48* c
   return C_KZG_OK;
 }
 
-// verify_blob_kzg_proof_batch over the GPUs of lwkzg_set_devices (SURVEY 8e): contiguous shards, one host thread
-// per device.  Phase 1 is local (decode, challenge, evaluation -> 160-byte tuples); exchange A brings the tuples
-// to the primary device, which derives r (one sequential hash over ALL tuples, utils.rs:166-206); phase 2 is local
-// again (the two MSMs of the shard with r^(first + i)); exchange B brings 288 bytes per device back; the primary
-// device adds them and runs the 2-pairing check.  Both exchanges are a few hundred KB at most and go through
-// pinned host memory of this one process.  Group addition is exact: the boolean does not depend on the sharding.
+// ---- the three phases of a batched verification, on a context whose lock the caller holds.  The batched call, the
+// same call over several GPUs and the distributed phase entry points below are all assembled from these.
+
+// Phase 1: per-item preparation into the workspace (hash_r: the batch challenge r into vb_r as well), the first invalid
+// item's code, then -- when tuples_out is given -- the 160-byte tuples copied there on s0 and waited for.
+static C_KZG_RET phase1_on(Ctx* c, const Blob* blobs, const Bytes48* commitments, const Bytes48* proofs, size_t n, bool inputs_on_device,
+                           bool hash_r, void* tuples_out, bool out_on_device) {
+  if (!verify_prepare(c, blobs, commitments, proofs, n, hash_r, inputs_on_device)) return C_KZG_ERROR;
+  int bad = 0;
+  if (!first_bad_status(c, n, bad)) return C_KZG_ERROR;
+  if (bad) { set_err("invalid commitment, proof or field element bytes"); return bad_code(bad); }
+  if (!tuples_out) return C_KZG_OK;
+  // on the context's stream and waited for: a plain cudaMemcpy between device buffers may still be running when it
+  // returns, on the legacy stream, which the library's non-blocking streams (phase 2 reads these tuples) do not wait for
+  cudaStream_t s0 = c->slot[0].st;
+  if (cudaMemcpyAsync(tuples_out, c->vb_tuples.p, n * 160, out_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s0) != cudaSuccess ||
+      cudaStreamSynchronize(s0) != cudaSuccess) {
+    set_err("tuple copy failed");
+    return C_KZG_ERROR;
+  }
+  return C_KZG_OK;
+}
+
+// Phase 2: the partial sums of items [first, first + count) with weights r^(first + i), r already in vb_r, into
+// vb_partial.  When partial_out is given, the 288 bytes are copied there and waited for.
+static bool phase2_on(Ctx* c, size_t first, size_t count, void* partial_out, bool out_on_device) {
+  if (!c->vb_partial.ensure(288) || !c->vb_scratch.ensure(batch_partials_scratch_bytes((int)std::max<size_t>(count, 1)))) return false;
+  cudaStream_t s0 = c->slot[0].st;
+  launch_batch_partials(c->vb_partial.p, c->vb_r.p, c->vb_caff.p, c->vb_piaff.p, c->vb_z.p, c->vb_y.p, first, (int)count, c->vb_scratch.p, s0,
+                        c->slot[0].aux, c->slot[0].ev_fork, c->slot[0].ev_aux);
+  if (!partial_out) return true;
+  CU_TRY(cudaMemcpyAsync(partial_out, c->vb_partial.p, 288, out_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s0));
+  CU_TRY(cudaStreamSynchronize(s0));
+  CU_TRY(cudaGetLastError());
+  return true;
+}
+
+// Phase 3: the sum of `count` partial sums (host or device memory) and the 2-pairing check
+static C_KZG_RET phase3_on(Ctx* c, bool* ok, const void* partials288, bool on_device, size_t count) {
+  cudaStream_t s0 = c->slot[0].st;
+  DevBuf staged;   // the partial sums, when they come from host memory
+  if (!on_device && !staged.ensure(std::max<size_t>(count, 1) * 288)) { set_err("cudaMalloc failed"); return C_KZG_MALLOC; }
+  int okv = 0;
+  bool good = [&]() -> bool {
+    if (!c->vb_ok.ensure(sizeof(int))) return false;
+    if (!on_device) CU_TRY(cudaMemcpyAsync(staged.p, partials288, count * 288, cudaMemcpyHostToDevice, s0));
+    launch_batch_final((int*)c->vb_ok.p, on_device ? partials288 : staged.p, (int)count, c->d_prep0, c->d_prep1, s0);
+    CU_TRY(cudaMemcpyAsync(&okv, c->vb_ok.p, sizeof(int), cudaMemcpyDeviceToHost, s0));
+    CU_TRY(cudaStreamSynchronize(s0));
+    CU_TRY(cudaGetLastError());
+    return true;
+  }();
+  if (!good) return C_KZG_ERROR;
+  *ok = okv != 0;
+  return C_KZG_OK;
+}
+
+// verify_blob_kzg_proof_batch over the GPUs of lwkzg_set_devices (SURVEY 8e): the distributed phases, with one host
+// thread per device instead of one process.  Phase 1 on every shard; the tuples meet in host memory and the primary
+// device derives r (one sequential hash over ALL tuples, utils.rs:166-206) and hands it to the others; phase 2 on
+// every shard; phase 3 on the primary device over the g partial sums.  Both exchanges are a few hundred KB at most.
+// Group addition is exact: the boolean does not depend on the sharding.
 static C_KZG_RET verify_blob_batch_multi(bool* ok, const Blob* blobs, const Bytes48* cs, const Bytes48* ps, size_t n, std::vector<Ctx*>& ctxs) {
   const size_t g = ctxs.size();
   Ctx* c0 = ctxs[0];
   std::vector<std::unique_lock<std::mutex>> locks;
   for (Ctx* c : ctxs) locks.emplace_back(c->mu);
   std::vector<uint8_t> tuples(n * 160), partials(g * 288);
-  std::vector<int> rc(g, 0), bad(g, 0);
-  std::vector<std::string> errs(g);
-  auto run_all = [&](auto fn) {
-    std::vector<std::thread> th;
-    for (size_t k = 0; k < g; k++)
-      th.emplace_back([&, k]() {
-        size_t first, cnt;
-        shard_of(n, g, k, first, cnt);
-        DeviceGuard dg(ctxs[k]->device);
-        if (!fn(k, ctxs[k], first, cnt)) { rc[k] = 1; errs[k] = tl_err; }
-      });
-    for (auto& t : th) t.join();
-    for (size_t k = 0; k < g; k++)
-      if (rc[k]) { set_err(errs[k]); return false; }
-    return true;
-  };
-  // phase 1 + exchange A
-  if (!run_all([&](size_t k, Ctx* c, size_t first, size_t cnt) -> bool {
-        if (!verify_prepare(c, blobs + first, cs + first, ps + first, cnt)) return false;
-        if (!first_bad_status(c, cnt, bad[k])) return false;
-        CU_TRY(cudaMemcpy(tuples.data() + first * 160, c->vb_tuples.p, cnt * 160, cudaMemcpyDeviceToHost));
-        return true;
-      }))
-    return C_KZG_ERROR;
-  for (size_t k = 0; k < g; k++)
-    if (bad[k]) { for (Ctx* c : ctxs) c->vb_n = 0; set_err("invalid commitment, proof or field element bytes"); return bad_code(bad[k]); }
-  // r on the primary device
+  C_KZG_RET rc = for_shards(ctxs, n, [&](size_t, Ctx* c, size_t first, size_t count) {
+    return phase1_on(c, blobs + first, cs + first, ps + first, count, false, false, tuples.data() + first * 160, false);
+  });
   uint32_t r_host[8];
-  {
+  if (rc == C_KZG_OK) {
     DeviceGuard dg(c0->device);
     cudaStream_t s0 = c0->slot[0].st;
-    void* d_all = nullptr;
-    if (cudaMalloc(&d_all, n * 160) != cudaSuccess) { set_err("cudaMalloc failed"); return C_KZG_MALLOC; }
-    bool good = [&]() -> bool {
-      CU_TRY(cudaMemcpyAsync(d_all, tuples.data(), n * 160, cudaMemcpyHostToDevice, s0));
-      launch_batch_challenge(c0->vb_r.p, d_all, n, s0, c0->mode);
+    DevBuf all;
+    auto derive_r = [&]() -> bool {
+      CU_TRY(cudaMemcpyAsync(all.p, tuples.data(), n * 160, cudaMemcpyHostToDevice, s0));
+      launch_batch_challenge(c0->vb_r.p, all.p, n, s0, c0->mode);
       CU_TRY(cudaMemcpyAsync(r_host, c0->vb_r.p, 32, cudaMemcpyDeviceToHost, s0));
       CU_TRY(cudaStreamSynchronize(s0));
       return true;
-    }();
-    cudaFree(d_all);
-    if (!good) return C_KZG_ERROR;
+    };
+    if (!all.ensure(n * 160)) { set_err("cudaMalloc failed"); rc = C_KZG_MALLOC; }
+    else if (!derive_r()) rc = C_KZG_ERROR;
   }
-  // phase 2 + exchange B
-  if (!run_all([&](size_t k, Ctx* c, size_t first, size_t cnt) -> bool {
-        cudaStream_t s0 = c->slot[0].st;
-        CU_TRY(cudaMemcpyAsync(c->vb_r.p, r_host, 32, cudaMemcpyHostToDevice, s0));
-        launch_batch_partials(c->vb_partial.p, c->vb_r.p, c->vb_caff.p, c->vb_piaff.p, c->vb_z.p, c->vb_y.p, first, (int)cnt, c->vb_scratch.p, s0,
-                              c->slot[0].aux, c->slot[0].ev_fork, c->slot[0].ev_aux);
-        CU_TRY(cudaMemcpyAsync(partials.data() + k * 288, c->vb_partial.p, 288, cudaMemcpyDeviceToHost, s0));
-        CU_TRY(cudaStreamSynchronize(s0));
-        CU_TRY(cudaGetLastError());
-        c->vb_n = 0;
-        return true;
-      }))
-    return C_KZG_ERROR;
-  // phase 3
+  if (rc == C_KZG_OK) {
+    rc = for_shards(ctxs, n, [&](size_t k, Ctx* c, size_t first, size_t count) {
+      const bool good = cudaMemcpyAsync(c->vb_r.p, r_host, 32, cudaMemcpyHostToDevice, c->slot[0].st) == cudaSuccess &&
+                        phase2_on(c, first, count, partials.data() + k * 288, false);
+      return good ? C_KZG_OK : C_KZG_ERROR;
+    });
+  }
+  for (Ctx* c : ctxs) c->vb_n = 0;
+  if (rc != C_KZG_OK) return rc;
   DeviceGuard dg(c0->device);
-  cudaStream_t s0 = c0->slot[0].st;
-  void* d_p = nullptr;
-  if (cudaMalloc(&d_p, g * 288) != cudaSuccess) { set_err("cudaMalloc failed"); return C_KZG_MALLOC; }
-  int okv = 0;
-  bool good = [&]() -> bool {
-    CU_TRY(cudaMemcpyAsync(d_p, partials.data(), g * 288, cudaMemcpyHostToDevice, s0));
-    launch_batch_final((int*)c0->vb_ok.p, d_p, (int)g, c0->d_prep0, c0->d_prep1, s0);
-    CU_TRY(cudaMemcpyAsync(&okv, c0->vb_ok.p, sizeof(int), cudaMemcpyDeviceToHost, s0));
-    CU_TRY(cudaStreamSynchronize(s0));
-    CU_TRY(cudaGetLastError());
-    return true;
-  }();
-  cudaFree(d_p);
-  if (!good) return C_KZG_ERROR;
-  *ok = okv != 0;
-  return C_KZG_OK;
+  return phase3_on(c0, ok, partials.data(), false, g);
 }
 
 static C_KZG_RET verify_blob_batch(bool* ok, const Blob* blobs, const Bytes48* commitments_bytes, const Bytes48* proofs_bytes, size_t n,
@@ -1831,32 +1881,21 @@ static C_KZG_RET verify_blob_batch(bool* ok, const Blob* blobs, const Bytes48* c
   Ctx* c = ctx_of(s);
   if (!c) return C_KZG_ERROR;
   if (!dev_inputs) {
-    std::vector<Ctx*> ctxs = ctxs_for(c);
-    if (ctxs.size() > 1 && n >= 2 * ctxs.size()) return verify_blob_batch_multi(ok, blobs, commitments_bytes, proofs_bytes, n, ctxs);
+    std::vector<Ctx*> ctxs = ctxs_for(c, n);
+    if (ctxs.size() > 1) return verify_blob_batch_multi(ok, blobs, commitments_bytes, proofs_bytes, n, ctxs);
   }
   CtxLock L(c);
   static const bool trace = getenv("LWKZG_VERIFY_TRACE") != nullptr;
   auto now = []() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double t0 = now();
-  if (!verify_prepare(c, blobs, commitments_bytes, proofs_bytes, n, true, dev_inputs)) return C_KZG_ERROR;  // leaves r in vb_r
+  if (C_KZG_RET rc = phase1_on(c, blobs, commitments_bytes, proofs_bytes, n, dev_inputs, true, nullptr, false)) return rc;   // leaves r in vb_r
   const double t1 = now();
-  int bad = 0;
-  if (!first_bad_status(c, n, bad)) return C_KZG_ERROR;
-  if (bad) { set_err("invalid commitment, proof or field element bytes"); return bad_code(bad); }
-  const double t2 = now();
-  cudaStream_t s0 = c->slot[0].st;
-  launch_batch_partials(c->vb_partial.p, c->vb_r.p, c->vb_caff.p, c->vb_piaff.p, c->vb_z.p, c->vb_y.p, 0, (int)n, c->vb_scratch.p, s0, c->slot[0].aux,
-                        c->slot[0].ev_fork, c->slot[0].ev_aux);
-  launch_batch_final((int*)c->vb_ok.p, c->vb_partial.p, 1, c->d_prep0, c->d_prep1, s0);
-  int okv = 0;
-  if (cudaMemcpyAsync(&okv, c->vb_ok.p, sizeof(int), cudaMemcpyDeviceToHost, s0) != cudaSuccess || cudaStreamSynchronize(s0) != cudaSuccess ||
-      cudaGetLastError() != cudaSuccess) {
+  if (!phase2_on(c, 0, n, nullptr, false) || phase3_on(c, ok, c->vb_partial.p, true, 1) != C_KZG_OK) {
     set_err("CUDA failure in batch verification");
     return C_KZG_ERROR;
   }
   c->vb_n = 0;
-  if (trace) fprintf(stderr, "[lwkzg] verify batch n=%zu: prepare %.2f ms, status %.2f ms, partials+pairing %.2f ms\n", n, t1 - t0, t2 - t1, now() - t2);
-  *ok = okv != 0;
+  if (trace) fprintf(stderr, "[lwkzg] verify batch n=%zu: prepare + status %.2f ms, partials+pairing %.2f ms\n", n, t1 - t0, now() - t1);
   return C_KZG_OK;
 }
 
@@ -1883,20 +1922,7 @@ static C_KZG_RET phase1_impl(uint8_t* tuples_out, bool out_on_device, const Blob
   CtxLock L(c);
   c->vb_n = 0;
   if (n_local == 0) return C_KZG_OK;
-  if (!verify_prepare(c, blobs, commitments, proofs, n_local, false, inputs_on_device)) return C_KZG_ERROR;
-  int bad = 0;
-  if (!first_bad_status(c, n_local, bad)) return C_KZG_ERROR;
-  if (bad) { set_err("invalid commitment, proof or field element bytes"); return bad_code(bad); }
-  if (!c->srs_valid || !c->g2_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
-  // on the context's stream and waited for: a plain cudaMemcpy between device buffers may still be running when it
-  // returns, on the legacy stream, which the library's non-blocking streams (phase 2 reads these tuples) do not wait for
-  cudaStream_t s0 = c->slot[0].st;
-  if (cudaMemcpyAsync(tuples_out, c->vb_tuples.p, n_local * 160, out_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s0) != cudaSuccess ||
-      cudaStreamSynchronize(s0) != cudaSuccess) {
-    set_err("tuple copy failed");
-    return C_KZG_ERROR;
-  }
-  return C_KZG_OK;
+  return phase1_on(c, blobs, commitments, proofs, n_local, inputs_on_device, false, tuples_out, out_on_device);
 }
 C_KZG_RET lwkzg_verify_batch_phase1(uint8_t* tuples160, const Blob* blobs, const Bytes48* commitments, const Bytes48* proofs, size_t n_local,
                                     const KZGSettings* s) {
@@ -1915,20 +1941,14 @@ static C_KZG_RET phase2_impl(uint8_t* partial288, const uint8_t* all_tuples160, 
   CtxLock L(c);
   if (c->vb_n != n_local || first + n_local > n_total) { set_err("phase2 does not match the preceding phase1"); return C_KZG_BADARGS; }
   cudaStream_t s0 = c->slot[0].st;
-  void* d_all = nullptr;
-  if (!on_device && cudaMalloc(&d_all, std::max<size_t>(n_total, 1) * 160) != cudaSuccess) { set_err("cudaMalloc failed"); return C_KZG_MALLOC; }
+  DevBuf staged;   // all tuples, when they come from host memory
+  if (!on_device && !staged.ensure(std::max<size_t>(n_total, 1) * 160)) { set_err("cudaMalloc failed"); return C_KZG_MALLOC; }
   bool good = [&]() -> bool {
-    if (!on_device) CU_TRY(cudaMemcpyAsync(d_all, all_tuples160, n_total * 160, cudaMemcpyHostToDevice, s0));
-    if (!c->vb_r.ensure(32) || !c->vb_partial.ensure(288) || !c->vb_scratch.ensure(batch_partials_scratch_bytes((int)std::max<size_t>(n_local, 1)))) return false;
-    launch_batch_challenge(c->vb_r.p, on_device ? (const void*)all_tuples160 : d_all, n_total, s0, c->mode);
-    launch_batch_partials(c->vb_partial.p, c->vb_r.p, c->vb_caff.p, c->vb_piaff.p, c->vb_z.p, c->vb_y.p, first, (int)n_local, c->vb_scratch.p, s0,
-                          c->slot[0].aux, c->slot[0].ev_fork, c->slot[0].ev_aux);
-    CU_TRY(cudaMemcpyAsync(partial288, c->vb_partial.p, 288, on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s0));
-    CU_TRY(cudaStreamSynchronize(s0));
-    CU_TRY(cudaGetLastError());
-    return true;
+    if (!on_device) CU_TRY(cudaMemcpyAsync(staged.p, all_tuples160, n_total * 160, cudaMemcpyHostToDevice, s0));
+    if (!c->vb_r.ensure(32)) return false;
+    launch_batch_challenge(c->vb_r.p, on_device ? (const void*)all_tuples160 : staged.p, n_total, s0, c->mode);
+    return phase2_on(c, first, n_local, partial288, on_device);
   }();
-  if (d_all) cudaFree(d_all);
   return good ? C_KZG_OK : C_KZG_ERROR;
 }
 C_KZG_RET lwkzg_verify_batch_phase2(uint8_t* partial288, const uint8_t* all_tuples160, size_t n_total, size_t first, size_t n_local,
@@ -1947,23 +1967,7 @@ static C_KZG_RET phase3_impl(bool* ok, const uint8_t* partials288, bool on_devic
   if (!c) return C_KZG_ERROR;
   CtxLock L(c);
   if (!c->srs_valid || !c->g2_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
-  cudaStream_t s0 = c->slot[0].st;
-  void* d_p = nullptr;
-  if (!on_device && cudaMalloc(&d_p, std::max<size_t>(n_ranks, 1) * 288) != cudaSuccess) { set_err("cudaMalloc failed"); return C_KZG_MALLOC; }
-  int okv = 0;
-  bool good = [&]() -> bool {
-    if (!c->vb_ok.ensure(sizeof(int))) return false;
-    if (!on_device) CU_TRY(cudaMemcpyAsync(d_p, partials288, n_ranks * 288, cudaMemcpyHostToDevice, s0));
-    launch_batch_final((int*)c->vb_ok.p, on_device ? (const void*)partials288 : d_p, (int)n_ranks, c->d_prep0, c->d_prep1, s0);
-    CU_TRY(cudaMemcpyAsync(&okv, c->vb_ok.p, sizeof(int), cudaMemcpyDeviceToHost, s0));
-    CU_TRY(cudaStreamSynchronize(s0));
-    CU_TRY(cudaGetLastError());
-    return true;
-  }();
-  if (d_p) cudaFree(d_p);
-  if (!good) return C_KZG_ERROR;
-  *ok = okv != 0;
-  return C_KZG_OK;
+  return phase3_on(c, ok, partials288, on_device, n_ranks);
 }
 C_KZG_RET lwkzg_verify_batch_phase3(bool* ok, const uint8_t* partials288, size_t n_ranks, const KZGSettings* s) {
   return phase3_impl(ok, partials288, false, n_ranks, s);
@@ -2004,7 +2008,7 @@ double lwkzg_bench_msm_kernel(const void* d_blobs, size_t n, int blocks_per_blob
   Slot& sl = c->slot[0];
   int bpb = blocks_per_blob > 0 ? blocks_per_blob : auto_bpb((int)n);
   cudaStreamSynchronize(sl.st);
-  if (!slot_reserve(sl, (int)n, bpb, false)) return -1.0;
+  if (!reserve(slot_buffers(sl, (int)n, bpb, false))) return -1.0;
   cudaEvent_t e0, e1;
   cudaEventCreate(&e0);
   cudaEventCreate(&e1);
@@ -2117,8 +2121,8 @@ struct LincombWs {
 };
 std::mutex g_lincomb_mu;
 std::map<int, LincombWs>& lincomb_ws() {
-  static std::map<int, LincombWs> m;
-  return m;
+  static auto* m = new std::map<int, LincombWs>();   // never destroyed: no cudaFree during static destruction at exit
+  return *m;
 }
 }  // namespace
 
