@@ -268,6 +268,35 @@ C_KZG_RET lwkzg_recover_cells_and_kzg_proofs_batch_device(void *d_cells_out, voi
                                                           const void *d_cell_indices, const void *d_cells,
                                                           size_t num_cells, size_t n, const KZGSettings *s,
                                                           void *stream, void *d_status);
+/* additive: K = n_batches independent verify_cell_kzg_proof_batch checks in one call (a PeerDAS node checks each data
+ * column sidecar it receives as a batch of its own).  Batch b is cells [offsets[b], offsets[b+1]) of the flat arrays
+ * commitments / cell_indices / cells / proofs (one commitment per cell, as in the single call).  offsets: K + 1 host
+ * integers, offsets[0] == 0, non-decreasing.  ok[b] (K bools) gets the verdict of batch b alone; status[b] (may be
+ * NULL) gets the code verify_cell_kzg_proof_batch would return for batch b alone, and ok[b] is false when it is not
+ * C_KZG_OK.  An empty batch verifies.  A cell index >= 128, a cell word >= r, or a proof or commitment that does not
+ * decode or is not in G1 fails its own batch only: C_KZG_BADARGS in modes 1 and 2, C_KZG_ERROR in mode 0.  Each batch
+ * has its own challenge r_b over its own commitments, deduplicated in order of first appearance, exactly as the
+ * single call.  Whole-call errors: n_batches == 0 returns C_KZG_OK and writes nothing; a NULL required pointer,
+ * offsets that do not start at 0 or decrease, or more than 2^24 cells in total return C_KZG_BADARGS; with status ==
+ * NULL the first failing batch's code is returned (ok is still filled).  One call runs in passes of whole batches of
+ * at most "cell_chunk_blobs" x 128 cells (a larger batch gets a pass of its own); a pass is a fixed sequence of
+ * launches whatever its number of batches: one hash warp per batch, one segmented MSM over all batches, one pairing
+ * block per batch.  After lwkzg_set_devices the batches are sharded over the GPUs. */
+C_KZG_RET lwkzg_verify_cell_kzg_proof_batches(bool *ok, const Bytes48 *commitments, const uint64_t *cell_indices,
+                                              const Cell *cells, const Bytes48 *proofs, const uint64_t *offsets,
+                                              size_t n_batches, const KZGSettings *s, int *status);
+/* the same with commitments, cell_indices, cells and proofs in device memory (16-byte aligned); offsets stay on the
+ * host (the caller knows its batch sizes, and the host plans the passes from them without a synchronisation).
+ * Asynchronous, ordered after / before work on `stream`; d_ok and d_status are n_batches ints on the device (1 / 0 and
+ * C_KZG_RET values), d_status may be NULL.  Indices are validated on the device: a malformed batch gets its status and
+ * d_ok = 0, its later stages run on zeroed data. */
+C_KZG_RET lwkzg_verify_cell_kzg_proof_batches_device(void *d_ok, const void *d_commitments, const void *d_cell_indices,
+                                                     const void *d_cells, const void *d_proofs, const uint64_t *offsets,
+                                                     size_t n_batches, const KZGSettings *s, void *stream, void *d_status);
+/* Test hook: the challenge r_b of every non-empty batch that the last call of either form on these settings derived,
+ * 32 little-endian bytes each (as lwkzg_debug_batch_challenge); zeros for empty batches.  n_batches must not exceed
+ * the last call's. */
+C_KZG_RET lwkzg_debug_cell_batch_challenges(uint8_t *out32, size_t n_batches, const KZGSettings *s);
 /* Test hook: intermediate values of the FK20 pipeline for one blob, so a parity test can name the stage that deviates:
  * scalars = the 8192 MSM scalars DFT_128(circulant column b)_j / 128 as 32-byte little-endian integers, at index
  * (j / 64) * 4096 + b * 64 + j % 64 (the order of the two half tables);

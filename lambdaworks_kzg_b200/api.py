@@ -84,6 +84,9 @@ def load_library() -> ctypes.CDLL:
         "lwkzg_compute_cells_and_kzg_proofs_batch_device": [vp, vp, vp, sz, sp, vp, vp],
         "lwkzg_recover_cells_and_kzg_proofs_batch": [vp, vp, vp, vp, sz, sz, sp, ip],
         "lwkzg_recover_cells_and_kzg_proofs_batch_device": [vp, vp, vp, vp, sz, sz, sp, vp, vp],
+        "lwkzg_verify_cell_kzg_proof_batches": [bp, vp, vp, vp, vp, vp, sz, sp, ip],
+        "lwkzg_verify_cell_kzg_proof_batches_device": [vp, vp, vp, vp, vp, vp, sz, sp, vp, vp],
+        "lwkzg_debug_cell_batch_challenges": [vp, sz, sp],
         "lwkzg_cell_window_bits": [sp],
         "lwkzg_table_share": [sp],
         "lwkzg_debug_cell_stages": [vp, vp, vp, vp, vp, sp],
@@ -539,6 +542,44 @@ def verify_cell_kzg_proof_batch(commitments: Sequence[bytes], cell_indices: Sequ
     _check(load_library().verify_cell_kzg_proof_batch(ctypes.byref(ok), _cat(commitments, 48) or b"\0", idx, _cat(cells, BYTES_PER_CELL) or b"\0",
                                                       _cat(proofs, 48) or b"\0", n, _sp(s)), "verify_cell_kzg_proof_batch")
     return bool(ok.value)
+
+
+def verify_cell_kzg_proof_batches(batches: Sequence[Tuple[Sequence[bytes], Sequence[int], Sequence[bytes], Sequence[bytes]]], s) -> Tuple[List[bool], List[int]]:
+    """K independent verify_cell_kzg_proof_batch checks in one call.  batches: (commitments, cell_indices, cells, proofs)
+    per batch -> (verdict list, status list: the code the single call would return for each batch)."""
+    k = len(batches)
+    offsets = [0]
+    for com, idx, cl, pr in batches:
+        assert len(com) == len(idx) == len(cl) == len(pr)
+        offsets.append(offsets[-1] + len(idx))
+    n = offsets[-1]
+    idx = (ctypes.c_uint64 * max(1, n))(*[i for b in batches for i in b[1]])
+    off = (ctypes.c_uint64 * (k + 1))(*offsets)
+    oks = (ctypes.c_bool * max(1, k))()
+    st = _status_list(k)
+    _check(load_library().lwkzg_verify_cell_kzg_proof_batches(oks, b"".join(_cat(b[0], 48) for b in batches) or b"\0", idx,
+                                                              b"".join(_cat(b[2], BYTES_PER_CELL) for b in batches) or b"\0",
+                                                              b"".join(_cat(b[3], 48) for b in batches) or b"\0", off, k, _sp(s), st),
+           "lwkzg_verify_cell_kzg_proof_batches")
+    return [bool(oks[i]) for i in range(k)], list(st)[:k]
+
+
+def verify_cell_kzg_proof_batches_device(d_ok: int, d_commitments: int, d_cell_indices: int, d_cells: int, d_proofs: int, offsets: Sequence[int], s,
+                                         stream: int = 0, d_status: int = 0):
+    """All buffers are raw device addresses (torch: tensor.data_ptr()) except offsets (K + 1 host integers); d_ok and
+    d_status are K int32 each.  Asynchronous on `stream`."""
+    k = len(offsets) - 1
+    off = (ctypes.c_uint64 * max(1, k + 1))(*offsets)
+    _check(load_library().lwkzg_verify_cell_kzg_proof_batches_device(d_ok or None, d_commitments or None, d_cell_indices or None, d_cells or None,
+                                                                     d_proofs or None, off, k, _sp(s), stream or None, d_status or None),
+           "lwkzg_verify_cell_kzg_proof_batches_device")
+
+
+def debug_cell_batch_challenges(n_batches: int, s) -> List[int]:
+    """The challenges r_b the last verify_cell_kzg_proof_batches[_device] call derived (0 for empty batches; test hook)."""
+    out = ctypes.create_string_buffer(32 * max(1, n_batches))
+    _check(load_library().lwkzg_debug_cell_batch_challenges(out, n_batches, _sp(s)), "lwkzg_debug_cell_batch_challenges")
+    return [int.from_bytes(out.raw[32 * i: 32 * i + 32], "little") for i in range(n_batches)]
 
 
 def cell_window_bits(s) -> int:

@@ -13,6 +13,7 @@
 // (E * Z) on the whole domain, division on the coset 7 * <w8192> -- as one block working out of shared memory.
 #include "kernels_cells.h"
 #include "field.cuh"
+#include "g1.cuh"
 #include "kernels.h"
 #include "sha256.cuh"
 
@@ -106,6 +107,7 @@ __global__ void cell_parse_kernel(uint32_t* __restrict__ evals, int* __restrict_
 // Every piece is a multiple of 4 bytes; the message is addressed in big-endian 32-bit words.
 struct CellMsg {
   const uint32_t* commitments;   // 12 words each
+  const uint32_t* uniq;          // NULL: commitment j is commitments[j]; else it is the commitment of cell uniq[j]
   const uint32_t* commitment_indices;
   const uint64_t* cell_indices;
   const uint32_t* cells;         // 512 words each
@@ -113,6 +115,17 @@ struct CellMsg {
   uint32_t head[12];
   unsigned long long n_commitments, n_cells;
   int le;                        // little-endian integers (MODE_CKZG_LE)
+  __host__ __device__ static uint32_t bswap(uint32_t v) { return (v >> 24) | ((v >> 8) & 0xff00u) | ((v << 8) & 0xff0000u) | (v << 24); }
+  // domain || u64(4096) || u64(64) || u64(n_commitments) || u64(n_cells), from n_commitments / n_cells / le
+  __host__ __device__ void set_head() {
+    const uint32_t dom[4] = {0x52434b5au, 0x47434241u, 0x5443485fu, 0x5f56315fu};   // "RCKZGCBATCH__V1_"
+    for (int i = 0; i < 4; i++) head[i] = dom[i];
+    const unsigned long long v[4] = {4096ull, (unsigned long long)CELL_ELEMS, n_commitments, n_cells};
+    for (int i = 0; i < 4; i++) {
+      if (le) { head[4 + 2 * i] = bswap((uint32_t)v[i]); head[5 + 2 * i] = bswap((uint32_t)(v[i] >> 32)); }
+      else { head[4 + 2 * i] = (uint32_t)(v[i] >> 32); head[5 + 2 * i] = (uint32_t)v[i]; }
+    }
+  }
   __device__ __forceinline__ void u64_words(uint32_t* out2, unsigned long long v) const {
     if (le) { out2[0] = bswap32((uint32_t)v); out2[1] = bswap32((uint32_t)(v >> 32)); }
     else { out2[0] = (uint32_t)(v >> 32); out2[1] = (uint32_t)v; }
@@ -121,7 +134,10 @@ struct CellMsg {
   __device__ __forceinline__ uint32_t word(unsigned long long wi) const {
     if (wi < 12) return head[wi];
     wi -= 12;
-    if (wi < 12ull * n_commitments) return bswap32(__ldg(commitments + wi));
+    if (wi < 12ull * n_commitments) {
+      if (!uniq) return bswap32(__ldg(commitments + wi));
+      return bswap32(__ldg(commitments + (size_t)__ldg(uniq + wi / 12) * 12 + wi % 12));
+    }
     wi -= 12ull * n_commitments;
     const unsigned long long kk = wi / 528;
     const uint32_t o = (uint32_t)(wi % 528);
@@ -135,8 +151,8 @@ struct CellMsg {
   }
 };
 
-__global__ void __launch_bounds__(32) cell_batch_challenge_kernel(uint32_t* __restrict__ r_out, CellMsg msg) {
-  __shared__ uint32_t wk[64 * 32];
+// r = SHA-256(message) mod r (canonical limbs) by one warp; wk: 64 x 32 words of shared memory
+__device__ void cell_challenge_warp(uint32_t* __restrict__ r_out, const CellMsg& msg, uint32_t* wk) {
   const int lane = threadIdx.x;
   const unsigned long long words = msg.total_words();
   const int nfull = (int)(words / 16);
@@ -162,19 +178,38 @@ __global__ void __launch_bounds__(32) cell_batch_challenge_kernel(uint32_t* __re
   for (int i = 0; i < 8; i++) r_out[i] = r.l[i];
 }
 
+__global__ void __launch_bounds__(32) cell_batch_challenge_kernel(uint32_t* __restrict__ r_out, CellMsg msg) {
+  __shared__ uint32_t wk[64 * 32];
+  cell_challenge_warp(r_out, msg, wk);
+}
+
 // ------------------------------------------------------------------ scalars of the two MSMs
 // One warp per cell: a = IDFT_64 of the cell's evaluations (given in bit-reversed order), coefficient m of the
 // interpolation polynomial = a_m h^-m / 64; weighted by r^k and written to wcoef[k][m] (Montgomery).
 // Lane 0 also writes r^k (rpow, canonical) and r^k h^64 (scalars_b[k], canonical).
-__global__ void __launch_bounds__(32) cell_interp_kernel(Fr* __restrict__ wcoef, uint32_t* __restrict__ rpow, uint32_t* __restrict__ scalars_b,
+// BATCHED: cell kq belongs to batch b = cell_batch[kq] with cells [boff[b], boff[b + 1]) and challenge r_canon[b]; k is
+// its index inside the batch, and r^k / r^k h^64 go to terms base + k / base + n_b + k of the batch's MSM segments
+// (rpow == scalars_b: the term scalars of cell_batch_term_base).
+template <bool BATCHED>
+__global__ void __launch_bounds__(32) cell_interp_kernel(Fr* __restrict__ wcoef, uint32_t* rpow, uint32_t* scalars_b,
                                                         const uint32_t* __restrict__ evals, const uint64_t* __restrict__ cell_indices,
-                                                        const uint32_t* __restrict__ r_canon, const Fr* __restrict__ tw) {
+                                                        const uint32_t* __restrict__ r_canon, const Fr* __restrict__ tw,
+                                                        const int* __restrict__ cell_batch, const int* __restrict__ boff) {
   __shared__ uint32_t sm[8 * 64];
   const int kq = blockIdx.x, lane = threadIdx.x;
+  uint32_t k = (uint32_t)kq;
+  size_t ia = (size_t)kq, ib = (size_t)kq;
+  if (BATCHED) {
+    const int b = cell_batch[kq], s0 = boff[b], n = boff[b + 1] - s0;
+    k = (uint32_t)(kq - s0);
+    r_canon += (size_t)b * 8;
+    ia = cell_batch_term_base(s0, b) + k;
+    ib = ia + (size_t)n;
+  }
   const uint32_t hexp = brp7((uint32_t)cell_indices[kq] & 127u);   // h_k = w8192^brp7(cell index)
   Fr r;
   for (int i = 0; i < 8; i++) r.l[i] = r_canon[i];
-  const Fr rk = fr_pow_small(fr_to_mont(r), (uint32_t)kq);
+  const Fr rk = fr_pow_small(fr_to_mont(r), k);
   for (int i = lane; i < 64; i += 32) {
     Fr v;
     for (int l = 0; l < 8; l++) v.l[l] = evals[((size_t)kq * 64 + i) * 8 + l];
@@ -189,7 +224,7 @@ __global__ void __launch_bounds__(32) cell_interp_kernel(Fr* __restrict__ wcoef,
   }
   if (lane == 0) {
     const Fr a = fr_from_mont(rk), b = fr_from_mont(fr_mul(rk, tw[64u * hexp]));
-    for (int l = 0; l < 8; l++) { rpow[(size_t)kq * 8 + l] = a.l[l]; scalars_b[(size_t)kq * 8 + l] = b.l[l]; }
+    for (int l = 0; l < 8; l++) { rpow[ia * 8 + l] = a.l[l]; scalars_b[ib * 8 + l] = b.l[l]; }
   }
 }
 
@@ -215,6 +250,185 @@ __global__ void __launch_bounds__(128) cell_verify_finish_kernel(uint32_t* __res
     }
     for (int l = 0; l < 8; l++) scalars_b[((size_t)n + i) * 8 + l] = acc.l[l];
   }
+}
+
+// ------------------------------------------------------------------ many independent batches per call
+// A pass holds nb batches; batch b is the pass's cells [boff[b], boff[b + 1]).  Every per-cell array is indexed by the
+// pass-local cell, every per-batch array by the pass-local batch.
+
+// One block per batch: folds the per-cell statuses (parse | proof decode | commitment decode, 3 x n_cells) and the
+// index range into the batch's status, and deduplicates its commitments in order of first appearance:
+// cidx[k] = index of cell k's commitment among the batch's distinct ones, uniq[boff[b] + j] = the first cell holding
+// distinct commitment j, nc[b] = their number.  first: n_cells ints of scratch.
+__global__ void __launch_bounds__(256) cell_batches_prepare_kernel(int* __restrict__ bstatus, int* __restrict__ nc, uint32_t* __restrict__ cidx,
+                                                                  uint32_t* __restrict__ uniq, int* __restrict__ first, int* __restrict__ cell_batch,
+                                                                  const uint8_t* __restrict__ commit48, const uint64_t* __restrict__ cell_indices,
+                                                                  const int* __restrict__ cell_status, int n_cells, const int* __restrict__ boff, int mode) {
+  __shared__ int n_uniq;
+  const int b = blockIdx.x, s0 = boff[b], e = boff[b + 1];
+  if (threadIdx.x == 0) n_uniq = 0;
+  bool fail = false;
+  for (int g = s0 + threadIdx.x; g < e; g += blockDim.x) {
+    cell_batch[g] = b;
+    fail = fail || cell_indices[g] >= (uint64_t)N_CELLS || cell_status[g] || cell_status[n_cells + g] || cell_status[2 * n_cells + g];
+    const uint4* mine = reinterpret_cast<const uint4*>(commit48 + (size_t)g * 48);
+    const uint4 m0 = mine[0], m1 = mine[1], m2 = mine[2];
+    int f = g;
+    for (int j = s0; j < g; j++) {
+      const uint4* o = reinterpret_cast<const uint4*>(commit48 + (size_t)j * 48);
+      const uint4 o0 = o[0];
+      if (o0.x != m0.x || o0.y != m0.y || o0.z != m0.z || o0.w != m0.w) continue;
+      const uint4 o1 = o[1], o2 = o[2];
+      if (o1.x == m1.x && o1.y == m1.y && o1.z == m1.z && o1.w == m1.w && o2.x == m2.x && o2.y == m2.y && o2.z == m2.z && o2.w == m2.w) { f = j; break; }
+    }
+    first[g] = f;
+  }
+  fail = __syncthreads_or(fail);
+  int mine_uniq = 0;
+  for (int g = s0 + threadIdx.x; g < e; g += blockDim.x) {
+    const int f = first[g];
+    uint32_t cnt = 0;
+    for (int j = s0; j < f; j++) cnt += first[j] == j;
+    cidx[g] = cnt;
+    if (f == g) { uniq[s0 + cnt] = (uint32_t)g; mine_uniq++; }
+  }
+  if (mine_uniq) atomicAdd(&n_uniq, mine_uniq);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    nc[b] = n_uniq;
+    bstatus[b] = fail ? (mode == 0 ? 2 : 1) : 0;   // C_KZG_ERROR in MODE_REFERENCE, C_KZG_BADARGS in the c-kzg modes
+  }
+}
+
+// One warp per batch: its challenge r_b over the batch's own message (the single call's), zeros for an empty batch.
+__global__ void __launch_bounds__(32) cell_batches_challenge_kernel(uint32_t* __restrict__ rs, const uint32_t* __restrict__ commit, const uint32_t* __restrict__ uniq,
+                                                                   const uint32_t* __restrict__ cidx, const uint64_t* __restrict__ cell_indices,
+                                                                   const uint32_t* __restrict__ cells, const uint32_t* __restrict__ proofs,
+                                                                   const int* __restrict__ nc, const int* __restrict__ boff, int le) {
+  __shared__ uint32_t wk[64 * 32];
+  const int b = blockIdx.x, s0 = boff[b], n = boff[b + 1] - s0;
+  if (n == 0) {
+    if (threadIdx.x < 8) rs[(size_t)b * 8 + threadIdx.x] = 0;
+    return;
+  }
+  CellMsg m;
+  m.commitments = commit;
+  m.uniq = uniq + s0;
+  m.commitment_indices = cidx + s0;
+  m.cell_indices = cell_indices + s0;
+  m.cells = cells + (size_t)s0 * 512;
+  m.proofs = proofs + (size_t)s0 * 12;
+  m.n_commitments = (unsigned long long)nc[b];
+  m.n_cells = (unsigned long long)n;
+  m.le = le;
+  m.set_head();
+  cell_challenge_warp(rs + (size_t)b * 8, m, wk);
+}
+
+// One block per batch: the scalars of the monomial terms (minus the summed interpolation coefficients) and of the
+// commitment slots (w_j = sum of r^k over the batch's cells with commitment j, 0 for the unused slots j >= nc).
+__global__ void __launch_bounds__(128) cell_batches_finish_kernel(uint32_t* __restrict__ scal, const Fr* __restrict__ wcoef, const uint32_t* __restrict__ cidx,
+                                                                 const int* __restrict__ nc, const int* __restrict__ boff) {
+  const int b = blockIdx.x, s0 = boff[b], n = boff[b + 1] - s0, t = threadIdx.x;
+  const size_t base = cell_batch_term_base(s0, b);
+  if (t < 64) {
+    Fr acc = fr_zero();
+    for (int k = 0; k < n; k++) acc = fr_add(acc, wcoef[(size_t)(s0 + k) * 64 + t]);
+    const Fr v = fr_from_mont(fr_neg(acc));
+    for (int l = 0; l < 8; l++) scal[(base + 3 * (size_t)n + t) * 8 + l] = v.l[l];
+  }
+  const int nb_c = nc[b];
+  for (int j = t; j < n; j += blockDim.x) {
+    Fr acc = fr_zero();
+    if (j < nb_c) {
+      for (int k = 0; k < n; k++) {
+        if ((int)cidx[s0 + k] == j) {
+          Fr v;
+          for (int l = 0; l < 8; l++) v.l[l] = scal[(base + k) * 8 + l];   // r^k, canonical
+          acc = fr_add(acc, v);
+        }
+      }
+    }
+    for (int l = 0; l < 8; l++) scal[(base + 2 * (size_t)n + j) * 8 + l] = acc.l[l];
+  }
+}
+
+// Segmented variable-base MSM, pass 1: one thread per (point, scalar) term, [s]P by the GLV split (every point passed
+// the G1 check or is a monomial SRS point).  The batch of term t is found by bisection over the term bases.
+__global__ void __launch_bounds__(128) cell_segmsm_terms_kernel(G1Xyzz* __restrict__ out, const uint32_t* __restrict__ scal, const G1Affine* __restrict__ proof_pts,
+                                                               const G1Affine* __restrict__ commit_pts, const G1Affine* __restrict__ mono,
+                                                               const uint32_t* __restrict__ uniq, const int* __restrict__ nc, const int* __restrict__ boff,
+                                                               int nb, long n_terms) {
+  const long t = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_terms) return;
+  int lo = 0, hi = nb - 1;   // the last batch whose base is <= t
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if ((long)cell_batch_term_base(boff[mid], mid) <= t) lo = mid;
+    else hi = mid - 1;
+  }
+  const int b = lo, s0 = boff[b], n = boff[b + 1] - s0;
+  const long u = t - (long)cell_batch_term_base(s0, b);
+  G1Affine p;
+  bool use = true;
+  if (u < n) p = proof_pts[s0 + u];                       // LHS: r^k pi_k
+  else if (u < 2 * n) p = proof_pts[s0 + u - n];          // RHS: r^k h_k^64 pi_k
+  else if (u < 3 * n) {                                   // RHS: w_j C_j
+    const int j = (int)(u - 2 * n);
+    use = j < nc[b];
+    p = commit_pts[use ? uniq[s0 + j] : 0];
+  } else p = mono[u - 3 * n];                             // RHS: -s_m [tau^m]G
+  uint32_t k8[8];
+  for (int l = 0; l < 8; l++) k8[l] = scal[(size_t)t * 8 + l];
+  out[t] = use ? g1_mul_scalar_glv(p, k8) : xyzz_inf();
+}
+
+// pass 2: one block per segment (2b: LHS of batch b, 2b + 1: RHS), affine big-endian into the batch's 288-byte
+// partial: LHS at 0, 96 zero bytes, RHS at 192, infinity as zeros (what batch_final_kernel reads)
+__global__ void __launch_bounds__(128) cell_segmsm_reduce_kernel(uint8_t* __restrict__ out288, const G1Xyzz* __restrict__ terms, const int* __restrict__ boff) {
+  __shared__ G1Xyzz sh[128];
+  const int b = blockIdx.x >> 1, rhs = blockIdx.x & 1, s0 = boff[b], n = boff[b + 1] - s0;
+  const size_t base = cell_batch_term_base(s0, b);
+  const size_t lo = rhs ? base + n : base, hi = rhs ? base + 3 * (size_t)n + 64 : base + n;
+  G1Xyzz acc = xyzz_inf();
+  for (size_t i = lo + threadIdx.x; i < hi; i += blockDim.x) xyzz_add_ni(acc, terms[i]);
+  sh[threadIdx.x] = acc;
+  __syncthreads();
+  for (int d = blockDim.x / 2; d > 0; d >>= 1) {
+    if ((int)threadIdx.x < d) {
+      G1Xyzz a = sh[threadIdx.x];
+      xyzz_add_ni(a, sh[threadIdx.x + d]);
+      sh[threadIdx.x] = a;
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    uint8_t* o = out288 + (size_t)b * 288 + (rhs ? 192 : 0);
+    const G1Affine a = xyzz_to_affine(sh[0]);
+    if (g1a_is_inf(a)) {
+      for (int k = 0; k < 96; k++) o[k] = 0;
+    } else {
+      fp_canon_to_be48(o, fp_from_mont(a.x));
+      fp_canon_to_be48(o + 48, fp_from_mont(a.y));
+    }
+    if (!rhs)
+      for (int k = 96; k < 192; k++) o[k] = 0;
+  }
+}
+
+__global__ void fill_int_kernel(int* __restrict__ out, int v, int n) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = v;
+}
+
+// verdicts: a failed batch is false, an empty one true, any other the pairing check's
+__global__ void cell_batches_fold_kernel(int* __restrict__ ok, int* __restrict__ status, const int* __restrict__ pair_ok, const int* __restrict__ bstatus,
+                                         const int* __restrict__ boff, int nb) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= nb) return;
+  const int st = bstatus[b];
+  ok[b] = st ? 0 : (boff[b + 1] == boff[b] ? 1 : (pair_ok[b] != 0));
+  if (status) status[b] = st;
 }
 
 // ------------------------------------------------------------------ recovery
@@ -389,17 +603,8 @@ void launch_cell_batch_challenge(void* d_r, const void* d_commitments48, int n_c
   m.n_commitments = (unsigned long long)n_commitments;
   m.n_cells = (unsigned long long)n_cells;
   m.le = mode == 1 ? 1 : 0;
-  const char dom[17] = "RCKZGCBATCH__V1_";
-  for (int i = 0; i < 4; i++)
-    m.head[i] = ((uint32_t)(uint8_t)dom[4 * i] << 24) | ((uint32_t)(uint8_t)dom[4 * i + 1] << 16) | ((uint32_t)(uint8_t)dom[4 * i + 2] << 8) | (uint32_t)(uint8_t)dom[4 * i + 3];
-  auto put = [&](int at, unsigned long long v) {
-    if (m.le) { m.head[at] = __builtin_bswap32((uint32_t)v); m.head[at + 1] = __builtin_bswap32((uint32_t)(v >> 32)); }
-    else { m.head[at] = (uint32_t)(v >> 32); m.head[at + 1] = (uint32_t)v; }
-  };
-  put(4, 4096);
-  put(6, CELL_ELEMS);
-  put(8, m.n_commitments);
-  put(10, m.n_cells);
+  m.uniq = nullptr;
+  m.set_head();
   LW_SAME_CARVEOUT(cell_batch_challenge_kernel);
   cell_batch_challenge_kernel<<<1, 32, 0, st>>>((uint32_t*)d_r, m);
   count_launch();
@@ -408,10 +613,10 @@ void launch_cell_batch_challenge(void* d_r, const void* d_commitments48, int n_c
 void launch_cell_verify_scalars(void* d_wcoef, void* d_rpow, void* d_scalars_b, const void* d_evals, const uint64_t* d_cell_indices,
                                 const uint32_t* d_commitment_indices, int n_cells, int n_commitments, const void* d_r, const void* d_tw8192, cudaStream_t st) {
   if (n_cells <= 0) return;
-  LW_SAME_CARVEOUT(cell_interp_kernel);
+  LW_SAME_CARVEOUT(cell_interp_kernel<false>);
   LW_SAME_CARVEOUT(cell_verify_finish_kernel);
-  cell_interp_kernel<<<n_cells, 32, 0, st>>>((Fr*)d_wcoef, (uint32_t*)d_rpow, (uint32_t*)d_scalars_b, (const uint32_t*)d_evals, d_cell_indices,
-                                            (const uint32_t*)d_r, (const Fr*)d_tw8192);
+  cell_interp_kernel<false><<<n_cells, 32, 0, st>>>((Fr*)d_wcoef, (uint32_t*)d_rpow, (uint32_t*)d_scalars_b, (const uint32_t*)d_evals, d_cell_indices,
+                                                   (const uint32_t*)d_r, (const Fr*)d_tw8192, nullptr, nullptr);
   cell_verify_finish_kernel<<<1, 128, 0, st>>>((uint32_t*)d_scalars_b, (const Fr*)d_wcoef, (const uint32_t*)d_rpow, d_commitment_indices, n_cells, n_commitments);
   count_launch(2);
 }
@@ -428,6 +633,61 @@ void launch_cell_recover(void* d_coef, int* d_status, void* d_ws, const void* d_
   }
   cell_recover_kernel<<<n_blobs, REC_THREADS, REC_SMEM, st>>>((Fr*)d_coef, d_status, (Fr*)d_ws, (const uint32_t*)d_evals, d_cell_status, d_cell_indices,
                                                              n_cells, mode, (const Fr*)d_tw8192);
+  count_launch();
+}
+
+void launch_cell_batches_prepare(int* d_bstatus, int* d_nc, uint32_t* d_cidx, uint32_t* d_uniq, int* d_first, int* d_cell_batch, const void* d_commit48,
+                                 const uint64_t* d_cell_indices, const int* d_cell_status, int n_cells, const int* d_boff, int nb, int mode, cudaStream_t st) {
+  if (nb <= 0) return;
+  cell_batches_prepare_kernel<<<nb, 256, 0, st>>>(d_bstatus, d_nc, d_cidx, d_uniq, d_first, d_cell_batch, (const uint8_t*)d_commit48, d_cell_indices, d_cell_status,
+                                                  n_cells, d_boff, mode);
+  count_launch();
+}
+
+void launch_cell_batches_challenge(void* d_rs, const void* d_commit48, const uint32_t* d_uniq, const uint32_t* d_cidx, const uint64_t* d_cell_indices,
+                                   const void* d_cells, const void* d_proofs48, const int* d_nc, const int* d_boff, int nb, int mode, cudaStream_t st) {
+  if (nb <= 0) return;
+  LW_SAME_CARVEOUT(cell_batches_challenge_kernel);
+  cell_batches_challenge_kernel<<<nb, 32, 0, st>>>((uint32_t*)d_rs, (const uint32_t*)d_commit48, d_uniq, d_cidx, d_cell_indices, (const uint32_t*)d_cells,
+                                                   (const uint32_t*)d_proofs48, d_nc, d_boff, mode == 1 ? 1 : 0);
+  count_launch();
+}
+
+void launch_cell_batches_scalars(void* d_wcoef, void* d_scal, const void* d_evals, const uint64_t* d_cell_indices, const uint32_t* d_cidx, const int* d_nc,
+                                 const int* d_cell_batch, const int* d_boff, int n_cells, int nb, const void* d_rs, const void* d_tw8192, cudaStream_t st) {
+  if (nb <= 0) return;
+  if (n_cells > 0) {
+    LW_SAME_CARVEOUT(cell_interp_kernel<true>);
+    cell_interp_kernel<true><<<n_cells, 32, 0, st>>>((Fr*)d_wcoef, (uint32_t*)d_scal, (uint32_t*)d_scal, (const uint32_t*)d_evals, d_cell_indices,
+                                                    (const uint32_t*)d_rs, (const Fr*)d_tw8192, d_cell_batch, d_boff);
+    count_launch();
+  }
+  cell_batches_finish_kernel<<<nb, 128, 0, st>>>((uint32_t*)d_scal, (const Fr*)d_wcoef, d_cidx, d_nc, d_boff);
+  count_launch();
+}
+
+size_t cell_segmsm_terms(int n_cells, int nb) { return cell_batch_term_base(n_cells, nb); }
+
+void launch_cell_segmsm(void* d_out288, void* d_terms, const void* d_scal, const void* d_proof_aff, const void* d_commit_aff, const void* d_mono_aff,
+                        const uint32_t* d_uniq, const int* d_nc, const int* d_boff, int n_cells, int nb, cudaStream_t st) {
+  if (nb <= 0) return;
+  const long n_terms = (long)cell_segmsm_terms(n_cells, nb);
+  cell_segmsm_terms_kernel<<<(unsigned)((n_terms + 127) / 128), 128, 0, st>>>((G1Xyzz*)d_terms, (const uint32_t*)d_scal, (const G1Affine*)d_proof_aff,
+                                                                             (const G1Affine*)d_commit_aff, (const G1Affine*)d_mono_aff, d_uniq, d_nc, d_boff,
+                                                                             nb, n_terms);
+  cell_segmsm_reduce_kernel<<<2 * nb, 128, 0, st>>>((uint8_t*)d_out288, (const G1Xyzz*)d_terms, d_boff);
+  count_launch(2);
+}
+
+void launch_fill_int(int* d_out, int value, int n, cudaStream_t st) {
+  if (n <= 0) return;
+  fill_int_kernel<<<(n + 127) / 128, 128, 0, st>>>(d_out, value, n);
+  count_launch();
+}
+
+void launch_cell_batches_fold(int* d_ok, int* d_status, const int* d_pair_ok, const int* d_bstatus, const int* d_boff, int nb, cudaStream_t st) {
+  if (nb <= 0) return;
+  cell_batches_fold_kernel<<<(nb + 127) / 128, 128, 0, st>>>(d_ok, d_status, d_pair_ok, d_bstatus, d_boff, nb);
   count_launch();
 }
 

@@ -123,6 +123,8 @@ void launch_batch_partials(void* d_partial288, const void* d_r, const void* d_c_
 size_t batch_partials_scratch_bytes(int n_local);
 // sum n_ranks partial triples, then e(rhs, g2_0) * e(-proof_lincomb, g2_1) == 1
 void launch_batch_final(int* d_ok, const void* d_partials288, int n_ranks, const void* d_prep0, const void* d_prep1, cudaStream_t st);
+// n_checks independent checks, one block each: d_ok[i] from the 288 bytes at d_partials288 + 288 i
+void launch_batch_final_each(int* d_ok, const void* d_partials288, int n_checks, const void* d_prep0, const void* d_prep1, cudaStream_t st);
 
 // ---- MODE_CKZG_LE (le.cu)
 void launch_write_generator(void* d_out, cudaStream_t st);                 // the G1 generator, affine Montgomery

@@ -73,4 +73,32 @@ void launch_cell_recover(void* d_coef, int* d_status, void* d_ws, const void* d_
 // coefficient form (Montgomery) -> cells (both halves computed by FFT) -- the tail of launch_cell_poly for callers that already hold coefficients
 void launch_cell_coef_to_cells(void* d_cells, const void* d_coef, int n, int mode, const void* d_tw8192, cudaStream_t st);
 
+// ---- many independent verify_cell_kzg_proof_batch checks per launch sequence (cells_verify.cu).  A pass holds nb
+// batches: batch b is the pass's cells [d_boff[b], d_boff[b + 1]); every per-cell array is indexed by the pass's cell,
+// every per-batch one by the pass's batch.  Each batch owns two MSM segments over consecutive terms starting at
+// cell_batch_term_base(first cell, b): n_b LHS terms r^k pi_k, then the RHS: n_b terms r^k h_k^64 pi_k, n_b commitment
+// slots (w_j C_j for j < nc_b, scalar 0 above) and 64 monomial terms -s_m [tau^m]G.
+__host__ __device__ inline size_t cell_batch_term_base(int first_cell, int b) { return 3 * (size_t)first_cell + 64 * (size_t)b; }
+size_t cell_segmsm_terms(int n_cells, int nb);
+// d_cell_status: 3 x n_cells (parse | proof decode | commitment decode).  d_bstatus[b] = 0, or 1 / 2 (C_KZG_BADARGS /
+// C_KZG_ERROR: mode 0 -> 2) when a cell index is >= 128 or a status is set; commitments deduplicated per batch in order of
+// first appearance: d_cidx[k] (index among the batch's distinct commitments), d_uniq[d_boff[b] + j] (first cell of
+// distinct commitment j), d_nc[b]; d_cell_batch[k] = b; d_first: n_cells ints of scratch
+void launch_cell_batches_prepare(int* d_bstatus, int* d_nc, uint32_t* d_cidx, uint32_t* d_uniq, int* d_first, int* d_cell_batch, const void* d_commit48,
+                                 const uint64_t* d_cell_indices, const int* d_cell_status, int n_cells, const int* d_boff, int nb, int mode, cudaStream_t st);
+// one warp per batch: r_b (canonical, 8 u32 each) over the batch's message as launch_cell_batch_challenge; zeros if empty
+void launch_cell_batches_challenge(void* d_rs, const void* d_commit48, const uint32_t* d_uniq, const uint32_t* d_cidx, const uint64_t* d_cell_indices,
+                                   const void* d_cells, const void* d_proofs48, const int* d_nc, const int* d_boff, int nb, int mode, cudaStream_t st);
+// the term scalars (canonical, cell_segmsm_terms(n_cells, nb) x 8 u32); d_wcoef: n_cells x 64 x 32 B of scratch
+void launch_cell_batches_scalars(void* d_wcoef, void* d_scal, const void* d_evals, const uint64_t* d_cell_indices, const uint32_t* d_cidx, const int* d_nc,
+                                 const int* d_cell_batch, const int* d_boff, int n_cells, int nb, const void* d_rs, const void* d_tw8192, cudaStream_t st);
+// segmented variable-base MSM: batch b's 288-byte partial (LHS at 0, 96 zero bytes, RHS at 192; big-endian affine,
+// infinity as zeros); d_terms: cell_segmsm_terms(n_cells, nb) x 192 B of scratch
+void launch_cell_segmsm(void* d_out288, void* d_terms, const void* d_scal, const void* d_proof_aff, const void* d_commit_aff, const void* d_mono_aff,
+                        const uint32_t* d_uniq, const int* d_nc, const int* d_boff, int n_cells, int nb, cudaStream_t st);
+// d_ok[b] = 0 if d_bstatus[b] != 0, 1 if batch b is empty, else d_pair_ok[b]; d_status[b] = d_bstatus[b] (d_status may be NULL)
+// d_out[0, n) = value
+void launch_fill_int(int* d_out, int value, int n, cudaStream_t st);
+void launch_cell_batches_fold(int* d_ok, int* d_status, const int* d_pair_ok, const int* d_bstatus, const int* d_boff, int nb, cudaStream_t st);
+
 }  // namespace lw

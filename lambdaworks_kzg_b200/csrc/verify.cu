@@ -333,6 +333,8 @@ __global__ void __launch_bounds__(LW_PAIR_LANES) batch_final_kernel(int* __restr
   __shared__ WarpPairingMem sh_m;
   __shared__ G1Affine sh_pts[2];
   const int lane = threadIdx.x;
+  partials += (size_t)blockIdx.x * n_ranks * 288;   // one check per block (launch_batch_final_each)
+  ok_out += blockIdx.x;
   if (lane < 2) {
     G1Xyzz acc = xyzz_inf();
     for (int r = 0; r < n_ranks; r++) {
@@ -439,6 +441,11 @@ void launch_batch_partials(void* d_partial288, const void* d_r, const void* d_c_
 }
 void launch_batch_final(int* d_ok, const void* d_partials288, int n_ranks, const void* d_prep0, const void* d_prep1, cudaStream_t st) {
   batch_final_kernel<<<1, LW_PAIR_LANES, 0, st>>>(d_ok, (const uint8_t*)d_partials288, n_ranks, (const G2Prepared*)d_prep0, (const G2Prepared*)d_prep1);
+  count_launch();
+}
+void launch_batch_final_each(int* d_ok, const void* d_partials288, int n_checks, const void* d_prep0, const void* d_prep1, cudaStream_t st) {
+  if (n_checks <= 0) return;
+  batch_final_kernel<<<n_checks, LW_PAIR_LANES, 0, st>>>(d_ok, (const uint8_t*)d_partials288, 1, (const G2Prepared*)d_prep0, (const G2Prepared*)d_prep1);
   count_launch();
 }
 }  // namespace lw

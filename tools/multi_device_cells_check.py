@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """lwkzg_set_devices for the PeerDAS calls: ONE process, one C call, every visible GPU.  The sharded cell batch and the
-sharded recovery batch must return the bytes of the single-device calls (MODE_DENEB: the replicas get the monomial SRS
-from the primary context).  Prints MULTI_DEVICE_CELLS_OK on success."""
+sharded recovery batch must return the bytes of the single-device calls, and the sharded many-batch cell verification
+their verdicts, statuses and challenges (MODE_DENEB: the replicas get the monomial SRS from the primary context).  Prints MULTI_DEVICE_CELLS_OK on success."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -42,11 +42,31 @@ idx = keep * n
 sel = b"".join(c1[(b * 128 + i) * 2048: (b * 128 + i + 1) * 2048] for b in range(n) for i in keep)
 rc1, rp1 = recover("1 device ", idx, sel)
 assert rc1 == c1 and rp1 == p1, "recovered outputs differ from the computed ones"
+# one batch per column over the first 48 blobs, plus a batch whose proof is swapped and one with an index >= 128
+coms, st = lw.blob_to_kzg_commitment_batch(blobs[: 48 * 131072], 48, s)
+assert not any(st)
+vb = [([coms[b] for b in range(48)], [col] * 48, [c1[(b * 128 + col) * 2048: (b * 128 + col + 1) * 2048] for b in range(48)],
+       [p1[(b * 128 + col) * 48: (b * 128 + col + 1) * 48] for b in range(48)]) for col in range(128)]
+vb[5] = (vb[5][0], vb[5][1], vb[5][2], [vb[5][3][1], vb[5][3][0]] + vb[5][3][2:])
+vb[77] = (vb[77][0], [128] + vb[77][1][1:], vb[77][2], vb[77][3])
+
+
+def verify(tag):
+    t0 = time.perf_counter()
+    oks, sts = lw.verify_cell_kzg_proof_batches(vb, s)
+    dt = time.perf_counter() - t0
+    print("%s: verified %d cell batches in %.1f ms" % (tag, len(vb), dt * 1e3), flush=True)
+    return oks, sts, lw.debug_cell_batch_challenges(len(vb), s)
+
+
+v1 = verify("1 device ")
+assert v1[0] == [b not in (5, 77) for b in range(128)] and v1[1] == [lw.C_KZG_BADARGS if b == 77 else 0 for b in range(128)]
 lw.set_devices(list(range(g)))
 run("%d devices (first call builds the replicas)" % g)
 c2, p2 = run("%d devices" % g)
 assert c1 == c2 and p1 == p2, "multi-device cell outputs differ from the single-device outputs"
 rc2, rp2 = recover("%d devices" % g, idx, sel)
 assert rc2 == rc1 and rp2 == rp1, "multi-device recovery outputs differ from the single-device outputs"
+assert verify("%d devices" % g) == v1, "multi-device cell verification differs from the single-device verdicts, statuses or challenges"
 lw.set_devices([])
 print("MULTI_DEVICE_CELLS_OK", flush=True)
