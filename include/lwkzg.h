@@ -293,9 +293,34 @@ C_KZG_RET lwkzg_verify_cell_kzg_proof_batches(bool *ok, const Bytes48 *commitmen
 C_KZG_RET lwkzg_verify_cell_kzg_proof_batches_device(void *d_ok, const void *d_commitments, const void *d_cell_indices,
                                                      const void *d_cells, const void *d_proofs, const uint64_t *offsets,
                                                      size_t n_batches, const KZGSettings *s, void *stream, void *d_status);
-/* Test hook: the challenge r_b of every non-empty batch that the last call of either form on these settings derived,
- * 32 little-endian bytes each (as lwkzg_debug_batch_challenge); zeros for empty batches.  n_batches must not exceed
- * the last call's. */
+/* additive: K = n_batches checks of blob transactions as the EIP-7594 network wrapper carries them (blobs, one
+ * commitment per blob, CELLS_PER_EXT_BLOB cell proofs per blob, no cells).  Batch b is blobs [offsets[b], offsets[b+1])
+ * (typically one transaction); offsets: K + 1 host integers, offsets[0] == 0, non-decreasing.  commitments: one per
+ * blob; cell_proofs: 128 per blob, blob-major, proof j belongs to cell j.  ok[b] / status[b] (may be NULL) are exactly
+ * what a caller gets from compute_cells_and_kzg_proofs on every blob of the batch -- (false, that code) if one fails --
+ * and otherwise from ONE verify_cell_kzg_proof_batch over the batch's blobs in order: blob i's commitment 128 times, cell
+ * indices 0..127, its cells and its 128 proofs.  So each batch has its own challenge over its commitments
+ * deduplicated in order of first appearance, an empty batch verifies, and a blob word >= r (modes 1 and 2) or a
+ * commitment or proof that does not decode or is not in G1 fails its own batch only: C_KZG_BADARGS in modes 1 and 2,
+ * C_KZG_ERROR in mode 0.  Whole-call errors: n_batches == 0 returns C_KZG_OK and writes nothing; a NULL required
+ * pointer, offsets that do not start at 0 or decrease, or more than 2^24 cells (offsets[K] > 131072 blobs) return
+ * C_KZG_BADARGS; settings without the monomial SRS return C_KZG_ERROR; with status == NULL the first failing batch's
+ * code is returned (ok is still filled).  The cells are computed on the GPU and never leave it, each commitment is
+ * decoded once per blob, and the rest runs as lwkzg_verify_cell_kzg_proof_batches: passes of whole batches of at most
+ * "cell_chunk_blobs" blobs (a larger batch gets a pass of its own), sharded over the GPUs after lwkzg_set_devices. */
+C_KZG_RET lwkzg_verify_blob_cell_kzg_proof_batches(bool *ok, const Blob *blobs, const Bytes48 *commitments,
+                                                   const Bytes48 *cell_proofs, const uint64_t *offsets,
+                                                   size_t n_batches, const KZGSettings *s, int *status);
+/* the same with blobs, commitments and cell_proofs in device memory (16-byte aligned); offsets stay on the host.
+ * Asynchronous, ordered after / before work on `stream`; d_ok and d_status are n_batches ints on the device (1 / 0 and
+ * C_KZG_RET values), d_status may be NULL. */
+C_KZG_RET lwkzg_verify_blob_cell_kzg_proof_batches_device(void *d_ok, const void *d_blobs, const void *d_commitments,
+                                                          const void *d_cell_proofs, const uint64_t *offsets,
+                                                          size_t n_batches, const KZGSettings *s, void *stream,
+                                                          void *d_status);
+/* Test hook: the challenge r_b of every non-empty batch that the last lwkzg_verify_cell_kzg_proof_batches[_device] or
+ * lwkzg_verify_blob_cell_kzg_proof_batches[_device] call on these settings derived, 32 little-endian bytes each (as
+ * lwkzg_debug_batch_challenge); zeros for empty batches.  n_batches must not exceed the last call's. */
 C_KZG_RET lwkzg_debug_cell_batch_challenges(uint8_t *out32, size_t n_batches, const KZGSettings *s);
 /* Test hook: intermediate values of the FK20 pipeline for one blob, so a parity test can name the stage that deviates:
  * scalars = the 8192 MSM scalars DFT_128(circulant column b)_j / 128 as 32-byte little-endian integers, at index

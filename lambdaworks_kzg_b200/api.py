@@ -86,6 +86,8 @@ def load_library() -> ctypes.CDLL:
         "lwkzg_recover_cells_and_kzg_proofs_batch_device": [vp, vp, vp, vp, sz, sz, sp, vp, vp],
         "lwkzg_verify_cell_kzg_proof_batches": [bp, vp, vp, vp, vp, vp, sz, sp, ip],
         "lwkzg_verify_cell_kzg_proof_batches_device": [vp, vp, vp, vp, vp, vp, sz, sp, vp, vp],
+        "lwkzg_verify_blob_cell_kzg_proof_batches": [bp, vp, vp, vp, vp, sz, sp, ip],
+        "lwkzg_verify_blob_cell_kzg_proof_batches_device": [vp, vp, vp, vp, vp, sz, sp, vp, vp],
         "lwkzg_debug_cell_batch_challenges": [vp, sz, sp],
         "lwkzg_cell_window_bits": [sp],
         "lwkzg_table_share": [sp],
@@ -575,8 +577,38 @@ def verify_cell_kzg_proof_batches_device(d_ok: int, d_commitments: int, d_cell_i
            "lwkzg_verify_cell_kzg_proof_batches_device")
 
 
+def verify_blob_cell_kzg_proof_batches(batches: Sequence[Tuple[Sequence[bytes], Sequence[bytes], Sequence[bytes]]], s) -> Tuple[List[bool], List[int]]:
+    """K blob-transaction checks in one call.  batches: (blobs, commitments (one per blob), proofs (128 per blob,
+    blob-major)) per batch -> (verdict list, status list): per batch, what compute_cells_and_kzg_proofs on its blobs
+    followed by one verify_cell_kzg_proof_batch over all their cells gives."""
+    k = len(batches)
+    offsets = [0]
+    for bl, com, pr in batches:
+        assert len(bl) == len(com) and len(pr) == CELLS_PER_EXT_BLOB * len(bl)
+        offsets.append(offsets[-1] + len(bl))
+    off = (ctypes.c_uint64 * (k + 1))(*offsets)
+    oks = (ctypes.c_bool * max(1, k))()
+    st = _status_list(k)
+    _check(load_library().lwkzg_verify_blob_cell_kzg_proof_batches(oks, b"".join(_cat(b[0], BYTES_PER_BLOB) for b in batches) or b"\0",
+                                                                   b"".join(_cat(b[1], 48) for b in batches) or b"\0",
+                                                                   b"".join(_cat(b[2], 48) for b in batches) or b"\0", off, k, _sp(s), st),
+           "lwkzg_verify_blob_cell_kzg_proof_batches")
+    return [bool(oks[i]) for i in range(k)], list(st)[:k]
+
+
+def verify_blob_cell_kzg_proof_batches_device(d_ok: int, d_blobs: int, d_commitments: int, d_proofs: int, offsets: Sequence[int], s, stream: int = 0,
+                                              d_status: int = 0):
+    """All buffers are raw device addresses except offsets (K + 1 host integers, in blobs); d_ok and d_status are K
+    int32 each.  Asynchronous on `stream`."""
+    k = len(offsets) - 1
+    off = (ctypes.c_uint64 * max(1, k + 1))(*offsets)
+    _check(load_library().lwkzg_verify_blob_cell_kzg_proof_batches_device(d_ok or None, d_blobs or None, d_commitments or None, d_proofs or None, off, k,
+                                                                          _sp(s), stream or None, d_status or None),
+           "lwkzg_verify_blob_cell_kzg_proof_batches_device")
+
+
 def debug_cell_batch_challenges(n_batches: int, s) -> List[int]:
-    """The challenges r_b the last verify_cell_kzg_proof_batches[_device] call derived (0 for empty batches; test hook)."""
+    """The challenges r_b the last verify_[blob_]cell_kzg_proof_batches[_device] call derived (0 for empty batches; test hook)."""
     out = ctypes.create_string_buffer(32 * max(1, n_batches))
     _check(load_library().lwkzg_debug_cell_batch_challenges(out, n_batches, _sp(s)), "lwkzg_debug_cell_batch_challenges")
     return [int.from_bytes(out.raw[32 * i: 32 * i + 32], "little") for i in range(n_batches)]

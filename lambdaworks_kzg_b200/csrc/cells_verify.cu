@@ -416,6 +416,25 @@ __global__ void __launch_bounds__(128) cell_segmsm_reduce_kernel(uint8_t* __rest
   }
 }
 
+// Cells generated from blobs: one block of 128 threads per blob, thread k of blob b writes cell 128 b + k's inputs of
+// the pass -- the blob's commitment bytes (read by the deduplication and the hash), its decoded point (the segmented
+// MSM), its status (a blob word >= r, else the commitment's decode status) and the cell index k.
+__global__ void __launch_bounds__(128) cell_blob_broadcast_kernel(uint8_t* __restrict__ commit48, G1Affine* __restrict__ commit_pts, int* __restrict__ commit_status,
+                                                                 uint64_t* __restrict__ cell_indices, const uint8_t* __restrict__ blob_commit48,
+                                                                 const G1Affine* __restrict__ blob_pts, const int* __restrict__ blob_status, int n_blobs) {
+  const int b = blockIdx.x, k = threadIdx.x;
+  const size_t g = (size_t)b * N_CELLS + k;
+  const uint4* src = reinterpret_cast<const uint4*>(blob_commit48 + (size_t)b * 48);
+  uint4* dst = reinterpret_cast<uint4*>(commit48 + g * 48);
+  dst[0] = src[0];
+  dst[1] = src[1];
+  dst[2] = src[2];
+  commit_pts[g] = blob_pts[b];
+  const int valid = blob_status[b];
+  commit_status[g] = valid ? valid : blob_status[n_blobs + b];
+  cell_indices[g] = (uint64_t)k;
+}
+
 __global__ void fill_int_kernel(int* __restrict__ out, int v, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = v;
@@ -677,6 +696,14 @@ void launch_cell_segmsm(void* d_out288, void* d_terms, const void* d_scal, const
                                                                              nb, n_terms);
   cell_segmsm_reduce_kernel<<<2 * nb, 128, 0, st>>>((uint8_t*)d_out288, (const G1Xyzz*)d_terms, d_boff);
   count_launch(2);
+}
+
+void launch_cell_blob_broadcast(void* d_commit48, void* d_commit_aff, int* d_commit_status, uint64_t* d_cell_indices, const void* d_blob_commit48,
+                                const void* d_blob_aff, const int* d_blob_status, int n_blobs, cudaStream_t st) {
+  if (n_blobs <= 0) return;
+  cell_blob_broadcast_kernel<<<n_blobs, N_CELLS, 0, st>>>((uint8_t*)d_commit48, (G1Affine*)d_commit_aff, d_commit_status, d_cell_indices,
+                                                          (const uint8_t*)d_blob_commit48, (const G1Affine*)d_blob_aff, d_blob_status, n_blobs);
+  count_launch();
 }
 
 void launch_fill_int(int* d_out, int value, int n, cudaStream_t st) {

@@ -96,6 +96,12 @@ void launch_cell_batches_scalars(void* d_wcoef, void* d_scal, const void* d_eval
 // infinity as zeros); d_terms: cell_segmsm_terms(n_cells, nb) x 192 B of scratch
 void launch_cell_segmsm(void* d_out288, void* d_terms, const void* d_scal, const void* d_proof_aff, const void* d_commit_aff, const void* d_mono_aff,
                         const uint32_t* d_uniq, const int* d_nc, const int* d_boff, int n_cells, int nb, cudaStream_t st);
+// The per-cell inputs of a pass whose cells were generated from n_blobs blobs (cell g = 128 blob + g % 128): the blob's
+// 48 commitment bytes -> d_commit48[g], its decoded commitment (affine Montgomery) -> d_commit_aff[g], cell index g % 128
+// -> d_cell_indices[g], and d_commit_status[g] = d_blob_status[blob] if set (the blob's validity), else
+// d_blob_status[n_blobs + blob] (the commitment's decode status).  Each commitment is decoded once per blob.
+void launch_cell_blob_broadcast(void* d_commit48, void* d_commit_aff, int* d_commit_status, uint64_t* d_cell_indices, const void* d_blob_commit48,
+                                const void* d_blob_aff, const int* d_blob_status, int n_blobs, cudaStream_t st);
 // d_ok[b] = 0 if d_bstatus[b] != 0, 1 if batch b is empty, else d_pair_ok[b]; d_status[b] = d_bstatus[b] (d_status may be NULL)
 // d_out[0, n) = value
 void launch_fill_int(int* d_out, int value, int n, cudaStream_t st);

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """lwkzg_set_devices for the PeerDAS calls: ONE process, one C call, every visible GPU.  The sharded cell batch and the
 sharded recovery batch must return the bytes of the single-device calls, and the sharded many-batch cell verification
-their verdicts, statuses and challenges (MODE_DENEB: the replicas get the monomial SRS from the primary context).  Prints MULTI_DEVICE_CELLS_OK on success."""
+their verdicts, statuses and challenges, as must the sharded verification from blobs (MODE_DENEB: the replicas get the monomial SRS from the primary context).  Prints MULTI_DEVICE_CELLS_OK on success."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -59,7 +59,27 @@ def verify(tag):
     return oks, sts, lw.debug_cell_batch_challenges(len(vb), s)
 
 
+# blob transactions of 1 to 6 blobs over the first 48 blobs, one with swapped commitments and one whose commitment
+# does not decode
+txs = []
+for t in range(64):
+    sel = [(t * 7 + j) % 48 for j in range(1 + t % 6)]
+    txs.append(([blobs[b * 131072: (b + 1) * 131072] for b in sel], [coms[b] for b in sel], [p1[(b * 128 + k) * 48: (b * 128 + k + 1) * 48] for b in sel for k in range(128)]))
+txs[9] = (txs[9][0], txs[9][1][::-1], txs[9][2])
+txs[40] = (txs[40][0], [b"\xff" * 48] + txs[40][1][1:], txs[40][2])
+
+
+def verify_blobs(tag):
+    t0 = time.perf_counter()
+    oks, sts = lw.verify_blob_cell_kzg_proof_batches(txs, s)
+    dt = time.perf_counter() - t0
+    print("%s: verified %d blob transactions in %.1f ms" % (tag, len(txs), dt * 1e3), flush=True)
+    return oks, sts, lw.debug_cell_batch_challenges(len(txs), s)
+
+
 v1 = verify("1 device ")
+b1 = verify_blobs("1 device ")
+assert b1[0] == [t not in (9, 40) for t in range(64)] and b1[1] == [lw.C_KZG_BADARGS if t == 40 else 0 for t in range(64)]
 assert v1[0] == [b not in (5, 77) for b in range(128)] and v1[1] == [lw.C_KZG_BADARGS if b == 77 else 0 for b in range(128)]
 lw.set_devices(list(range(g)))
 run("%d devices (first call builds the replicas)" % g)
@@ -68,5 +88,6 @@ assert c1 == c2 and p1 == p2, "multi-device cell outputs differ from the single-
 rc2, rp2 = recover("%d devices" % g, idx, sel)
 assert rc2 == rc1 and rp2 == rp1, "multi-device recovery outputs differ from the single-device outputs"
 assert verify("%d devices" % g) == v1, "multi-device cell verification differs from the single-device verdicts, statuses or challenges"
+assert verify_blobs("%d devices" % g) == b1, "multi-device verification from blobs differs from the single-device verdicts, statuses or challenges"
 lw.set_devices([])
 print("MULTI_DEVICE_CELLS_OK", flush=True)
