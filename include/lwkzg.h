@@ -248,6 +248,24 @@ C_KZG_RET lwkzg_compute_cells_and_kzg_proofs_batch(Cell *cells, KZGProof *proofs
  * are zeroed; d_status (n ints) may be NULL */
 C_KZG_RET lwkzg_compute_cells_and_kzg_proofs_batch_device(void *d_cells, void *d_proofs, const void *d_blobs, size_t n,
                                                           const KZGSettings *s, void *stream, void *d_status);
+/* additive: the producer side of an EIP-7594 blob transaction in one call -- each blob is read once and gets its
+ * commitment, its 128 cell proofs and, if wanted, its 128 cells.  commitments: n x 48 bytes and proofs: n x 128 proofs,
+ * both required; cells: n x 128 cells or NULL.  The bytes of every blob equal those of lwkzg_blob_to_kzg_commitment_batch
+ * and lwkzg_compute_cells_and_kzg_proofs_batch on it, in all three modes.  status[n] (may be NULL) gets one code per
+ * blob; a blob fails only where both of those calls fail on it -- a word >= r in modes 1 and 2, C_KZG_BADARGS (mode 0
+ * has no per-blob failure) -- and all its output slots, its commitment included, are left untouched.  Whole-call
+ * errors: n == 0 returns C_KZG_OK and writes nothing; a NULL blobs, commitments or proofs returns C_KZG_BADARGS;
+ * settings without the monomial SRS return C_KZG_ERROR; with status == NULL the first failing blob's code is returned.
+ * A pass of up to "cell_chunk_blobs" blobs copies its blobs to the device once; the commitment MSM of
+ * lwkzg_blob_to_kzg_commitment_batch reads them there on a stream of its own beside the FK20 pipeline.  After
+ * lwkzg_set_devices the blobs are sharded over the GPUs. */
+C_KZG_RET lwkzg_commit_and_compute_cells_and_kzg_proofs_batch(KZGCommitment *commitments, Cell *cells, KZGProof *proofs,
+                                                              const Blob *blobs, size_t n, const KZGSettings *s, int *status);
+/* the same on device buffers (16-byte aligned), asynchronous, ordered after / before work on `stream`; outputs of
+ * failed blobs are zeroed; d_cells and d_status (n ints, C_KZG_RET values) may be NULL */
+C_KZG_RET lwkzg_commit_and_compute_cells_and_kzg_proofs_batch_device(void *d_commitments, void *d_cells, void *d_proofs,
+                                                                     const void *d_blobs, size_t n, const KZGSettings *s,
+                                                                     void *stream, void *d_status);
 /* additive: recover_cells_and_kzg_proofs over n blobs, each given by num_cells (64..128) of its cells.  cell_indices
  * and cells are n x num_cells, blob-major; the indices of each blob are strictly ascending and < 128 (blobs may use
  * different index sets of the same size).  recovered_cells: n x 128 cells or NULL; recovered_proofs: n x 128 proofs or

@@ -82,6 +82,8 @@ def load_library() -> ctypes.CDLL:
         "verify_cell_kzg_proof_batch": [bp, vp, vp, vp, vp, sz, sp],
         "lwkzg_compute_cells_and_kzg_proofs_batch": [vp, vp, vp, sz, sp, ip],
         "lwkzg_compute_cells_and_kzg_proofs_batch_device": [vp, vp, vp, sz, sp, vp, vp],
+        "lwkzg_commit_and_compute_cells_and_kzg_proofs_batch": [vp, vp, vp, vp, sz, sp, ip],
+        "lwkzg_commit_and_compute_cells_and_kzg_proofs_batch_device": [vp, vp, vp, vp, sz, sp, vp, vp],
         "lwkzg_recover_cells_and_kzg_proofs_batch": [vp, vp, vp, vp, sz, sz, sp, ip],
         "lwkzg_recover_cells_and_kzg_proofs_batch_device": [vp, vp, vp, vp, sz, sz, sp, vp, vp],
         "lwkzg_verify_cell_kzg_proof_batches": [bp, vp, vp, vp, vp, vp, sz, sp, ip],
@@ -500,6 +502,29 @@ def compute_cells_and_kzg_proofs_batch_device(d_cells: int, d_proofs: int, d_blo
     """Device-pointer variant: raw device addresses (0 = not wanted), asynchronous with respect to the host."""
     _check(load_library().lwkzg_compute_cells_and_kzg_proofs_batch_device(d_cells or None, d_proofs or None, d_blobs, n, _sp(s), stream or None,
                                                                           d_status or None), "lwkzg_compute_cells_and_kzg_proofs_batch_device")
+
+
+def commit_and_compute_cells_and_kzg_proofs_batch(blobs: bytes, n: int, s, want_cells: bool = False):
+    """-> (commitments list, cells bytes n x 128 x 2048 or b"", proofs bytes n x 128 x 48, status list): each blob read
+    once for its commitment, its 128 cell proofs and (want_cells) its cells."""
+    assert len(blobs) == n * BYTES_PER_BLOB
+    coms = ctypes.create_string_buffer(max(1, n * 48))
+    cells = ctypes.create_string_buffer(max(1, n * CELLS_PER_EXT_BLOB * BYTES_PER_CELL)) if want_cells else None
+    proofs = ctypes.create_string_buffer(max(1, n * CELLS_PER_EXT_BLOB * 48))
+    st = (ctypes.c_int * max(1, n))()
+    _check(load_library().lwkzg_commit_and_compute_cells_and_kzg_proofs_batch(coms, cells, proofs, blobs, n, _sp(s), st),
+           "lwkzg_commit_and_compute_cells_and_kzg_proofs_batch")
+    return ([coms.raw[48 * i: 48 * i + 48] for i in range(n)], cells.raw[: n * CELLS_PER_EXT_BLOB * BYTES_PER_CELL] if want_cells else b"",
+            proofs.raw[: n * CELLS_PER_EXT_BLOB * 48], list(st)[:n])
+
+
+def commit_and_compute_cells_and_kzg_proofs_batch_device(d_commitments: int, d_cells: int, d_proofs: int, d_blobs: int, n: int, s, stream: int = 0,
+                                                         d_status: int = 0):
+    """Device-pointer variant: raw device addresses (d_cells, d_status: 0 = not wanted), asynchronous with respect to
+    the host."""
+    _check(load_library().lwkzg_commit_and_compute_cells_and_kzg_proofs_batch_device(d_commitments or None, d_cells or None, d_proofs or None, d_blobs or None,
+                                                                                     n, _sp(s), stream or None, d_status or None),
+           "lwkzg_commit_and_compute_cells_and_kzg_proofs_batch_device")
 
 
 def recover_cells_and_kzg_proofs(cell_indices: Sequence[int], cells: Sequence[bytes], s, want_cells: bool = True, want_proofs: bool = True):
