@@ -161,6 +161,23 @@ C_KZG_RET lwkzg_verify_blob_kzg_proof_batch_device(bool *ok, const void *d_blobs
                                                    const void *d_commitments, const void *d_proofs,
                                                    size_t n, const KZGSettings *s);
 
+/* n independent verify_kzg_proof checks.  ok[i] / status[i] are exactly what verify_kzg_proof returns for item i. */
+/* Per item, in every mode: a commitment or proof that does not decode or is not in G1, or -- modes 1 and 2 -- a z or
+ * y >= r (mode 0 reduces them mod r, as the single call does) fails the item with C_KZG_BADARGS (modes 1 and 2) or
+ * C_KZG_ERROR (mode 0), and ok[i] = false.  Each verdict comes from its own pairing check, never from an aggregate
+ * (the reference's internal verify_kzg_proof_batch, src/lib.rs:639-692, is an aggregate with one verdict).  Whole
+ * call: n == 0 returns C_KZG_OK and writes nothing; a NULL ok or input pointer returns C_KZG_BADARGS; with
+ * status == NULL the first failing item's code is returned and ok is still filled.  The host form shards its items
+ * over lwkzg_set_devices.  Both forms run in passes of a fixed size, so device memory stays bounded whatever n is.
+ * The device form is asynchronous on `stream`: d_ok (n ints, 1 or 0) and d_status (n ints of C_KZG_RET, may be NULL)
+ * are device memory, the inputs are device addresses, 16-byte aligned.  Built for throughput: one item per thread,
+ * so a single opening is faster through verify_kzg_proof. */
+C_KZG_RET lwkzg_verify_kzg_proofs(bool *ok, const Bytes48 *commitments, const Bytes32 *zs, const Bytes32 *ys,
+                                  const Bytes48 *proofs, size_t n, const KZGSettings *s, int *status);
+C_KZG_RET lwkzg_verify_kzg_proofs_device(void *d_ok, const void *d_commitments, const void *d_zs, const void *d_ys,
+                                         const void *d_proofs, size_t n, const KZGSettings *s, void *stream,
+                                         void *d_status);
+
 /* Generic G1 multi-scalar multiplication (the reference's g1_lincomb,
  * src/lib.rs:241-243): out = sum scalars[i] * points[i].  points: n x 96 bytes
  * canonical big-endian affine x||y (all-zero = infinity); scalars: n x 32 bytes

@@ -64,6 +64,8 @@ def load_library() -> ctypes.CDLL:
         "lwkzg_commit_and_prove_batch_device": [vp, vp, vp, sz, sp, vp, vp],
         "lwkzg_blob_to_kzg_commitment_batch_device": [vp, vp, sz, sp, vp, vp],
         "lwkzg_verify_blob_kzg_proof_batch_device": [bp, vp, vp, vp, sz, sp],
+        "lwkzg_verify_kzg_proofs": [bp, vp, vp, vp, vp, sz, sp, ip],
+        "lwkzg_verify_kzg_proofs_device": [vp, vp, vp, vp, vp, sz, sp, vp, vp],
         "lwkzg_compute_blob_kzg_proof_batch_device": [vp, vp, vp, sz, sp, vp, vp],
         "lwkzg_g1_lincomb": [vp, vp, vp, sz],
         "lwkzg_verify_batch_phase1": [vp, vp, vp, vp, sz, sp],
@@ -239,6 +241,25 @@ def verify_kzg_proof(commitment: bytes, z_bytes: bytes, y_bytes: bytes, proof: b
     ok = ctypes.c_bool(False)
     _check(load_library().verify_kzg_proof(ctypes.byref(ok), commitment, z_bytes, y_bytes, proof, _sp(s)), "verify_kzg_proof")
     return bool(ok.value)
+
+
+def verify_kzg_proofs(commitments: Sequence[bytes], zs: Sequence[bytes], ys: Sequence[bytes], proofs: Sequence[bytes], s) -> Tuple[List[bool], List[int]]:
+    """n independent verify_kzg_proof checks in one call -> (verdict list, status list): for each item the verdict and
+    code verify_kzg_proof returns for it (a failed item has verdict False)."""
+    n = len(commitments)
+    assert len(zs) == len(ys) == len(proofs) == n
+    oks = (ctypes.c_bool * max(1, n))()
+    st = _status_list(n)
+    _check(load_library().lwkzg_verify_kzg_proofs(oks, _cat(commitments, 48) or b"\0", _cat(zs, 32) or b"\0", _cat(ys, 32) or b"\0",
+                                                  _cat(proofs, 48) or b"\0", n, _sp(s), st), "lwkzg_verify_kzg_proofs")
+    return [bool(oks[i]) for i in range(n)], list(st)[:n]
+
+
+def verify_kzg_proofs_device(d_ok: int, d_commitments: int, d_zs: int, d_ys: int, d_proofs: int, n: int, s, stream: int = 0, d_status: int = 0):
+    """All buffers are raw device addresses (torch: tensor.data_ptr()); d_ok and d_status (0 = not wanted) are n int32
+    each.  Asynchronous on `stream`."""
+    _check(load_library().lwkzg_verify_kzg_proofs_device(d_ok or None, d_commitments or None, d_zs or None, d_ys or None, d_proofs or None, n, _sp(s),
+                                                         stream or None, d_status or None), "lwkzg_verify_kzg_proofs_device")
 
 
 def verify_blob_kzg_proof(blob: bytes, commitment: bytes, proof: bytes, s) -> bool:

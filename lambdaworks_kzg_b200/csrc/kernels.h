@@ -126,6 +126,14 @@ void launch_batch_final(int* d_ok, const void* d_partials288, int n_ranks, const
 // n_checks independent checks, one block each: d_ok[i] from the 288 bytes at d_partials288 + 288 i
 void launch_batch_final_each(int* d_ok, const void* d_partials288, int n_checks, const void* d_prep0, const void* d_prep1, cudaStream_t st);
 
+// ---- many independent single-opening checks (verify_proofs.cu), one item per thread
+// d_pts[2 i] = C_i - y_i G + z_i pi_i, d_pts[2 i + 1] = -pi_i (affine Montgomery) from decoded C, pi (in G1 or infinity) and
+// canonical z, y; glv_g: G is in the r-torsion
+void launch_verify_proofs_g1(void* d_pts, const void* d_c_aff, const void* d_pi_aff, const void* d_z, const void* d_y, const void* d_g_aff, bool glv_g, int n,
+                             cudaStream_t st);
+// d_ok[i] = d_status[i] == 0 && e(d_pts[2 i], g2_0) e(d_pts[2 i + 1], g2_1) == 1
+void launch_verify_proofs_pairing(int* d_ok, const int* d_status, const void* d_pts, const void* d_prep0, const void* d_prep1, int n, cudaStream_t st);
+
 // ---- MODE_CKZG_LE (le.cu)
 void launch_write_generator(void* d_out, cudaStream_t st);                 // the G1 generator, affine Montgomery
 void launch_le_roots(void* d_roots, cudaStream_t st);                      // 4096 Fr (Montgomery), bit-reversed order

@@ -290,6 +290,9 @@ struct Ctx {
   cudaEvent_t ev_hash = nullptr;
   std::vector<cudaEvent_t> ev_pool;   // per chunk: blob copy landed / tuples written
   DevBuf vb_hstate, vb_blobs, vb_states, vb_status2, vb_sub;
+  // lwkzg_verify_kzg_proofs, one pass: inputs (host-buffer calls), decoded points and scalars, the G1 stage's pairs,
+  // per-item statuses, verdicts
+  DevBuf vp_in, vp_aff, vp_zy, vp_pts, vp_st, vp_io;
   // pinned host staging for batch results: a D2H copy into pageable memory would block the host
   // until the chunk's kernels finish and serialise the two pipeline slots
   void* h_stage = nullptr;
@@ -1538,6 +1541,116 @@ struct CtxLock {
   explicit CtxLock(Ctx* ctx) : c(ctx), lk(ctx->mu), dg(ctx->device) {}
 };
 
+// ------------------------------------------------------------------ lwkzg_verify_kzg_proofs
+// n independent verify_kzg_proof checks in passes of at most VP_PASS items, so device memory stays bounded whatever n
+// is (about 0.6 KB per item of a pass).  A pass is a fixed launch sequence on one stream: decode C and pi (r-torsion
+// tests included) and z, y, fold their statuses, the G1 stage, the pairing stage.
+constexpr size_t VP_PASS = 32768;
+
+// own_io: the pass's inputs, verdicts and statuses are the context's own (host-buffer calls)
+BufList vp_buffers(Ctx* c, size_t m, bool own_io) {
+  BufList bufs = {{&c->vp_aff, 2 * m * AFFINE_BYTES}, {&c->vp_zy, 2 * m * 32}, {&c->vp_pts, 2 * m * AFFINE_BYTES}, {&c->vp_st, 3 * m * sizeof(int)},
+                  {&c->vp_io, 2 * m * sizeof(int)}};
+  if (own_io) bufs.push_back({&c->vp_in, m * (48 + 32 + 32 + 48)});
+  return bufs;
+}
+
+// one pass of m items on st: device inputs d_c, d_z, d_y, d_pi; d_ok and d_st receive the m verdicts and codes
+bool vp_enqueue_pass(Ctx* c, int m, const void* d_c, const void* d_z, const void* d_y, const void* d_pi, int* d_ok, int* d_st, cudaStream_t st) {
+  const bool le = c->lagrange();
+  uint8_t* aff = (uint8_t*)c->vp_aff.p;   // C | pi
+  uint8_t* zy = (uint8_t*)c->vp_zy.p;     // z | y
+  int* st2 = (int*)c->vp_st.p;            // pi | z | y
+  launch_g1_decompress(aff, nullptr, d_st, d_c, m, st, le);
+  launch_g1_decompress(aff + (size_t)m * AFFINE_BYTES, nullptr, st2, d_pi, m, st, le);
+  launch_status_or(d_st, st2, m, st);
+  if (le) {
+    CU_TRY(cudaMemsetAsync(st2 + m, 0, 2 * (size_t)m * sizeof(int), st));
+    launch_le_fr_parse(zy, st2 + m, d_z, m, st, c->be_wire());
+    launch_le_fr_parse(zy + (size_t)m * 32, st2 + 2 * m, d_y, m, st, c->be_wire());
+    launch_status_or(d_st, st2 + m, m, st);
+    launch_status_or(d_st, st2 + 2 * m, m, st);
+  } else {
+    launch_fr_from_be(zy, d_z, m, st);
+    launch_fr_from_be(zy + (size_t)m * 32, d_y, m, st);
+  }
+  // G as verify_single_from_workspace chooses it: c-kzg verifies against the generator, the reference against g1[0]
+  launch_verify_proofs_g1(c->vp_pts.p, aff, aff + (size_t)m * AFFINE_BYTES, zy, zy + (size_t)m * 32, c->lagrange() ? c->d_gen : c->d_srs,
+                          c->lagrange() || c->srs_in_g1, m, st);
+  launch_verify_proofs_pairing(d_ok, d_st, c->vp_pts.p, c->d_prep0, c->d_prep1, m, st);
+  return true;
+}
+
+C_KZG_RET verify_proofs_host(bool* ok, const Bytes48* commitments, const Bytes32* zs, const Bytes32* ys, const Bytes48* proofs, size_t n,
+                             const KZGSettings* s, int* status) {
+  if (n == 0) return C_KZG_OK;
+  if (!ok || !commitments || !zs || !ys || !proofs) { set_err("null argument"); return C_KZG_BADARGS; }
+  Ctx* c = ctx_of(s);
+  if (!c) return C_KZG_ERROR;
+  if (c->srs_valid && !c->g2_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
+  return sharded_batch(c, n, status, "invalid commitment, proof or field element bytes", [&](Ctx* x, size_t first, size_t cnt, int* st) -> C_KZG_RET {
+    CtxLock lock(x);
+    if (!reserve(vp_buffers(x, std::min(cnt, VP_PASS), true))) return C_KZG_ERROR;
+    cudaStream_t s0 = x->slot[0].st;
+    std::vector<int> h_io;
+    for (size_t off = 0; off < cnt; off += VP_PASS) {
+      const size_t m = std::min(VP_PASS, cnt - off), i0 = first + off;
+      uint8_t* in = (uint8_t*)x->vp_in.p;   // C | pi | z | y
+      int* d_io = (int*)x->vp_io.p;         // ok | status
+      h_io.resize(2 * m);
+      bool good = [&]() -> bool {
+        CU_TRY(cudaMemcpyAsync(in, commitments + i0, m * 48, cudaMemcpyHostToDevice, s0));
+        CU_TRY(cudaMemcpyAsync(in + m * 48, proofs + i0, m * 48, cudaMemcpyHostToDevice, s0));
+        CU_TRY(cudaMemcpyAsync(in + m * 96, zs + i0, m * 32, cudaMemcpyHostToDevice, s0));
+        CU_TRY(cudaMemcpyAsync(in + m * 128, ys + i0, m * 32, cudaMemcpyHostToDevice, s0));
+        if (!vp_enqueue_pass(x, (int)m, in, in + m * 96, in + m * 128, in + m * 48, d_io, d_io + m, s0)) return false;
+        CU_TRY(cudaMemcpyAsync(h_io.data(), d_io, 2 * m * sizeof(int), cudaMemcpyDeviceToHost, s0));
+        CU_TRY(cudaStreamSynchronize(s0));
+        CU_TRY(cudaGetLastError());
+        return true;
+      }();
+      if (!good) return C_KZG_ERROR;
+      for (size_t i = 0; i < m; i++) {
+        ok[i0 + i] = h_io[i] != 0;
+        st[off + i] = h_io[m + i];
+      }
+    }
+    return C_KZG_OK;
+  });
+}
+
+// the device form: asynchronous, ordered after and before `user`; the host waits for earlier work only when a buffer
+// has to grow (which frees the old one)
+C_KZG_RET verify_proofs_device(void* d_ok, const void* d_c, const void* d_z, const void* d_y, const void* d_pi, size_t n, const KZGSettings* s,
+                               cudaStream_t user, void* d_status) {
+  if (n == 0) return C_KZG_OK;
+  if (!d_ok || !d_c || !d_z || !d_y || !d_pi) { set_err("null argument"); return C_KZG_BADARGS; }
+  Ctx* c = ctx_of(s);
+  if (!c) return C_KZG_ERROR;
+  if (!c->srs_valid || !c->g2_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
+  CtxLock lock(c);
+  Slot& sl = c->slot[0];
+  const BufList bufs = vp_buffers(c, std::min(n, VP_PASS), false);
+  if (!fits(bufs)) cudaStreamSynchronize(sl.st);
+  if (!reserve(bufs)) return C_KZG_ERROR;
+  bool good = [&]() -> bool {
+    CU_TRY(cudaEventRecord(sl.ev_fork, user));
+    CU_TRY(cudaStreamWaitEvent(sl.st, sl.ev_fork, 0));
+    for (size_t off = 0; off < n; off += VP_PASS) {
+      const int m = (int)std::min(VP_PASS, n - off);
+      int* st = d_status ? (int*)d_status + off : (int*)c->vp_io.p;
+      if (!vp_enqueue_pass(c, m, (const uint8_t*)d_c + off * 48, (const uint8_t*)d_z + off * 32, (const uint8_t*)d_y + off * 32,
+                           (const uint8_t*)d_pi + off * 48, (int*)d_ok + off, st, sl.st))
+        return false;
+    }
+    CU_TRY(cudaEventRecord(sl.ev_done, sl.st));
+    CU_TRY(cudaStreamWaitEvent(user, sl.ev_done, 0));
+    CU_TRY(cudaGetLastError());
+    return true;
+  }();
+  return good ? C_KZG_OK : C_KZG_ERROR;
+}
+
 #include "cells_host.inl"
 
 }  // namespace
@@ -1747,6 +1860,15 @@ C_KZG_RET verify_kzg_proof(bool* ok, const Bytes48* commitment_bytes, const Byte
   if (bad) { set_err("invalid commitment, proof or field element bytes"); return bad_code(bad); }
   *ok = res;
   return C_KZG_OK;
+}
+
+C_KZG_RET lwkzg_verify_kzg_proofs(bool* ok, const Bytes48* commitments, const Bytes32* zs, const Bytes32* ys, const Bytes48* proofs, size_t n,
+                                  const KZGSettings* s, int* status) {
+  return verify_proofs_host(ok, commitments, zs, ys, proofs, n, s, status);
+}
+C_KZG_RET lwkzg_verify_kzg_proofs_device(void* d_ok, const void* d_commitments, const void* d_zs, const void* d_ys, const void* d_proofs, size_t n,
+                                         const KZGSettings* s, void* stream, void* d_status) {
+  return verify_proofs_device(d_ok, d_commitments, d_zs, d_ys, d_proofs, n, s, (cudaStream_t)stream, d_status);
 }
 
 static C_KZG_RET verify_blob_single(bool* ok, const Blob* blob, const Bytes48* commitment_bytes, const Bytes48* proof_bytes, const KZGSettings* s,
