@@ -178,6 +178,33 @@ C_KZG_RET lwkzg_verify_kzg_proofs_device(void *d_ok, const void *d_commitments, 
                                          const void *d_proofs, size_t n, const KZGSettings *s, void *stream,
                                          void *d_status);
 
+/* K independent verify_blob_kzg_proof_batch checks, one per transaction or sidecar set.  Batch b is blobs
+ * [offsets[b], offsets[b + 1]) of the flat blobs / commitments / proofs arrays; offsets (K + 1 host integers,
+ * offsets[0] == 0, non-decreasing) stays on the host in the device form too.  ok[b] / status[b] are exactly what ONE
+ * verify_blob_kzg_proof_batch call over that batch alone returns, in every mode:
+ *  - an empty batch: ok = false in mode 0 (src/lib.rs:538-543), true in modes 1 and 2, C_KZG_OK;
+ *  - one blob: verify_blob_kzg_proof's verdict (mode 0 subtracts y g1_values[0], as the single call does);
+ *  - n_b >= 2 blobs: the batch's own challenge r_b, hashed over its own tuples with n_b in the header, weights
+ *    r_b^0 .. r_b^(n_b - 1), y summed against the generator;
+ *  - a commitment or proof that does not decode or is not in G1, or -- modes 1 and 2 -- a blob word >= r fails its
+ *    own batch only: C_KZG_BADARGS (modes 1 and 2) or C_KZG_ERROR (mode 0), and ok = false.
+ * Whole call: n_batches == 0 returns C_KZG_OK and writes nothing; a NULL ok or offsets, a NULL input pointer when
+ * offsets[K] > 0, offsets[0] != 0, decreasing offsets, or more than 2^24 blobs return C_KZG_BADARGS; with status ==
+ * NULL the first failing batch's code is returned and ok is still filled.  The host form shards whole batches over
+ * lwkzg_set_devices.  Both forms run in passes of whole batches of at most "verify_super_blobs" blobs (a larger batch
+ * gets a pass of its own), so device memory is bounded by that option and the largest batch, not by K.  The device
+ * form is asynchronous on `stream`: d_ok (K ints, 1 or 0) and d_status (K ints of C_KZG_RET, may be NULL) are device
+ * memory, the inputs are device addresses, 16-byte aligned, read in place. */
+C_KZG_RET lwkzg_verify_blob_kzg_proof_batches(bool *ok, const Blob *blobs, const Bytes48 *commitments,
+                                              const Bytes48 *proofs, const uint64_t *offsets, size_t n_batches,
+                                              const KZGSettings *s, int *status);
+C_KZG_RET lwkzg_verify_blob_kzg_proof_batches_device(void *d_ok, const void *d_blobs, const void *d_commitments,
+                                                     const void *d_proofs, const uint64_t *offsets, size_t n_batches,
+                                                     const KZGSettings *s, void *stream, void *d_status);
+/* test hook: r_b of every batch of the last call on these settings, 32 little-endian bytes each; zeros for batches of
+ * < 2 blobs */
+C_KZG_RET lwkzg_debug_blob_batch_challenges(uint8_t *out32, size_t n_batches, const KZGSettings *s);
+
 /* Generic G1 multi-scalar multiplication (the reference's g1_lincomb,
  * src/lib.rs:241-243): out = sum scalars[i] * points[i].  points: n x 96 bytes
  * canonical big-endian affine x||y (all-zero = infinity); scalars: n x 32 bytes

@@ -66,6 +66,9 @@ def load_library() -> ctypes.CDLL:
         "lwkzg_verify_blob_kzg_proof_batch_device": [bp, vp, vp, vp, sz, sp],
         "lwkzg_verify_kzg_proofs": [bp, vp, vp, vp, vp, sz, sp, ip],
         "lwkzg_verify_kzg_proofs_device": [vp, vp, vp, vp, vp, sz, sp, vp, vp],
+        "lwkzg_verify_blob_kzg_proof_batches": [bp, vp, vp, vp, vp, sz, sp, ip],
+        "lwkzg_verify_blob_kzg_proof_batches_device": [vp, vp, vp, vp, vp, sz, sp, vp, vp],
+        "lwkzg_debug_blob_batch_challenges": [vp, sz, sp],
         "lwkzg_compute_blob_kzg_proof_batch_device": [vp, vp, vp, sz, sp, vp, vp],
         "lwkzg_g1_lincomb": [vp, vp, vp, sz],
         "lwkzg_verify_batch_phase1": [vp, vp, vp, vp, sz, sp],
@@ -295,6 +298,43 @@ def verify_blob_kzg_proof_batch_device(d_blobs: int, d_commitments: int, d_proof
     _check(load_library().lwkzg_verify_blob_kzg_proof_batch_device(ctypes.byref(ok), d_blobs, d_commitments, d_proofs, n, _sp(s)),
            "lwkzg_verify_blob_kzg_proof_batch_device")
     return bool(ok.value)
+
+
+def verify_blob_kzg_proof_batches(batches: Sequence[Tuple[Sequence[bytes], Sequence[bytes], Sequence[bytes]]], s) -> Tuple[List[bool], List[int]]:
+    """K independent verify_blob_kzg_proof_batch checks in one call.  batches: (blobs, commitments, proofs) per batch ->
+    (verdict list, status list): per batch, what verify_blob_kzg_proof_batch over that batch alone returns."""
+    k = len(batches)
+    offsets = [0]
+    for bl, com, pr in batches:
+        assert len(bl) == len(com) == len(pr)
+        offsets.append(offsets[-1] + len(bl))
+    off = (ctypes.c_uint64 * (k + 1))(*offsets)
+    oks = (ctypes.c_bool * max(1, k))()
+    st = _status_list(k)
+    _check(load_library().lwkzg_verify_blob_kzg_proof_batches(oks, b"".join(_cat(b[0], BYTES_PER_BLOB) for b in batches) or b"\0",
+                                                              b"".join(_cat(b[1], 48) for b in batches) or b"\0",
+                                                              b"".join(_cat(b[2], 48) for b in batches) or b"\0", off, k, _sp(s), st),
+           "lwkzg_verify_blob_kzg_proof_batches")
+    return [bool(oks[i]) for i in range(k)], list(st)[:k]
+
+
+def verify_blob_kzg_proof_batches_device(d_ok: int, d_blobs: int, d_commitments: int, d_proofs: int, offsets: Sequence[int], s, stream: int = 0,
+                                         d_status: int = 0):
+    """All buffers are raw device addresses (torch: tensor.data_ptr()) except offsets (K + 1 host integers, in blobs);
+    d_ok and d_status (0 = not wanted) are K int32 each.  Asynchronous on `stream`."""
+    k = len(offsets) - 1
+    off = (ctypes.c_uint64 * max(1, k + 1))(*offsets)
+    _check(load_library().lwkzg_verify_blob_kzg_proof_batches_device(d_ok or None, d_blobs or None, d_commitments or None, d_proofs or None, off, k,
+                                                                     _sp(s), stream or None, d_status or None),
+           "lwkzg_verify_blob_kzg_proof_batches_device")
+
+
+def debug_blob_batch_challenges(n_batches: int, s) -> List[int]:
+    """The challenges r_b the last verify_blob_kzg_proof_batches[_device] call derived (0 for batches of fewer than two
+    blobs; test hook)."""
+    out = ctypes.create_string_buffer(32 * max(1, n_batches))
+    _check(load_library().lwkzg_debug_blob_batch_challenges(out, n_batches, _sp(s)), "lwkzg_debug_blob_batch_challenges")
+    return [int.from_bytes(out.raw[32 * i: 32 * i + 32], "little") for i in range(n_batches)]
 
 
 # ------------------------------------------------------------------ batch extensions (host buffers)

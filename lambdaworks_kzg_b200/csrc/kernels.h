@@ -134,6 +134,21 @@ void launch_verify_proofs_g1(void* d_pts, const void* d_c_aff, const void* d_pi_
 // d_ok[i] = d_status[i] == 0 && e(d_pts[2 i], g2_0) e(d_pts[2 i + 1], g2_1) == 1
 void launch_verify_proofs_pairing(int* d_ok, const int* d_status, const void* d_pts, const void* d_prep0, const void* d_prep1, int n, cudaStream_t st);
 
+// ---- many independent blob-proof batches per pass (verify_batches.cu); batch b is the pass's blobs [d_boff[b], d_boff[b + 1])
+// d_bstatus[b] = code if any of the batch's d_item_status is non-zero, else 0
+void launch_blob_batches_status(int* d_bstatus, const int* d_item_status, const int* d_boff, int nb, int code, cudaStream_t st);
+// r_b over the batch's tuples (160 B per blob, n_b in the header, wire as in launch_batch_challenge), zeros when n_b < 2
+void launch_blob_batches_challenge(void* d_rs, const void* d_tuples160, const int* d_boff, int nb, int wire, cudaStream_t st);
+// the 288-byte partial of every non-empty batch b at d_out288 + 288 d_slot[b] (d_slot[b] = -1: empty): sum r_b^j pi_j |
+// infinity | sum r_b^j (C_j + z_j pi_j) - (sum r_b^j y_j) G, G = d_g_one for a one-blob batch (one_glv: it is in G1),
+// else the generator.  d_scalars / d_terms: blob_batches_terms(n_items, nb) x 32 / 192 bytes of scratch
+size_t blob_batches_terms(int n_items, int nb);
+void launch_blob_batches_msm(void* d_out288, void* d_terms, void* d_scalars, const void* d_rs, const void* d_z, const void* d_y, const void* d_c_aff,
+                             const void* d_pi_aff, const void* d_g_one, bool one_glv, const int* d_boff, const int* d_slot, int n_items, int nb,
+                             cudaStream_t st);
+// d_ok[b] = d_bstatus[b] ? 0 : empty batch ? empty_ok : d_pair_ok[d_slot[b]]; d_status (may be NULL) = d_bstatus
+void launch_blob_batches_fold(int* d_ok, int* d_status, const int* d_pair_ok, const int* d_bstatus, const int* d_slot, int nb, bool empty_ok, cudaStream_t st);
+
 // ---- MODE_CKZG_LE (le.cu)
 void launch_write_generator(void* d_out, cudaStream_t st);                 // the G1 generator, affine Montgomery
 void launch_le_roots(void* d_roots, cudaStream_t st);                      // 4096 Fr (Montgomery), bit-reversed order

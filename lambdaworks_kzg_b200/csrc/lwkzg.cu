@@ -293,6 +293,17 @@ struct Ctx {
   // lwkzg_verify_kzg_proofs, one pass: inputs (host-buffer calls), decoded points and scalars, the G1 stage's pairs,
   // per-item statuses, verdicts
   DevBuf vp_in, vp_aff, vp_zy, vp_pts, vp_st, vp_io;
+  // lwkzg_verify_blob_kzg_proof_batches, one pass: per blob (inputs and staged blobs of host-buffer calls, points,
+  // re-encodings, hash states, z | y, tuples, statuses), per term (scalars, products), per batch (offsets and partial
+  // slots of every pass, statuses, partials, pairing results, verdicts), the challenges of the call; the offsets are
+  // staged in pinned memory (h_bb, rewritten once the copy ev_bb marks has completed)
+  DevBuf bb_in, bb_blobs, bb_aff, bb_c48r, bb_p48r, bb_states, bb_zy, bb_tuples, bb_st, bb_sc, bb_terms, bb_boff, bb_bst, bb_out, bb_pok, bb_io, bb_rs;
+  int* h_bb = nullptr;
+  size_t h_bb_cap = 0;
+  cudaEvent_t ev_bb = nullptr;
+  std::vector<uint8_t> bb_h_rs;   // the last call's challenges, when they came back to the host
+  size_t bb_rs_n = 0;
+  bool bb_rs_on_host = true;
   // pinned host staging for batch results: a D2H copy into pageable memory would block the host
   // until the chunk's kernels finish and serialise the two pipeline slots
   void* h_stage = nullptr;
@@ -403,6 +414,8 @@ void destroy_ctx(Ctx* c) {
   if (c->d_roots) cudaFree(c->d_roots);
   if (c->d_gen) cudaFree(c->d_gen);
   if (c->h_stage) cudaFreeHost(c->h_stage);
+  if (c->ev_bb) { cudaEventSynchronize(c->ev_bb); cudaEventDestroy(c->ev_bb); }
+  if (c->h_bb) cudaFreeHost(c->h_bb);
   c->ring.release();
   c->magic = 0;
   delete c;
@@ -1653,6 +1666,279 @@ C_KZG_RET verify_proofs_device(void* d_ok, const void* d_c, const void* d_z, con
 
 #include "cells_host.inl"
 
+// ------------------------------------------------------------------ lwkzg_verify_blob_kzg_proof_batches
+// K independent verify_blob_kzg_proof_batch checks.  A call runs in passes of whole batches holding at most
+// verify_super_blobs blobs, planned as the cell calls plan theirs (cell_batch_passes); a larger batch gets a pass of its
+// own, whose host blobs are staged verify_super_blobs at a time while its per-blob state (points, z, y, tuples,
+// statuses: about 0.6 KB per blob) covers the whole batch.  A pass is one fixed launch sequence whatever its number of
+// batches (bb_enqueue_pass).  This is not verify_prepare, which is built for one huge batch, synchronises the host and
+// owns the vb_* workspace that the aggregate call, the distributed phases and their test hooks read.
+
+// The buffers of a call planned as `plan` (own_io: the inputs, staged blobs and verdicts of a pass too, for host-buffer
+// calls): per-blob and per-batch buffers for its largest pass, the offsets of every pass, the challenges of rs_batches
+// batches.
+BufList bb_buffers(Ctx* c, const std::vector<CellBatchPass>& plan, size_t rs_batches, size_t stage, bool own_io) {
+  size_t m = 1, nb = 1, offs = 0;
+  for (const CellBatchPass& p : plan) {
+    m = std::max(m, p.o1 - p.o0);
+    nb = std::max(nb, p.b1 - p.b0);
+    offs += 2 * (p.b1 - p.b0) + 1;
+  }
+  const size_t terms = blob_batches_terms((int)m, (int)nb);
+  BufList bufs = {{&c->bb_aff, 2 * m * AFFINE_BYTES}, {&c->bb_c48r, m * 48}, {&c->bb_p48r, m * 48}, {&c->bb_states, m * 32}, {&c->bb_zy, 2 * m * 32},
+                  {&c->bb_tuples, m * 160}, {&c->bb_st, 3 * m * sizeof(int)}, {&c->bb_sc, terms * 32}, {&c->bb_terms, terms * XYZZ_BYTES},
+                  {&c->bb_boff, offs * sizeof(int)}, {&c->bb_bst, nb * sizeof(int)}, {&c->bb_out, nb * 288}, {&c->bb_pok, nb * sizeof(int)},
+                  {&c->bb_rs, std::max<size_t>(rs_batches, 1) * 32}};
+  if (own_io) bufs.insert(bufs.end(), {{&c->bb_in, m * 96}, {&c->bb_blobs, std::min(m, stage) * BLOB_BYTES}, {&c->bb_io, 2 * nb * sizeof(int)}});
+  return bufs;
+}
+
+// Pass i's offsets at c->bb_boff + at[i]: its nb + 1 batch offsets rebased to its first blob, then the nb partial slots
+// (-1 for an empty batch, else the index among the pass's n_ne[i] non-empty batches).  Staged in pinned memory, which is
+// rewritten only after the previous call's copy out of it has completed, and copied with ONE copy on st.
+bool bb_stage_offsets(Ctx* c, const std::vector<CellBatchPass>& plan, const uint64_t* offsets, std::vector<size_t>& at, std::vector<int>& n_ne,
+                      cudaStream_t st) {
+  size_t total = 0;
+  at.clear();
+  n_ne.clear();
+  for (const CellBatchPass& p : plan) {
+    at.push_back(total);
+    total += 2 * (p.b1 - p.b0) + 1;
+  }
+  if (!c->ev_bb) CU_TRY(cudaEventCreateWithFlags(&c->ev_bb, cudaEventDisableTiming));
+  CU_TRY(cudaEventSynchronize(c->ev_bb));
+  if (total > c->h_bb_cap) {
+    if (c->h_bb) cudaFreeHost(c->h_bb);
+    c->h_bb = nullptr;
+    c->h_bb_cap = 0;
+    CU_TRY(cudaMallocHost(&c->h_bb, total * sizeof(int)));
+    c->h_bb_cap = total;
+  }
+  for (size_t i = 0; i < plan.size(); i++) {
+    const CellBatchPass& p = plan[i];
+    int* o = c->h_bb + at[i];
+    int* slot = o + (p.b1 - p.b0) + 1;
+    int k = 0;
+    for (size_t b = p.b0; b <= p.b1; b++) o[b - p.b0] = (int)(offsets[b] - p.o0);
+    for (size_t b = p.b0; b < p.b1; b++) slot[b - p.b0] = offsets[b + 1] > offsets[b] ? k++ : -1;
+    n_ne.push_back(k);
+  }
+  CU_TRY(cudaMemcpyAsync(c->bb_boff.p, c->h_bb, total * sizeof(int), cudaMemcpyHostToDevice, st));
+  CU_TRY(cudaEventRecord(c->ev_bb, st));
+  return true;
+}
+
+// One pass on slot 0's stream (the point decompressions forked to its aux stream, beside the first blob hashes).  The
+// pass's blobs are d_blobs (device memory, read in place) or, with h_blobs, copied from the host into bb_blobs `stage`
+// blobs at a time (through the pinned ring when pageable); d_com / d_pi are its commitments and proofs on the device, its
+// offsets and slots are at d_boff.  d_ok, d_status (may be NULL) and d_rs receive its batches' verdicts, codes and
+// challenges.
+bool bb_enqueue_pass(Ctx* c, const CellBatchPass& p, const int* d_boff, int n_ne, const void* d_blobs, const Blob* h_blobs, bool pageable, size_t stage,
+                     const void* d_com, const void* d_pi, int* d_ok, int* d_status, void* d_rs) {
+  Slot& sl = c->slot[0];
+  cudaStream_t st = sl.st, aux = sl.aux;
+  const int nb = (int)(p.b1 - p.b0), m = (int)(p.o1 - p.o0);
+  const bool le = c->lagrange(), be = c->be_wire();
+  const int* d_slot = d_boff + nb + 1;
+  if (m == 0) {   // only empty batches
+    launch_fill_int(d_ok, le ? 1 : 0, nb, st);
+    if (d_status) launch_fill_int(d_status, C_KZG_OK, nb, st);
+    CU_TRY(cudaMemsetAsync(d_rs, 0, (size_t)nb * 32, st));
+    return true;
+  }
+  if (!h_blobs) stage = (size_t)m;
+  uint8_t* aff = (uint8_t*)c->bb_aff.p;   // C | pi
+  uint8_t* states = (uint8_t*)c->bb_states.p;
+  uint8_t* z = (uint8_t*)c->bb_zy.p;
+  uint8_t* y = z + (size_t)m * 32;
+  int* ist = (int*)c->bb_st.p;            // C | pi | blob words
+  CU_TRY(cudaEventRecord(sl.ev_in, st));
+  CU_TRY(cudaStreamWaitEvent(aux, sl.ev_in, 0));
+  launch_g1_decompress(aff, c->bb_c48r.p, ist, d_com, m, aux, le);
+  launch_g1_decompress(aff + (size_t)m * AFFINE_BYTES, c->bb_p48r.p, ist + m, d_pi, m, aux, le);
+  CU_TRY(cudaEventRecord(sl.ev_aux, aux));
+  if (le) CU_TRY(cudaMemsetAsync(ist + 2 * m, 0, (size_t)m * sizeof(int), st));
+  // the hash of z_i reads the commitment as given in the c-kzg modes, its canonical re-encoding in MODE_REFERENCE
+  const uint8_t* com_for_hash = le ? (const uint8_t*)d_com : (const uint8_t*)c->bb_c48r.p;
+  const size_t piece = pageable ? std::max<size_t>(c->ring.cap / BLOB_BYTES, 1) : stage;
+  for (size_t off = 0; off < (size_t)m; off += stage) {
+    const size_t k = std::min(stage, (size_t)m - off);
+    const uint8_t* blobs = h_blobs ? (const uint8_t*)c->bb_blobs.p : (const uint8_t*)d_blobs + off * BLOB_BYTES;
+    for (size_t q = 0; h_blobs && q < k; q += piece) {
+      const size_t w = std::min(piece, k - q);
+      if (pageable) {
+        if (!c->ring.h2d((uint8_t*)c->bb_blobs.p + q * BLOB_BYTES, h_blobs + p.o0 + off + q, w * BLOB_BYTES, c->ring_seq++, st)) return false;
+      } else {
+        CU_TRY(cudaMemcpyAsync((uint8_t*)c->bb_blobs.p + q * BLOB_BYTES, h_blobs + p.o0 + off + q, w * BLOB_BYTES, cudaMemcpyHostToDevice, st));
+      }
+    }
+    launch_challenge_midstate(states + off * 32, blobs, (int)k, st, true, be);
+    if (le) launch_le_blob_check(ist + 2 * m + off, blobs, (int)k, st, be);
+    if (off == 0) CU_TRY(cudaStreamWaitEvent(st, sl.ev_aux, 0));
+    launch_challenge_finish(z + off * 32, states + off * 32, blobs, com_for_hash + off * 48, (int)k, st, le && !be);
+    if (le) launch_le_eval_quot(nullptr, y + off * 32, nullptr, blobs, z + off * 32, c->d_roots, (int)k, st, be);
+    else launch_poly_eval_quot(nullptr, y + off * 32, nullptr, blobs, z + off * 32, (int)k, st);
+  }
+  launch_make_tuples(c->bb_tuples.p, c->bb_c48r.p, z, y, c->bb_p48r.p, m, st, le && !be);
+  launch_status_or(ist, ist + m, m, st);
+  if (le) launch_status_or(ist, ist + 2 * m, m, st);
+  launch_blob_batches_status((int*)c->bb_bst.p, ist, d_boff, nb, le ? C_KZG_BADARGS : C_KZG_ERROR, st);
+  launch_blob_batches_challenge(d_rs, c->bb_tuples.p, d_boff, nb, c->mode, st);
+  // G of a one-blob batch as verify_single_from_workspace chooses it: c-kzg's generator, the reference's g1_values[0]
+  launch_blob_batches_msm(c->bb_out.p, c->bb_terms.p, c->bb_sc.p, d_rs, z, y, aff, aff + (size_t)m * AFFINE_BYTES, le ? c->d_gen : c->d_srs,
+                          le || c->srs_in_g1, d_boff, d_slot, m, nb, st);
+  launch_batch_final_each((int*)c->bb_pok.p, c->bb_out.p, n_ne, c->d_prep0, c->d_prep1, st);
+  // an empty batch: the reference rejects it (lib.rs:538-543), c-kzg accepts it
+  launch_blob_batches_fold(d_ok, d_status, (const int*)c->bb_pok.p, (const int*)c->bb_bst.p, d_slot, nb, le, st);
+  return true;
+}
+
+long bb_ring_blobs() {
+  std::lock_guard<std::mutex> lk(g_mu);
+  return std::max(1L, opts().chunk_blobs);
+}
+
+C_KZG_RET blob_batches_host(bool* ok, const Blob* blobs, const Bytes48* commitments, const Bytes48* proofs, const uint64_t* offsets, size_t nb,
+                            const KZGSettings* s, int* status) {
+  if (nb == 0) return C_KZG_OK;
+  if (!ok || !offsets) { set_err("null argument"); return C_KZG_BADARGS; }
+  Ctx* c = ctx_of(s);
+  if (!c) return C_KZG_ERROR;
+  size_t total = 0;
+  if (C_KZG_RET rc = cell_batches_check(offsets, nb, blobs && commitments && proofs, 1, &total)) return rc;
+  std::vector<uint8_t> rs(nb * 32, 0);
+  if (total == 0) {   // only empty batches: each gets the single call's verdict for an empty batch
+    for (size_t b = 0; b < nb; b++) {
+      ok[b] = c->lagrange();
+      if (status) status[b] = C_KZG_OK;
+    }
+  } else {
+    if (!c->g2_valid && c->srs_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
+    const size_t super = vb_super_blobs();
+    C_KZG_RET rc = sharded_batch(c, nb, status, "invalid commitment, proof or blob", [&](Ctx* x, size_t first, size_t cnt, int* st) -> C_KZG_RET {
+      CtxLock lock(x);
+      const std::vector<CellBatchPass> plan = cell_batch_passes(offsets, first, cnt, super);
+      if (!reserve(bb_buffers(x, plan, cnt, super, true))) return C_KZG_ERROR;
+      size_t max_m = 0;
+      for (const CellBatchPass& p : plan) max_m = std::max(max_m, p.o1 - p.o0);
+      const size_t shard_blobs = (size_t)(offsets[first + cnt] - offsets[first]);
+      const bool pageable = shard_blobs * BLOB_BYTES >= (size_t(4) << 20) && is_pageable_host(blobs) &&
+                            x->ring.ensure(std::min<size_t>(std::min(max_m, super), (size_t)bb_ring_blobs()) * BLOB_BYTES);
+      cudaStream_t s0 = x->slot[0].st;
+      std::vector<size_t> at;
+      std::vector<int> n_ne;
+      if (!bb_stage_offsets(x, plan, offsets, at, n_ne, s0)) return C_KZG_ERROR;
+      std::vector<int> h_io;
+      for (size_t i = 0; i < plan.size(); i++) {
+        const CellBatchPass& p = plan[i];
+        const size_t m = p.o1 - p.o0, k = p.b1 - p.b0;
+        uint8_t* in = (uint8_t*)x->bb_in.p;   // C | pi
+        int* d_io = (int*)x->bb_io.p;         // ok | status
+        uint8_t* d_rs = (uint8_t*)x->bb_rs.p + (p.b0 - first) * 32;
+        h_io.resize(2 * k);
+        bool good = [&]() -> bool {
+          if (m) {
+            CU_TRY(cudaMemcpyAsync(in, commitments + p.o0, m * 48, cudaMemcpyHostToDevice, s0));
+            CU_TRY(cudaMemcpyAsync(in + m * 48, proofs + p.o0, m * 48, cudaMemcpyHostToDevice, s0));
+          }
+          if (!bb_enqueue_pass(x, p, (const int*)x->bb_boff.p + at[i], n_ne[i], nullptr, blobs, pageable, super, in, in + m * 48, d_io, d_io + k, d_rs))
+            return false;
+          CU_TRY(cudaMemcpyAsync(h_io.data(), d_io, 2 * k * sizeof(int), cudaMemcpyDeviceToHost, s0));
+          CU_TRY(cudaMemcpyAsync(rs.data() + p.b0 * 32, d_rs, k * 32, cudaMemcpyDeviceToHost, s0));
+          CU_TRY(cudaStreamSynchronize(s0));
+          CU_TRY(cudaGetLastError());
+          return true;
+        }();
+        if (!good) {
+          cudaStreamSynchronize(x->slot[0].aux);
+          return C_KZG_ERROR;
+        }
+        for (size_t j = 0; j < k; j++) {
+          ok[p.b0 + j] = h_io[j] != 0;
+          st[p.b0 - first + j] = h_io[k + j];
+        }
+      }
+      return C_KZG_OK;
+    });
+    if (rc != C_KZG_OK) return rc;
+  }
+  CtxLock lock(c);
+  c->bb_h_rs = std::move(rs);
+  c->bb_rs_n = nb;
+  c->bb_rs_on_host = true;
+  return C_KZG_OK;
+}
+
+// the device form: asynchronous, ordered after and before `user`; the host waits for earlier work only when a buffer
+// has to grow (which frees the old one)
+C_KZG_RET blob_batches_device(void* d_ok, const void* d_blobs, const void* d_com, const void* d_pi, const uint64_t* offsets, size_t nb, const KZGSettings* s,
+                              cudaStream_t user, void* d_status) {
+  if (nb == 0) return C_KZG_OK;
+  if (!d_ok || !offsets) { set_err("null argument"); return C_KZG_BADARGS; }
+  Ctx* c = ctx_of(s);
+  if (!c) return C_KZG_ERROR;
+  size_t total = 0;
+  if (C_KZG_RET rc = cell_batches_check(offsets, nb, d_blobs && d_com && d_pi, 1, &total)) return rc;
+  if (total == 0) {   // only empty batches
+    CtxLock lock(c);
+    c->bb_h_rs.assign(nb * 32, 0);
+    c->bb_rs_n = nb;
+    c->bb_rs_on_host = true;
+    launch_fill_int((int*)d_ok, c->lagrange() ? 1 : 0, (int)nb, user);
+    if (d_status) launch_fill_int((int*)d_status, C_KZG_OK, (int)nb, user);
+    if (cudaGetLastError() != cudaSuccess) { set_err("launch failed"); return C_KZG_ERROR; }
+    return C_KZG_OK;
+  }
+  if (!c->srs_valid || !c->g2_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
+  CtxLock lock(c);
+  Slot& sl = c->slot[0];
+  const std::vector<CellBatchPass> plan = cell_batch_passes(offsets, 0, nb, vb_super_blobs());
+  const BufList bufs = bb_buffers(c, plan, nb, 0, false);
+  if (!fits(bufs)) {
+    cudaStreamSynchronize(sl.st);
+    cudaStreamSynchronize(sl.aux);
+  }
+  if (!reserve(bufs)) return C_KZG_ERROR;
+  c->bb_rs_n = nb;
+  c->bb_rs_on_host = false;
+  bool good = [&]() -> bool {
+    CU_TRY(cudaEventRecord(sl.ev_fork, user));
+    CU_TRY(cudaStreamWaitEvent(sl.st, sl.ev_fork, 0));
+    std::vector<size_t> at;
+    std::vector<int> n_ne;
+    if (!bb_stage_offsets(c, plan, offsets, at, n_ne, sl.st)) return false;
+    for (size_t i = 0; i < plan.size(); i++) {
+      const CellBatchPass& p = plan[i];
+      if (!bb_enqueue_pass(c, p, (const int*)c->bb_boff.p + at[i], n_ne[i], (const uint8_t*)d_blobs + p.o0 * BLOB_BYTES, nullptr, false, 0,
+                           (const uint8_t*)d_com + p.o0 * 48, (const uint8_t*)d_pi + p.o0 * 48, (int*)d_ok + p.b0, d_status ? (int*)d_status + p.b0 : nullptr,
+                           (uint8_t*)c->bb_rs.p + p.b0 * 32))
+        return false;
+    }
+    CU_TRY(cudaEventRecord(sl.ev_done, sl.st));
+    CU_TRY(cudaStreamWaitEvent(user, sl.ev_done, 0));
+    CU_TRY(cudaGetLastError());
+    return true;
+  }();
+  return good ? C_KZG_OK : C_KZG_ERROR;
+}
+
+C_KZG_RET blob_batches_debug_challenges(uint8_t* out32, size_t nb, const KZGSettings* s) {
+  Ctx* c = ctx_of(s);
+  if (!c || !out32) return C_KZG_ERROR;
+  CtxLock lock(c);
+  if (nb > c->bb_rs_n) { set_err("no such batch in the last call"); return C_KZG_BADARGS; }
+  if (nb == 0) return C_KZG_OK;
+  if (c->bb_rs_on_host) {
+    memcpy(out32, c->bb_h_rs.data(), nb * 32);
+    return C_KZG_OK;
+  }
+  if (cudaStreamSynchronize(c->slot[0].st) != cudaSuccess || cudaMemcpy(out32, c->bb_rs.p, nb * 32, cudaMemcpyDeviceToHost) != cudaSuccess) {
+    set_err("D2H failed");
+    return C_KZG_ERROR;
+  }
+  return C_KZG_OK;
+}
+
 }  // namespace
 
 // =================================================================== C ABI
@@ -1869,6 +2155,18 @@ C_KZG_RET lwkzg_verify_kzg_proofs(bool* ok, const Bytes48* commitments, const By
 C_KZG_RET lwkzg_verify_kzg_proofs_device(void* d_ok, const void* d_commitments, const void* d_zs, const void* d_ys, const void* d_proofs, size_t n,
                                          const KZGSettings* s, void* stream, void* d_status) {
   return verify_proofs_device(d_ok, d_commitments, d_zs, d_ys, d_proofs, n, s, (cudaStream_t)stream, d_status);
+}
+
+C_KZG_RET lwkzg_verify_blob_kzg_proof_batches(bool* ok, const Blob* blobs, const Bytes48* commitments, const Bytes48* proofs, const uint64_t* offsets,
+                                              size_t n_batches, const KZGSettings* s, int* status) {
+  return blob_batches_host(ok, blobs, commitments, proofs, offsets, n_batches, s, status);
+}
+C_KZG_RET lwkzg_verify_blob_kzg_proof_batches_device(void* d_ok, const void* d_blobs, const void* d_commitments, const void* d_proofs,
+                                                     const uint64_t* offsets, size_t n_batches, const KZGSettings* s, void* stream, void* d_status) {
+  return blob_batches_device(d_ok, d_blobs, d_commitments, d_proofs, offsets, n_batches, s, (cudaStream_t)stream, d_status);
+}
+C_KZG_RET lwkzg_debug_blob_batch_challenges(uint8_t* out32, size_t n_batches, const KZGSettings* s) {
+  return blob_batches_debug_challenges(out32, n_batches, s);
 }
 
 static C_KZG_RET verify_blob_single(bool* ok, const Blob* blob, const Bytes48* commitment_bytes, const Bytes48* proof_bytes, const KZGSettings* s,

@@ -12,6 +12,7 @@
 #include <algorithm>
 
 #include "kernels.h"
+#include "batch_challenge.cuh"
 #include "pairing_warp.cuh"
 #include "sha256.cuh"
 
@@ -148,73 +149,15 @@ __global__ void make_tuples_kernel(uint8_t* __restrict__ tuples, const uint8_t* 
   for (int k = 0; k < 48; k++) t[112 + k] = pi48[(size_t)i * 48 + k];
 }
 
-// r = H("RCKZGBATCH___V1_" || le64(4096) || le64(n) || tuples), read big-endian, mod r.
-// One SHA-256 stream: the warp expands message schedules in parallel, lane 0 runs the rounds.
-//
-// The hash is sequential, but its input becomes available chunk by chunk while a batch is being prepared
-// (tuple i exists as soon as blob i has been copied, hashed and evaluated), so the kernel works on a block
-// range of the message: [blk0, blk1) 64-byte blocks, state carried in `state` between launches
-// (FLAG_INIT: start from the SHA-256 IV; FLAG_FINAL: also absorb everything after blk1 -- the remaining
-// full blocks and the padded tail -- and write r).  One launch with both flags and blk0 = blk1 = 0 is
-// the monolithic hash.
-constexpr int BCH_INIT = 1, BCH_FINAL = 2, BCH_LE = 4, BCH_BE_HDR = 8;
+// The batch challenge over one batch (batch_challenge.cuh).  Its input becomes available chunk by chunk while a batch
+// is being prepared (tuple i exists as soon as blob i has been copied, hashed and evaluated), so the kernel works on a
+// block range of the message: [blk0, blk1) 64-byte blocks, state carried in `state` between launches.  One launch with
+// BCH_INIT | BCH_FINAL and blk0 = blk1 = 0 is the monolithic hash.
 __global__ void __launch_bounds__(32) batch_challenge_kernel(uint32_t* __restrict__ r_out, Sha256State* __restrict__ state, const uint8_t* __restrict__ tuples,
                                                               unsigned long long n_total, int blk0, int blk1, int flags) {
   __shared__ uint32_t wk[64 * 32];
   __shared__ uint8_t head[32];
-  const int lane = threadIdx.x;
-  if (lane == 0) {
-    const char dom[17] = "RCKZGBATCH___V1_";
-    for (int i = 0; i < 16; i++) head[i] = (uint8_t)dom[i];
-    for (int i = 0; i < 8; i++) head[16 + i] = 0;
-    if (flags & BCH_BE_HDR) {   // MODE_DENEB: be64(4096) || be64(n)
-      head[22] = 0x10;
-      for (int i = 0; i < 8; i++) head[24 + i] = (uint8_t)(n_total >> (8 * (7 - i)));
-    } else {
-      head[17] = 0x10;  // le64(4096)
-      for (int i = 0; i < 8; i++) head[24 + i] = (uint8_t)(n_total >> (8 * i));
-    }
-  }
-  __syncwarp();
-  const unsigned long long total = 32ull + 160ull * n_total;
-  const int nfull = (int)(total / 64);
-  if (flags & BCH_FINAL) blk1 = nfull;
-  auto byte_at = [&](unsigned long long off) -> uint8_t { return off < 32 ? head[off] : tuples[off - 32]; };
-  Sha256State s;
-  if (flags & BCH_INIT) sha256_init(s); else s = *state;
-  sha256_warp_blocks(s, blk1 - blk0, [&](int rel, uint32_t* w) {
-    const int blk = blk0 + rel;
-    unsigned long long off = 64ull * blk;
-    if (blk >= 1) {
-      const uint32_t* src = reinterpret_cast<const uint32_t*>(tuples + (off - 32));  // 32-byte aligned
-      for (int i = 0; i < 16; i++) w[i] = bswap32(src[i]);
-    } else {
-      for (int i = 0; i < 16; i++)
-        w[i] = ((uint32_t)byte_at(off + 4 * i) << 24) | ((uint32_t)byte_at(off + 4 * i + 1) << 16) | ((uint32_t)byte_at(off + 4 * i + 2) << 8) | byte_at(off + 4 * i + 3);
-    }
-  }, wk);
-  if (lane != 0) return;
-  if (!(flags & BCH_FINAL)) { *state = s; return; }
-  uint32_t w[16];
-  unsigned long long off = 64ull * nfull;
-  uint8_t tail[128];
-  int rem = (int)(total - off);
-  for (int i = 0; i < rem; i++) tail[i] = byte_at(off + i);
-  tail[rem] = 0x80;
-  int tl = (rem + 9 <= 64) ? 64 : 128;
-  for (int i = rem + 1; i < tl; i++) tail[i] = 0;
-  unsigned long long bits = total * 8ull;
-  for (int i = 0; i < 8; i++) tail[tl - 1 - i] = (uint8_t)(bits >> (8 * i));
-  for (int o = 0; o < tl; o += 64) {
-    for (int i = 0; i < 16; i++)
-      w[i] = ((uint32_t)tail[o + 4 * i] << 24) | ((uint32_t)tail[o + 4 * i + 1] << 16) | ((uint32_t)tail[o + 4 * i + 2] << 8) | tail[o + 4 * i + 3];
-    sha256_compress(s, w);
-  }
-  const int le = flags & BCH_LE;
-  Fr r;
-  for (int i = 0; i < 8; i++) r.l[i] = le ? bswap32(s.h[i]) : s.h[7 - i];
-  mod_reduce_small<FrCfg, 2>(r.l);
-  for (int i = 0; i < 8; i++) r_out[i] = r.l[i];
+  batch_challenge_warp(r_out, state, tuples, n_total, blk0, blk1, flags, wk, head);
 }
 
 // XYZZ block reduction helpers (same SoA shared-memory layout as msm.cu)
@@ -377,7 +320,6 @@ void launch_make_tuples(void* d_tuples160, const void* d_c48, const void* d_z, c
                                                   le ? 1 : 0);
   count_launch();
 }
-static int bch_wire_flags(int wire) { return wire == 1 ? BCH_LE : wire == 2 ? BCH_BE_HDR : 0; }
 // (measured and not kept: giving this one-warp kernel an SM of its own by asking for all of the SM's shared memory --
 // no change; what slowed the device-resident batch was eight chunk streams at once, see "verify_streams")
 void launch_batch_challenge(void* d_r, const void* d_tuples160, size_t n_total, cudaStream_t st, int wire) {
