@@ -300,6 +300,18 @@ def verify_blob_kzg_proof_batch_device(d_blobs: int, d_commitments: int, d_proof
     return bool(ok.value)
 
 
+def _offsets(offsets: Sequence[int]):
+    """The K + 1 batch offsets of a per-batch call as the uint64 array the C calls take."""
+    return (ctypes.c_uint64 * max(1, len(offsets)))(*offsets)
+
+
+def _debug_challenges(fn: str, n_batches: int, s) -> List[int]:
+    """The 32-byte little-endian challenges of the last call of a per-batch family, read by the C test hook `fn`."""
+    out = ctypes.create_string_buffer(32 * max(1, n_batches))
+    _check(getattr(load_library(), fn)(out, n_batches, _sp(s)), fn)
+    return [int.from_bytes(out.raw[32 * i: 32 * i + 32], "little") for i in range(n_batches)]
+
+
 def verify_blob_kzg_proof_batches(batches: Sequence[Tuple[Sequence[bytes], Sequence[bytes], Sequence[bytes]]], s) -> Tuple[List[bool], List[int]]:
     """K independent verify_blob_kzg_proof_batch checks in one call.  batches: (blobs, commitments, proofs) per batch ->
     (verdict list, status list): per batch, what verify_blob_kzg_proof_batch over that batch alone returns."""
@@ -308,7 +320,7 @@ def verify_blob_kzg_proof_batches(batches: Sequence[Tuple[Sequence[bytes], Seque
     for bl, com, pr in batches:
         assert len(bl) == len(com) == len(pr)
         offsets.append(offsets[-1] + len(bl))
-    off = (ctypes.c_uint64 * (k + 1))(*offsets)
+    off = _offsets(offsets)
     oks = (ctypes.c_bool * max(1, k))()
     st = _status_list(k)
     _check(load_library().lwkzg_verify_blob_kzg_proof_batches(oks, b"".join(_cat(b[0], BYTES_PER_BLOB) for b in batches) or b"\0",
@@ -323,7 +335,7 @@ def verify_blob_kzg_proof_batches_device(d_ok: int, d_blobs: int, d_commitments:
     """All buffers are raw device addresses (torch: tensor.data_ptr()) except offsets (K + 1 host integers, in blobs);
     d_ok and d_status (0 = not wanted) are K int32 each.  Asynchronous on `stream`."""
     k = len(offsets) - 1
-    off = (ctypes.c_uint64 * max(1, k + 1))(*offsets)
+    off = _offsets(offsets)
     _check(load_library().lwkzg_verify_blob_kzg_proof_batches_device(d_ok or None, d_blobs or None, d_commitments or None, d_proofs or None, off, k,
                                                                      _sp(s), stream or None, d_status or None),
            "lwkzg_verify_blob_kzg_proof_batches_device")
@@ -332,9 +344,7 @@ def verify_blob_kzg_proof_batches_device(d_ok: int, d_blobs: int, d_commitments:
 def debug_blob_batch_challenges(n_batches: int, s) -> List[int]:
     """The challenges r_b the last verify_blob_kzg_proof_batches[_device] call derived (0 for batches of fewer than two
     blobs; test hook)."""
-    out = ctypes.create_string_buffer(32 * max(1, n_batches))
-    _check(load_library().lwkzg_debug_blob_batch_challenges(out, n_batches, _sp(s)), "lwkzg_debug_blob_batch_challenges")
-    return [int.from_bytes(out.raw[32 * i: 32 * i + 32], "little") for i in range(n_batches)]
+    return _debug_challenges("lwkzg_debug_blob_batch_challenges", n_batches, s)
 
 
 # ------------------------------------------------------------------ batch extensions (host buffers)
@@ -642,7 +652,7 @@ def verify_cell_kzg_proof_batches(batches: Sequence[Tuple[Sequence[bytes], Seque
         offsets.append(offsets[-1] + len(idx))
     n = offsets[-1]
     idx = (ctypes.c_uint64 * max(1, n))(*[i for b in batches for i in b[1]])
-    off = (ctypes.c_uint64 * (k + 1))(*offsets)
+    off = _offsets(offsets)
     oks = (ctypes.c_bool * max(1, k))()
     st = _status_list(k)
     _check(load_library().lwkzg_verify_cell_kzg_proof_batches(oks, b"".join(_cat(b[0], 48) for b in batches) or b"\0", idx,
@@ -657,7 +667,7 @@ def verify_cell_kzg_proof_batches_device(d_ok: int, d_commitments: int, d_cell_i
     """All buffers are raw device addresses (torch: tensor.data_ptr()) except offsets (K + 1 host integers); d_ok and
     d_status are K int32 each.  Asynchronous on `stream`."""
     k = len(offsets) - 1
-    off = (ctypes.c_uint64 * max(1, k + 1))(*offsets)
+    off = _offsets(offsets)
     _check(load_library().lwkzg_verify_cell_kzg_proof_batches_device(d_ok or None, d_commitments or None, d_cell_indices or None, d_cells or None,
                                                                      d_proofs or None, off, k, _sp(s), stream or None, d_status or None),
            "lwkzg_verify_cell_kzg_proof_batches_device")
@@ -672,7 +682,7 @@ def verify_blob_cell_kzg_proof_batches(batches: Sequence[Tuple[Sequence[bytes], 
     for bl, com, pr in batches:
         assert len(bl) == len(com) and len(pr) == CELLS_PER_EXT_BLOB * len(bl)
         offsets.append(offsets[-1] + len(bl))
-    off = (ctypes.c_uint64 * (k + 1))(*offsets)
+    off = _offsets(offsets)
     oks = (ctypes.c_bool * max(1, k))()
     st = _status_list(k)
     _check(load_library().lwkzg_verify_blob_cell_kzg_proof_batches(oks, b"".join(_cat(b[0], BYTES_PER_BLOB) for b in batches) or b"\0",
@@ -687,7 +697,7 @@ def verify_blob_cell_kzg_proof_batches_device(d_ok: int, d_blobs: int, d_commitm
     """All buffers are raw device addresses except offsets (K + 1 host integers, in blobs); d_ok and d_status are K
     int32 each.  Asynchronous on `stream`."""
     k = len(offsets) - 1
-    off = (ctypes.c_uint64 * max(1, k + 1))(*offsets)
+    off = _offsets(offsets)
     _check(load_library().lwkzg_verify_blob_cell_kzg_proof_batches_device(d_ok or None, d_blobs or None, d_commitments or None, d_proofs or None, off, k,
                                                                           _sp(s), stream or None, d_status or None),
            "lwkzg_verify_blob_cell_kzg_proof_batches_device")
@@ -695,9 +705,7 @@ def verify_blob_cell_kzg_proof_batches_device(d_ok: int, d_blobs: int, d_commitm
 
 def debug_cell_batch_challenges(n_batches: int, s) -> List[int]:
     """The challenges r_b the last verify_[blob_]cell_kzg_proof_batches[_device] call derived (0 for empty batches; test hook)."""
-    out = ctypes.create_string_buffer(32 * max(1, n_batches))
-    _check(load_library().lwkzg_debug_cell_batch_challenges(out, n_batches, _sp(s)), "lwkzg_debug_cell_batch_challenges")
-    return [int.from_bytes(out.raw[32 * i: 32 * i + 32], "little") for i in range(n_batches)]
+    return _debug_challenges("lwkzg_debug_cell_batch_challenges", n_batches, s)
 
 
 def cell_window_bits(s) -> int:

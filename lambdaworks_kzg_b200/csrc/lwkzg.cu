@@ -127,6 +127,41 @@ bool fits(const BufList& bufs) {
   return true;
 }
 
+// A stream that device-buffer work runs on, with an event of its own for the fork from the caller's stream and the
+// join back into it.
+struct Lane {
+  cudaStream_t st;
+  cudaEvent_t ev;
+};
+
+// Device-buffer work, asynchronous with respect to the host and ordered after and before the caller's stream `user`.
+// bufs is reserved first: the host waits for the `drain` streams only when a buffer has to grow (which frees the old
+// one), so back-to-back calls queue behind each other.  Every lane then waits for `user`, body() enqueues the work on
+// the lanes, and `user` waits for every lane -- also after a failed enqueue, so that the caller's stream never runs
+// ahead of work that still writes the caller's buffers.
+template <class Body>
+C_KZG_RET on_lanes(cudaStream_t user, const std::vector<Lane>& lanes, const std::vector<cudaStream_t>& drain, const BufList& bufs, const Body& body) {
+  if (!fits(bufs))
+    for (cudaStream_t s : drain) cudaStreamSynchronize(s);
+  if (!reserve(bufs)) return C_KZG_ERROR;
+  const bool good = [&]() -> bool {
+    for (const Lane& l : lanes) {
+      CU_TRY(cudaEventRecord(l.ev, user));
+      CU_TRY(cudaStreamWaitEvent(l.st, l.ev, 0));
+    }
+    return body();
+  }();
+  const bool joined = [&]() -> bool {
+    for (const Lane& l : lanes) {
+      CU_TRY(cudaEventRecord(l.ev, l.st));
+      CU_TRY(cudaStreamWaitEvent(user, l.ev, 0));
+    }
+    if (good) CU_TRY(cudaGetLastError());
+    return true;
+  }();
+  return good && joined ? C_KZG_OK : C_KZG_ERROR;
+}
+
 // ------------------------------------------------------------------ pageable host buffers
 // A c-kzg caller passes ordinary (pageable) memory.  cudaMemcpyAsync from pageable memory is a synchronous, single-
 // threaded staged copy inside the driver (~11 GB/s measured: 512 MiB of blobs in 46 ms against 9.8 ms from pinned
@@ -245,6 +280,24 @@ struct PinnedRing {   // per context: RING_SLOTS pinned buffers of one pipeline 
   }
 };
 
+// The per-batch workspace of a family of per-batch verification calls (batches_host): the offsets of a call's passes
+// on the device and their pinned staging (rewritten once ev_boff, its last copy, has completed), the verdicts and
+// codes of a host-buffer pass (ok | status), the challenges of the call's batches, and the last call's challenges for
+// the test hooks (gathered on the host by host-buffer calls and calls of empty batches only).
+struct BatchWs {
+  DevBuf boff, io, rs;
+  int* h_boff = nullptr;
+  size_t h_boff_cap = 0;
+  cudaEvent_t ev_boff = nullptr;
+  std::vector<uint8_t> h_rs;
+  size_t rs_n = 0;
+  bool rs_on_host = false;
+  ~BatchWs() {
+    if (ev_boff) { cudaEventSynchronize(ev_boff); cudaEventDestroy(ev_boff); }
+    if (h_boff) cudaFreeHost(h_boff);
+  }
+};
+
 constexpr uint64_t CTX_MAGIC = 0x4c574b5a47423230ull;  // "LWKZGB20"
 constexpr int NSLOT = 4;
 
@@ -294,16 +347,10 @@ struct Ctx {
   // per-item statuses, verdicts
   DevBuf vp_in, vp_aff, vp_zy, vp_pts, vp_st, vp_io;
   // lwkzg_verify_blob_kzg_proof_batches, one pass: per blob (inputs and staged blobs of host-buffer calls, points,
-  // re-encodings, hash states, z | y, tuples, statuses), per term (scalars, products), per batch (offsets and partial
-  // slots of every pass, statuses, partials, pairing results, verdicts), the challenges of the call; the offsets are
-  // staged in pinned memory (h_bb, rewritten once the copy ev_bb marks has completed)
-  DevBuf bb_in, bb_blobs, bb_aff, bb_c48r, bb_p48r, bb_states, bb_zy, bb_tuples, bb_st, bb_sc, bb_terms, bb_boff, bb_bst, bb_out, bb_pok, bb_io, bb_rs;
-  int* h_bb = nullptr;
-  size_t h_bb_cap = 0;
-  cudaEvent_t ev_bb = nullptr;
-  std::vector<uint8_t> bb_h_rs;   // the last call's challenges, when they came back to the host
-  size_t bb_rs_n = 0;
-  bool bb_rs_on_host = true;
+  // re-encodings, hash states, z | y, tuples, statuses), per term (scalars, products), per batch (statuses, partials,
+  // pairing results); its offsets, verdicts and challenges are in bb
+  DevBuf bb_in, bb_blobs, bb_aff, bb_c48r, bb_p48r, bb_states, bb_zy, bb_tuples, bb_st, bb_sc, bb_terms, bb_bst, bb_out, bb_pok;
+  BatchWs bb;
   // pinned host staging for batch results: a D2H copy into pageable memory would block the host
   // until the chunk's kernels finish and serialise the two pipeline slots
   void* h_stage = nullptr;
@@ -414,8 +461,6 @@ void destroy_ctx(Ctx* c) {
   if (c->d_roots) cudaFree(c->d_roots);
   if (c->d_gen) cudaFree(c->d_gen);
   if (c->h_stage) cudaFreeHost(c->h_stage);
-  if (c->ev_bb) { cudaEventSynchronize(c->ev_bb); cudaEventDestroy(c->ev_bb); }
-  if (c->h_bb) cudaFreeHost(c->h_bb);
   c->ring.release();
   c->magic = 0;
   delete c;
@@ -1117,48 +1162,35 @@ C_KZG_RET device_batch(Mode mode, const KZGSettings* s, size_t n, const void* d_
     plan.emplace_back(off, m);
     off += m;
   }
-  // The host only waits for earlier work when a buffer really has to grow: back-to-back calls (also from
-  // different user streams) then queue behind each other on the slot streams and the tail of one batch
-  // overlaps the head of the next.
-  std::vector<BufList> bufs;
-  bool all_fit = true;
+  BufList bufs;
   for (size_t k = 0; k < plan.size(); k++) {
-    bufs.push_back(slot_buffers(c->slot[k % NSLOT], (int)plan[k].second, auto_bpb((int)plan[k].second), false));
-    all_fit = all_fit && fits(bufs.back());
+    const BufList b = slot_buffers(c->slot[k % NSLOT], (int)plan[k].second, auto_bpb((int)plan[k].second), false);
+    bufs.insert(bufs.end(), b.begin(), b.end());
   }
-  if (!all_fit) {
-    for (auto& sl : c->slot) { cudaStreamSynchronize(sl.st); cudaStreamSynchronize(sl.aux); }
-    for (const BufList& b : bufs)
-      if (!reserve(b)) return C_KZG_ERROR;
+  std::vector<Lane> lanes;
+  std::vector<cudaStream_t> drain;
+  for (Slot& sl : c->slot) {
+    lanes.push_back({sl.st, sl.ev_done});
+    drain.insert(drain.end(), {sl.st, sl.aux});
   }
-  cudaEvent_t ev_user;
-  if (cudaEventCreateWithFlags(&ev_user, cudaEventDisableTiming) != cudaSuccess) { set_err("event"); return C_KZG_ERROR; }
-  cudaEventRecord(ev_user, user);
-  for (auto& sl : c->slot) cudaStreamWaitEvent(sl.st, ev_user, 0);
-  size_t k = 0;
-  bool ok = true;
-  for (; k < plan.size() && ok; k++) {
-    const size_t off = plan[k].first;
-    const int m = (int)plan[k].second;
-    Slot& sl = c->slot[k % NSLOT];
-    const uint8_t* b = (const uint8_t*)d_blobs + off * BLOB_BYTES;
-    void* co = d_c_out ? (uint8_t*)d_c_out + off * 48 : (mode == Mode::CommitProve ? sl.c48.p : nullptr);
-    void* po = d_p_out ? (uint8_t*)d_p_out + off * 48 : nullptr;
-    const void* ci = d_commit_in ? (const uint8_t*)d_commit_in + off * 48 : nullptr;
-    int* so = d_status ? (int*)d_status + off : (int*)sl.status.p;
-    ok = enqueue_chunk(c, sl, mode, b, m, co, po, nullptr, so, ci, nullptr);
-    if (ok && (mode == Mode::BlobProof || c->lagrange())) {   // the only ways an item can fail: bad commitment / non-canonical blob
-      if (co && d_c_out) launch_zero_failed(co, 48, so, m, sl.st);
-      if (po) launch_zero_failed(po, 48, so, m, sl.st);
+  return on_lanes(user, lanes, drain, bufs, [&]() -> bool {
+    for (size_t k = 0; k < plan.size(); k++) {
+      const size_t off = plan[k].first;
+      const int m = (int)plan[k].second;
+      Slot& sl = c->slot[k % NSLOT];
+      const uint8_t* b = (const uint8_t*)d_blobs + off * BLOB_BYTES;
+      void* co = d_c_out ? (uint8_t*)d_c_out + off * 48 : (mode == Mode::CommitProve ? sl.c48.p : nullptr);
+      void* po = d_p_out ? (uint8_t*)d_p_out + off * 48 : nullptr;
+      const void* ci = d_commit_in ? (const uint8_t*)d_commit_in + off * 48 : nullptr;
+      int* so = d_status ? (int*)d_status + off : (int*)sl.status.p;
+      if (!enqueue_chunk(c, sl, mode, b, m, co, po, nullptr, so, ci, nullptr)) return false;
+      if (mode == Mode::BlobProof || c->lagrange()) {   // the only ways an item can fail: bad commitment / non-canonical blob
+        if (co && d_c_out) launch_zero_failed(co, 48, so, m, sl.st);
+        if (po) launch_zero_failed(po, 48, so, m, sl.st);
+      }
     }
-  }
-  for (auto& sl : c->slot) {
-    cudaEventRecord(sl.ev_done, sl.st);
-    cudaStreamWaitEvent(user, sl.ev_done, 0);
-  }
-  cudaEventDestroy(ev_user);
-  if (!ok || cudaGetLastError() != cudaSuccess) { if (ok) set_err("CUDA launch failure"); return C_KZG_ERROR; }
-  return C_KZG_OK;
+    return true;
+  });
 }
 
 // ------------------------------------------------------------------ setup loading
@@ -1554,6 +1586,19 @@ struct CtxLock {
   explicit CtxLock(Ctx* ctx) : c(ctx), lk(ctx->mu), dg(ctx->device) {}
 };
 
+// The verdicts and codes of m items that work on st leaves in d_io (ok | status), into ok[m] and status[m] once st is done
+bool fetch_verdicts(bool* ok, int* status, const int* d_io, size_t m, cudaStream_t st) {
+  std::vector<int> h(2 * m);
+  CU_TRY(cudaMemcpyAsync(h.data(), d_io, 2 * m * sizeof(int), cudaMemcpyDeviceToHost, st));
+  CU_TRY(cudaStreamSynchronize(st));
+  CU_TRY(cudaGetLastError());
+  for (size_t i = 0; i < m; i++) {
+    ok[i] = h[i] != 0;
+    status[i] = h[m + i];
+  }
+  return true;
+}
+
 // ------------------------------------------------------------------ lwkzg_verify_kzg_proofs
 // n independent verify_kzg_proof checks in passes of at most VP_PASS items, so device memory stays bounded whatever n
 // is (about 0.6 KB per item of a pass).  A pass is a fixed launch sequence on one stream: decode C and pi (r-torsion
@@ -1605,35 +1650,24 @@ C_KZG_RET verify_proofs_host(bool* ok, const Bytes48* commitments, const Bytes32
     CtxLock lock(x);
     if (!reserve(vp_buffers(x, std::min(cnt, VP_PASS), true))) return C_KZG_ERROR;
     cudaStream_t s0 = x->slot[0].st;
-    std::vector<int> h_io;
     for (size_t off = 0; off < cnt; off += VP_PASS) {
       const size_t m = std::min(VP_PASS, cnt - off), i0 = first + off;
       uint8_t* in = (uint8_t*)x->vp_in.p;   // C | pi | z | y
       int* d_io = (int*)x->vp_io.p;         // ok | status
-      h_io.resize(2 * m);
-      bool good = [&]() -> bool {
+      const bool good = [&]() -> bool {
         CU_TRY(cudaMemcpyAsync(in, commitments + i0, m * 48, cudaMemcpyHostToDevice, s0));
         CU_TRY(cudaMemcpyAsync(in + m * 48, proofs + i0, m * 48, cudaMemcpyHostToDevice, s0));
         CU_TRY(cudaMemcpyAsync(in + m * 96, zs + i0, m * 32, cudaMemcpyHostToDevice, s0));
         CU_TRY(cudaMemcpyAsync(in + m * 128, ys + i0, m * 32, cudaMemcpyHostToDevice, s0));
-        if (!vp_enqueue_pass(x, (int)m, in, in + m * 96, in + m * 128, in + m * 48, d_io, d_io + m, s0)) return false;
-        CU_TRY(cudaMemcpyAsync(h_io.data(), d_io, 2 * m * sizeof(int), cudaMemcpyDeviceToHost, s0));
-        CU_TRY(cudaStreamSynchronize(s0));
-        CU_TRY(cudaGetLastError());
-        return true;
-      }();
+        return vp_enqueue_pass(x, (int)m, in, in + m * 96, in + m * 128, in + m * 48, d_io, d_io + m, s0);
+      }() && fetch_verdicts(ok + i0, st + off, d_io, m, s0);
       if (!good) return C_KZG_ERROR;
-      for (size_t i = 0; i < m; i++) {
-        ok[i0 + i] = h_io[i] != 0;
-        st[off + i] = h_io[m + i];
-      }
     }
     return C_KZG_OK;
   });
 }
 
-// the device form: asynchronous, ordered after and before `user`; the host waits for earlier work only when a buffer
-// has to grow (which frees the old one)
+// the device form: asynchronous, ordered after and before `user`
 C_KZG_RET verify_proofs_device(void* d_ok, const void* d_c, const void* d_z, const void* d_y, const void* d_pi, size_t n, const KZGSettings* s,
                                cudaStream_t user, void* d_status) {
   if (n == 0) return C_KZG_OK;
@@ -1643,12 +1677,7 @@ C_KZG_RET verify_proofs_device(void* d_ok, const void* d_c, const void* d_z, con
   if (!c->srs_valid || !c->g2_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
   CtxLock lock(c);
   Slot& sl = c->slot[0];
-  const BufList bufs = vp_buffers(c, std::min(n, VP_PASS), false);
-  if (!fits(bufs)) cudaStreamSynchronize(sl.st);
-  if (!reserve(bufs)) return C_KZG_ERROR;
-  bool good = [&]() -> bool {
-    CU_TRY(cudaEventRecord(sl.ev_fork, user));
-    CU_TRY(cudaStreamWaitEvent(sl.st, sl.ev_fork, 0));
+  return on_lanes(user, {{sl.st, sl.ev_done}}, {sl.st}, vp_buffers(c, std::min(n, VP_PASS), false), [&]() -> bool {
     for (size_t off = 0; off < n; off += VP_PASS) {
       const int m = (int)std::min(VP_PASS, n - off);
       int* st = d_status ? (int*)d_status + off : (int*)c->vp_io.p;
@@ -1656,30 +1685,242 @@ C_KZG_RET verify_proofs_device(void* d_ok, const void* d_c, const void* d_z, con
                            (const uint8_t*)d_pi + off * 48, (int*)d_ok + off, st, sl.st))
         return false;
     }
-    CU_TRY(cudaEventRecord(sl.ev_done, sl.st));
-    CU_TRY(cudaStreamWaitEvent(user, sl.ev_done, 0));
-    CU_TRY(cudaGetLastError());
     return true;
-  }();
-  return good ? C_KZG_OK : C_KZG_ERROR;
+  });
+}
+
+// ------------------------------------------------------------------ per-batch verification calls
+// lwkzg_verify_cell_kzg_proof_batches, lwkzg_verify_blob_cell_kzg_proof_batches and lwkzg_verify_blob_kzg_proof_batches:
+// K independent batch checks per call, one verdict, code and challenge per batch.  A call runs in passes of whole
+// batches holding at most a family's cap of items (a larger batch gets a pass of its own); one pass is a fixed launch
+// sequence whatever its number of batches.
+struct BatchPass {
+  size_t b0, b1, o0, o1;   // batches [b0, b1), items [o0, o1)
+};
+
+std::vector<BatchPass> batch_passes(const uint64_t* offsets, size_t first, size_t nb, size_t cap) {
+  std::vector<BatchPass> out;
+  for (size_t b = first; b < first + nb;) {
+    size_t e = b + 1;
+    while (e < first + nb && offsets[e + 1] - offsets[b] <= cap) e++;
+    out.push_back({b, e, (size_t)offsets[b], (size_t)offsets[e]});
+    b = e;
+  }
+  return out;
+}
+
+// The checks of every per-batch call (after nb = 0), in this order.  On success c is the settings' context and offs the
+// K + 1 offsets in pass items: the offsets times per_item (the 128 cells of a blob's extension for the blob cell call).
+C_KZG_RET batches_check(const KZGSettings* s, const void* ok, const uint64_t* offsets, size_t nb, bool have_inputs, size_t per_item, Ctx*& c,
+                        std::vector<uint64_t>& offs) {
+  if (!ok || !offsets) { set_err("null argument"); return C_KZG_BADARGS; }
+  c = ctx_of(s);
+  if (!c) return C_KZG_ERROR;
+  if (offsets[0] != 0) { set_err("offsets[0] must be 0"); return C_KZG_BADARGS; }
+  for (size_t b = 0; b < nb; b++)
+    if (offsets[b + 1] < offsets[b]) { set_err("offsets must not decrease"); return C_KZG_BADARGS; }
+  const size_t total = (size_t)offsets[nb];
+  if (total > (size_t(1) << 24) / per_item) { set_err("too many cells"); return C_KZG_BADARGS; }
+  if (total > 0 && !have_inputs) { set_err("null argument"); return C_KZG_BADARGS; }
+  offs.assign(offsets, offsets + nb + 1);
+  for (uint64_t& o : offs) o *= per_item;
+  return C_KZG_OK;
+}
+
+// Where a family of per-batch calls runs on one context: its workspace (NULL while the family's state does not exist),
+// the stream its passes run on with an event of its own, and a second stream whose work may still use its buffers.
+struct BatchSite {
+  BatchWs* ws;
+  cudaStream_t st;
+  cudaEvent_t ev;
+  cudaStream_t side;
+};
+
+// What sets a family of per-batch calls apart, for the drivers below
+struct BatchFamily {
+  BatchSite (*site)(Ctx*);
+  bool (*prep)(Ctx*);             // state its passes need, built under the context lock (NULL: none)
+  size_t (*cap)();                // items of a pass
+  bool (*empty_ok)(const Ctx*);   // the verdict of an empty batch
+  bool slots;                     // its passes read partial slots after their offsets (stage_offsets)
+};
+
+// The offsets of every pass of a plan, back to back in pinned memory, and ONE copy of them to w.boff on st; pass i reads
+// its own at w.boff + at[i]: its nb + 1 batch offsets rebased to its first item, then with `slots` its nb partial slots
+// (-1 for an empty batch, else the index among the pass's n_ne[i] non-empty batches).  The pinned area is rewritten
+// only after the previous call's copy out of it has completed.
+bool stage_offsets(BatchWs& w, const std::vector<BatchPass>& plan, const uint64_t* offsets, bool slots, std::vector<size_t>& at,
+                   std::vector<int>& n_ne, cudaStream_t st) {
+  size_t total = 0;
+  at.clear();
+  n_ne.clear();
+  for (const BatchPass& p : plan) {
+    at.push_back(total);
+    total += (slots ? 2 : 1) * (p.b1 - p.b0) + 1;
+  }
+  if (!w.ev_boff) CU_TRY(cudaEventCreateWithFlags(&w.ev_boff, cudaEventDisableTiming));
+  CU_TRY(cudaEventSynchronize(w.ev_boff));
+  if (total > w.h_boff_cap) {
+    if (w.h_boff) cudaFreeHost(w.h_boff);
+    w.h_boff = nullptr;
+    w.h_boff_cap = 0;
+    CU_TRY(cudaMallocHost(&w.h_boff, total * sizeof(int)));
+    w.h_boff_cap = total;
+  }
+  for (size_t i = 0; i < plan.size(); i++) {
+    const BatchPass& p = plan[i];
+    int* o = w.h_boff + at[i];
+    int* slot = o + (p.b1 - p.b0) + 1;
+    int k = 0;
+    for (size_t b = p.b0; b <= p.b1; b++) o[b - p.b0] = (int)(offsets[b] - p.o0);
+    for (size_t b = p.b0; b < p.b1; b++) {
+      const int v = offsets[b + 1] > offsets[b] ? k++ : -1;
+      if (slots) slot[b - p.b0] = v;
+    }
+    n_ne.push_back(k);
+  }
+  CU_TRY(cudaMemcpyAsync(w.boff.p, w.h_boff, total * sizeof(int), cudaMemcpyHostToDevice, st));
+  CU_TRY(cudaEventRecord(w.ev_boff, st));
+  return true;
+}
+
+// The host form of a per-batch call over the devices of lwkzg_set_devices: one shard of whole batches per device.
+// bufs(x, plan, cnt) lists the buffers of a shard planned as `plan`; pass(x, plan, i, d_boff, n_ne, d_ok, d_status, d_rs)
+// copies pass i's inputs to x's device and enqueues the pass on the family's stream.  Verdicts, codes and challenges
+// come back after each pass; the challenges are kept for the family's test hook.
+template <class Bufs, class Pass>
+C_KZG_RET batches_host(const BatchFamily& f, const KZGSettings* s, bool* ok, const uint64_t* offsets, size_t nb, bool have_inputs, size_t per_item,
+                       int* status, const char* what, const Bufs& bufs, const Pass& pass) {
+  if (nb == 0) return C_KZG_OK;
+  Ctx* c = nullptr;
+  std::vector<uint64_t> offs;
+  if (C_KZG_RET rc = batches_check(s, ok, offsets, nb, have_inputs, per_item, c, offs)) return rc;
+  std::vector<uint8_t> rs(nb * 32, 0);
+  if (offs[nb] == 0) {   // only empty batches: each gets the single call's verdict for an empty batch
+    for (size_t b = 0; b < nb; b++) {
+      ok[b] = f.empty_ok(c);
+      if (status) status[b] = C_KZG_OK;
+    }
+  } else {
+    if (!c->g2_valid && c->srs_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
+    const size_t cap = f.cap();
+    C_KZG_RET rc = sharded_batch(c, nb, status, what, [&](Ctx* x, size_t first, size_t cnt, int* st) -> C_KZG_RET {
+      CtxLock lock(x);
+      if (f.prep && !f.prep(x)) return C_KZG_ERROR;
+      const BatchSite w = f.site(x);
+      const std::vector<BatchPass> plan = batch_passes(offs.data(), first, cnt, cap);
+      if (!reserve(bufs(x, plan, cnt))) return C_KZG_ERROR;
+      const bool good = [&]() -> bool {
+        std::vector<size_t> at;
+        std::vector<int> n_ne;
+        if (!stage_offsets(*w.ws, plan, offs.data(), f.slots, at, n_ne, w.st)) return false;
+        for (size_t i = 0; i < plan.size(); i++) {
+          const BatchPass& p = plan[i];
+          const size_t k = p.b1 - p.b0;
+          int* d_io = (int*)w.ws->io.p;   // ok | status
+          uint8_t* d_rs = (uint8_t*)w.ws->rs.p + (p.b0 - first) * 32;
+          if (!pass(x, plan, i, (const int*)w.ws->boff.p + at[i], n_ne[i], d_io, d_io + k, d_rs)) return false;
+          CU_TRY(cudaMemcpyAsync(rs.data() + p.b0 * 32, d_rs, k * 32, cudaMemcpyDeviceToHost, w.st));
+          if (!fetch_verdicts(ok + p.b0, st + (p.b0 - first), d_io, k, w.st)) return false;
+        }
+        return true;
+      }();
+      if (!good) {   // work already enqueued may still read the caller's buffers
+        cudaStreamSynchronize(w.st);
+        cudaStreamSynchronize(w.side);
+        return C_KZG_ERROR;
+      }
+      return C_KZG_OK;
+    });
+    if (rc != C_KZG_OK) return rc;
+  }
+  CtxLock lock(c);
+  if (BatchWs* w = f.site(c).ws) {
+    w->h_rs = std::move(rs);
+    w->rs_n = nb;
+    w->rs_on_host = true;
+  }
+  return C_KZG_OK;
+}
+
+// The device form, asynchronous and ordered after / before `user`.  bufs as in batches_host; pass(x, p, d_boff, n_ne,
+// d_ok, d_status, d_rs) enqueues pass p on the family's stream with its batches' output slots.
+template <class Bufs, class Pass>
+C_KZG_RET batches_device(const BatchFamily& f, const KZGSettings* s, void* d_ok, const uint64_t* offsets, size_t nb, bool have_inputs, size_t per_item,
+                         cudaStream_t user, void* d_status, const Bufs& bufs, const Pass& pass) {
+  if (nb == 0) return C_KZG_OK;
+  Ctx* c = nullptr;
+  std::vector<uint64_t> offs;
+  if (C_KZG_RET rc = batches_check(s, d_ok, offsets, nb, have_inputs, per_item, c, offs)) return rc;
+  if (offs[nb] == 0) {   // only empty batches
+    CtxLock lock(c);
+    if (BatchWs* w = f.site(c).ws) {
+      w->h_rs.assign(nb * 32, 0);
+      w->rs_n = nb;
+      w->rs_on_host = true;
+    }
+    launch_fill_int((int*)d_ok, f.empty_ok(c) ? 1 : 0, (int)nb, user);
+    if (d_status) launch_fill_int((int*)d_status, C_KZG_OK, (int)nb, user);
+    if (cudaGetLastError() != cudaSuccess) { set_err("launch failed"); return C_KZG_ERROR; }
+    return C_KZG_OK;
+  }
+  if (!c->srs_valid || !c->g2_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
+  CtxLock lock(c);
+  if (f.prep && !f.prep(c)) return C_KZG_ERROR;
+  const BatchSite w = f.site(c);
+  const std::vector<BatchPass> plan = batch_passes(offs.data(), 0, nb, f.cap());
+  std::vector<size_t> at;
+  std::vector<int> n_ne;
+  return on_lanes(user, {{w.st, w.ev}}, {w.st, w.side}, bufs(c, plan, nb), [&]() -> bool {
+    w.ws->rs_n = nb;
+    w.ws->rs_on_host = false;
+    if (!stage_offsets(*w.ws, plan, offs.data(), f.slots, at, n_ne, w.st)) return false;
+    for (size_t i = 0; i < plan.size(); i++) {
+      const BatchPass& p = plan[i];
+      if (!pass(c, p, (const int*)w.ws->boff.p + at[i], n_ne[i], (int*)d_ok + p.b0, d_status ? (int*)d_status + p.b0 : nullptr,
+                (uint8_t*)w.ws->rs.p + p.b0 * 32))
+        return false;
+    }
+    return true;
+  });
+}
+
+// Test hook: the challenges of the family's last call (either form), 32 little-endian bytes per batch (zeros for a
+// batch without one)
+C_KZG_RET batch_challenges(const BatchFamily& f, uint8_t* out32, size_t nb, const KZGSettings* s) {
+  Ctx* c = ctx_of(s);
+  if (!c || !out32) return C_KZG_ERROR;
+  CtxLock lock(c);
+  const BatchSite w = f.site(c);
+  if (!w.ws || nb > w.ws->rs_n) { set_err("no such batch in the last call"); return C_KZG_BADARGS; }
+  if (nb == 0) return C_KZG_OK;
+  if (w.ws->rs_on_host) {
+    memcpy(out32, w.ws->h_rs.data(), nb * 32);
+    return C_KZG_OK;
+  }
+  if (cudaStreamSynchronize(w.st) != cudaSuccess || cudaMemcpy(out32, w.ws->rs.p, nb * 32, cudaMemcpyDeviceToHost) != cudaSuccess) {
+    set_err("D2H failed");
+    return C_KZG_ERROR;
+  }
+  return C_KZG_OK;
 }
 
 #include "cells_host.inl"
 
 // ------------------------------------------------------------------ lwkzg_verify_blob_kzg_proof_batches
-// K independent verify_blob_kzg_proof_batch checks.  A call runs in passes of whole batches holding at most
-// verify_super_blobs blobs, planned as the cell calls plan theirs (cell_batch_passes); a larger batch gets a pass of its
-// own, whose host blobs are staged verify_super_blobs at a time while its per-blob state (points, z, y, tuples,
-// statuses: about 0.6 KB per blob) covers the whole batch.  A pass is one fixed launch sequence whatever its number of
-// batches (bb_enqueue_pass).  This is not verify_prepare, which is built for one huge batch, synchronises the host and
-// owns the vb_* workspace that the aggregate call, the distributed phases and their test hooks read.
+// K independent verify_blob_kzg_proof_batch checks (batches_host), in passes of at most verify_super_blobs blobs; a
+// larger batch gets a pass of its own, whose host blobs are staged verify_super_blobs at a time while its per-blob
+// state (points, z, y, tuples, statuses: about 0.6 KB per blob) covers the whole batch.  A pass is one fixed launch
+// sequence whatever its number of batches (bb_enqueue_pass).  This is not verify_prepare, which is built for one huge
+// batch, synchronises the host and owns the vb_* workspace that the aggregate call, the distributed phases and their
+// test hooks read.
 
 // The buffers of a call planned as `plan` (own_io: the inputs, staged blobs and verdicts of a pass too, for host-buffer
 // calls): per-blob and per-batch buffers for its largest pass, the offsets of every pass, the challenges of rs_batches
 // batches.
-BufList bb_buffers(Ctx* c, const std::vector<CellBatchPass>& plan, size_t rs_batches, size_t stage, bool own_io) {
+BufList bb_buffers(Ctx* c, const std::vector<BatchPass>& plan, size_t rs_batches, size_t stage, bool own_io) {
   size_t m = 1, nb = 1, offs = 0;
-  for (const CellBatchPass& p : plan) {
+  for (const BatchPass& p : plan) {
     m = std::max(m, p.o1 - p.o0);
     nb = std::max(nb, p.b1 - p.b0);
     offs += 2 * (p.b1 - p.b0) + 1;
@@ -1687,45 +1928,10 @@ BufList bb_buffers(Ctx* c, const std::vector<CellBatchPass>& plan, size_t rs_bat
   const size_t terms = blob_batches_terms((int)m, (int)nb);
   BufList bufs = {{&c->bb_aff, 2 * m * AFFINE_BYTES}, {&c->bb_c48r, m * 48}, {&c->bb_p48r, m * 48}, {&c->bb_states, m * 32}, {&c->bb_zy, 2 * m * 32},
                   {&c->bb_tuples, m * 160}, {&c->bb_st, 3 * m * sizeof(int)}, {&c->bb_sc, terms * 32}, {&c->bb_terms, terms * XYZZ_BYTES},
-                  {&c->bb_boff, offs * sizeof(int)}, {&c->bb_bst, nb * sizeof(int)}, {&c->bb_out, nb * 288}, {&c->bb_pok, nb * sizeof(int)},
-                  {&c->bb_rs, std::max<size_t>(rs_batches, 1) * 32}};
-  if (own_io) bufs.insert(bufs.end(), {{&c->bb_in, m * 96}, {&c->bb_blobs, std::min(m, stage) * BLOB_BYTES}, {&c->bb_io, 2 * nb * sizeof(int)}});
+                  {&c->bb.boff, offs * sizeof(int)}, {&c->bb_bst, nb * sizeof(int)}, {&c->bb_out, nb * 288}, {&c->bb_pok, nb * sizeof(int)},
+                  {&c->bb.rs, std::max<size_t>(rs_batches, 1) * 32}};
+  if (own_io) bufs.insert(bufs.end(), {{&c->bb_in, m * 96}, {&c->bb_blobs, std::min(m, stage) * BLOB_BYTES}, {&c->bb.io, 2 * nb * sizeof(int)}});
   return bufs;
-}
-
-// Pass i's offsets at c->bb_boff + at[i]: its nb + 1 batch offsets rebased to its first blob, then the nb partial slots
-// (-1 for an empty batch, else the index among the pass's n_ne[i] non-empty batches).  Staged in pinned memory, which is
-// rewritten only after the previous call's copy out of it has completed, and copied with ONE copy on st.
-bool bb_stage_offsets(Ctx* c, const std::vector<CellBatchPass>& plan, const uint64_t* offsets, std::vector<size_t>& at, std::vector<int>& n_ne,
-                      cudaStream_t st) {
-  size_t total = 0;
-  at.clear();
-  n_ne.clear();
-  for (const CellBatchPass& p : plan) {
-    at.push_back(total);
-    total += 2 * (p.b1 - p.b0) + 1;
-  }
-  if (!c->ev_bb) CU_TRY(cudaEventCreateWithFlags(&c->ev_bb, cudaEventDisableTiming));
-  CU_TRY(cudaEventSynchronize(c->ev_bb));
-  if (total > c->h_bb_cap) {
-    if (c->h_bb) cudaFreeHost(c->h_bb);
-    c->h_bb = nullptr;
-    c->h_bb_cap = 0;
-    CU_TRY(cudaMallocHost(&c->h_bb, total * sizeof(int)));
-    c->h_bb_cap = total;
-  }
-  for (size_t i = 0; i < plan.size(); i++) {
-    const CellBatchPass& p = plan[i];
-    int* o = c->h_bb + at[i];
-    int* slot = o + (p.b1 - p.b0) + 1;
-    int k = 0;
-    for (size_t b = p.b0; b <= p.b1; b++) o[b - p.b0] = (int)(offsets[b] - p.o0);
-    for (size_t b = p.b0; b < p.b1; b++) slot[b - p.b0] = offsets[b + 1] > offsets[b] ? k++ : -1;
-    n_ne.push_back(k);
-  }
-  CU_TRY(cudaMemcpyAsync(c->bb_boff.p, c->h_bb, total * sizeof(int), cudaMemcpyHostToDevice, st));
-  CU_TRY(cudaEventRecord(c->ev_bb, st));
-  return true;
 }
 
 // One pass on slot 0's stream (the point decompressions forked to its aux stream, beside the first blob hashes).  The
@@ -1733,7 +1939,7 @@ bool bb_stage_offsets(Ctx* c, const std::vector<CellBatchPass>& plan, const uint
 // blobs at a time (through the pinned ring when pageable); d_com / d_pi are its commitments and proofs on the device, its
 // offsets and slots are at d_boff.  d_ok, d_status (may be NULL) and d_rs receive its batches' verdicts, codes and
 // challenges.
-bool bb_enqueue_pass(Ctx* c, const CellBatchPass& p, const int* d_boff, int n_ne, const void* d_blobs, const Blob* h_blobs, bool pageable, size_t stage,
+bool bb_enqueue_pass(Ctx* c, const BatchPass& p, const int* d_boff, int n_ne, const void* d_blobs, const Blob* h_blobs, bool pageable, size_t stage,
                      const void* d_com, const void* d_pi, int* d_ok, int* d_status, void* d_rs) {
   Slot& sl = c->slot[0];
   cudaStream_t st = sl.st, aux = sl.aux;
@@ -1798,145 +2004,44 @@ long bb_ring_blobs() {
   return std::max(1L, opts().chunk_blobs);
 }
 
+BatchSite bb_site(Ctx* c) { return {&c->bb, c->slot[0].st, c->slot[0].ev_done, c->slot[0].aux}; }
+
+// an empty batch: the reference rejects it (lib.rs:538-543), c-kzg accepts it
+const BatchFamily BLOB_BATCHES = {bb_site, nullptr, vb_super_blobs, [](const Ctx* c) { return c->lagrange(); }, true};
+
 C_KZG_RET blob_batches_host(bool* ok, const Blob* blobs, const Bytes48* commitments, const Bytes48* proofs, const uint64_t* offsets, size_t nb,
                             const KZGSettings* s, int* status) {
-  if (nb == 0) return C_KZG_OK;
-  if (!ok || !offsets) { set_err("null argument"); return C_KZG_BADARGS; }
-  Ctx* c = ctx_of(s);
-  if (!c) return C_KZG_ERROR;
-  size_t total = 0;
-  if (C_KZG_RET rc = cell_batches_check(offsets, nb, blobs && commitments && proofs, 1, &total)) return rc;
-  std::vector<uint8_t> rs(nb * 32, 0);
-  if (total == 0) {   // only empty batches: each gets the single call's verdict for an empty batch
-    for (size_t b = 0; b < nb; b++) {
-      ok[b] = c->lagrange();
-      if (status) status[b] = C_KZG_OK;
-    }
-  } else {
-    if (!c->g2_valid && c->srs_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
-    const size_t super = vb_super_blobs();
-    C_KZG_RET rc = sharded_batch(c, nb, status, "invalid commitment, proof or blob", [&](Ctx* x, size_t first, size_t cnt, int* st) -> C_KZG_RET {
-      CtxLock lock(x);
-      const std::vector<CellBatchPass> plan = cell_batch_passes(offsets, first, cnt, super);
-      if (!reserve(bb_buffers(x, plan, cnt, super, true))) return C_KZG_ERROR;
-      size_t max_m = 0;
-      for (const CellBatchPass& p : plan) max_m = std::max(max_m, p.o1 - p.o0);
-      const size_t shard_blobs = (size_t)(offsets[first + cnt] - offsets[first]);
-      const bool pageable = shard_blobs * BLOB_BYTES >= (size_t(4) << 20) && is_pageable_host(blobs) &&
-                            x->ring.ensure(std::min<size_t>(std::min(max_m, super), (size_t)bb_ring_blobs()) * BLOB_BYTES);
-      cudaStream_t s0 = x->slot[0].st;
-      std::vector<size_t> at;
-      std::vector<int> n_ne;
-      if (!bb_stage_offsets(x, plan, offsets, at, n_ne, s0)) return C_KZG_ERROR;
-      std::vector<int> h_io;
-      for (size_t i = 0; i < plan.size(); i++) {
-        const CellBatchPass& p = plan[i];
-        const size_t m = p.o1 - p.o0, k = p.b1 - p.b0;
+  const size_t super = vb_super_blobs();
+  return batches_host(
+      BLOB_BATCHES, s, ok, offsets, nb, blobs && commitments && proofs, 1, status, "invalid commitment, proof or blob",
+      [&](Ctx* x, const std::vector<BatchPass>& plan, size_t cnt) { return bb_buffers(x, plan, cnt, super, true); },
+      [&](Ctx* x, const std::vector<BatchPass>& plan, size_t i, const int* d_boff, int n_ne, int* d_ok, int* d_st, void* d_rs) -> bool {
+        const BatchPass& p = plan[i];
+        const size_t m = p.o1 - p.o0;
+        // blobs in pageable memory go through the pinned ring (see HostStager), sized for the shard's largest pass; tiny
+        // shards are not worth the ring
+        size_t max_m = 0;
+        for (const BatchPass& q : plan) max_m = std::max(max_m, q.o1 - q.o0);
+        const bool pageable = (plan.back().o1 - plan.front().o0) * BLOB_BYTES >= (size_t(4) << 20) && is_pageable_host(blobs) &&
+                              x->ring.ensure(std::min<size_t>(std::min(max_m, super), (size_t)bb_ring_blobs()) * BLOB_BYTES);
+        cudaStream_t s0 = x->slot[0].st;
         uint8_t* in = (uint8_t*)x->bb_in.p;   // C | pi
-        int* d_io = (int*)x->bb_io.p;         // ok | status
-        uint8_t* d_rs = (uint8_t*)x->bb_rs.p + (p.b0 - first) * 32;
-        h_io.resize(2 * k);
-        bool good = [&]() -> bool {
-          if (m) {
-            CU_TRY(cudaMemcpyAsync(in, commitments + p.o0, m * 48, cudaMemcpyHostToDevice, s0));
-            CU_TRY(cudaMemcpyAsync(in + m * 48, proofs + p.o0, m * 48, cudaMemcpyHostToDevice, s0));
-          }
-          if (!bb_enqueue_pass(x, p, (const int*)x->bb_boff.p + at[i], n_ne[i], nullptr, blobs, pageable, super, in, in + m * 48, d_io, d_io + k, d_rs))
-            return false;
-          CU_TRY(cudaMemcpyAsync(h_io.data(), d_io, 2 * k * sizeof(int), cudaMemcpyDeviceToHost, s0));
-          CU_TRY(cudaMemcpyAsync(rs.data() + p.b0 * 32, d_rs, k * 32, cudaMemcpyDeviceToHost, s0));
-          CU_TRY(cudaStreamSynchronize(s0));
-          CU_TRY(cudaGetLastError());
-          return true;
-        }();
-        if (!good) {
-          cudaStreamSynchronize(x->slot[0].aux);
-          return C_KZG_ERROR;
+        if (m) {
+          CU_TRY(cudaMemcpyAsync(in, commitments + p.o0, m * 48, cudaMemcpyHostToDevice, s0));
+          CU_TRY(cudaMemcpyAsync(in + m * 48, proofs + p.o0, m * 48, cudaMemcpyHostToDevice, s0));
         }
-        for (size_t j = 0; j < k; j++) {
-          ok[p.b0 + j] = h_io[j] != 0;
-          st[p.b0 - first + j] = h_io[k + j];
-        }
-      }
-      return C_KZG_OK;
-    });
-    if (rc != C_KZG_OK) return rc;
-  }
-  CtxLock lock(c);
-  c->bb_h_rs = std::move(rs);
-  c->bb_rs_n = nb;
-  c->bb_rs_on_host = true;
-  return C_KZG_OK;
+        return bb_enqueue_pass(x, p, d_boff, n_ne, nullptr, blobs, pageable, super, in, in + m * 48, d_ok, d_st, d_rs);
+      });
 }
 
-// the device form: asynchronous, ordered after and before `user`; the host waits for earlier work only when a buffer
-// has to grow (which frees the old one)
 C_KZG_RET blob_batches_device(void* d_ok, const void* d_blobs, const void* d_com, const void* d_pi, const uint64_t* offsets, size_t nb, const KZGSettings* s,
                               cudaStream_t user, void* d_status) {
-  if (nb == 0) return C_KZG_OK;
-  if (!d_ok || !offsets) { set_err("null argument"); return C_KZG_BADARGS; }
-  Ctx* c = ctx_of(s);
-  if (!c) return C_KZG_ERROR;
-  size_t total = 0;
-  if (C_KZG_RET rc = cell_batches_check(offsets, nb, d_blobs && d_com && d_pi, 1, &total)) return rc;
-  if (total == 0) {   // only empty batches
-    CtxLock lock(c);
-    c->bb_h_rs.assign(nb * 32, 0);
-    c->bb_rs_n = nb;
-    c->bb_rs_on_host = true;
-    launch_fill_int((int*)d_ok, c->lagrange() ? 1 : 0, (int)nb, user);
-    if (d_status) launch_fill_int((int*)d_status, C_KZG_OK, (int)nb, user);
-    if (cudaGetLastError() != cudaSuccess) { set_err("launch failed"); return C_KZG_ERROR; }
-    return C_KZG_OK;
-  }
-  if (!c->srs_valid || !c->g2_valid) { set_err("SRS re-hydration failed"); return C_KZG_ERROR; }
-  CtxLock lock(c);
-  Slot& sl = c->slot[0];
-  const std::vector<CellBatchPass> plan = cell_batch_passes(offsets, 0, nb, vb_super_blobs());
-  const BufList bufs = bb_buffers(c, plan, nb, 0, false);
-  if (!fits(bufs)) {
-    cudaStreamSynchronize(sl.st);
-    cudaStreamSynchronize(sl.aux);
-  }
-  if (!reserve(bufs)) return C_KZG_ERROR;
-  c->bb_rs_n = nb;
-  c->bb_rs_on_host = false;
-  bool good = [&]() -> bool {
-    CU_TRY(cudaEventRecord(sl.ev_fork, user));
-    CU_TRY(cudaStreamWaitEvent(sl.st, sl.ev_fork, 0));
-    std::vector<size_t> at;
-    std::vector<int> n_ne;
-    if (!bb_stage_offsets(c, plan, offsets, at, n_ne, sl.st)) return false;
-    for (size_t i = 0; i < plan.size(); i++) {
-      const CellBatchPass& p = plan[i];
-      if (!bb_enqueue_pass(c, p, (const int*)c->bb_boff.p + at[i], n_ne[i], (const uint8_t*)d_blobs + p.o0 * BLOB_BYTES, nullptr, false, 0,
-                           (const uint8_t*)d_com + p.o0 * 48, (const uint8_t*)d_pi + p.o0 * 48, (int*)d_ok + p.b0, d_status ? (int*)d_status + p.b0 : nullptr,
-                           (uint8_t*)c->bb_rs.p + p.b0 * 32))
-        return false;
-    }
-    CU_TRY(cudaEventRecord(sl.ev_done, sl.st));
-    CU_TRY(cudaStreamWaitEvent(user, sl.ev_done, 0));
-    CU_TRY(cudaGetLastError());
-    return true;
-  }();
-  return good ? C_KZG_OK : C_KZG_ERROR;
-}
-
-C_KZG_RET blob_batches_debug_challenges(uint8_t* out32, size_t nb, const KZGSettings* s) {
-  Ctx* c = ctx_of(s);
-  if (!c || !out32) return C_KZG_ERROR;
-  CtxLock lock(c);
-  if (nb > c->bb_rs_n) { set_err("no such batch in the last call"); return C_KZG_BADARGS; }
-  if (nb == 0) return C_KZG_OK;
-  if (c->bb_rs_on_host) {
-    memcpy(out32, c->bb_h_rs.data(), nb * 32);
-    return C_KZG_OK;
-  }
-  if (cudaStreamSynchronize(c->slot[0].st) != cudaSuccess || cudaMemcpy(out32, c->bb_rs.p, nb * 32, cudaMemcpyDeviceToHost) != cudaSuccess) {
-    set_err("D2H failed");
-    return C_KZG_ERROR;
-  }
-  return C_KZG_OK;
+  return batches_device(BLOB_BATCHES, s, d_ok, offsets, nb, d_blobs && d_com && d_pi, 1, user, d_status,
+                        [](Ctx* x, const std::vector<BatchPass>& plan, size_t cnt) { return bb_buffers(x, plan, cnt, 0, false); },
+                        [&](Ctx* x, const BatchPass& p, const int* d_boff, int n_ne, int* ok, int* st, void* rs) {
+                          return bb_enqueue_pass(x, p, d_boff, n_ne, (const uint8_t*)d_blobs + p.o0 * BLOB_BYTES, nullptr, false, 0,
+                                                 (const uint8_t*)d_com + p.o0 * 48, (const uint8_t*)d_pi + p.o0 * 48, ok, st, rs);
+                        });
 }
 
 }  // namespace
@@ -2166,7 +2271,7 @@ C_KZG_RET lwkzg_verify_blob_kzg_proof_batches_device(void* d_ok, const void* d_b
   return blob_batches_device(d_ok, d_blobs, d_commitments, d_proofs, offsets, n_batches, s, (cudaStream_t)stream, d_status);
 }
 C_KZG_RET lwkzg_debug_blob_batch_challenges(uint8_t* out32, size_t n_batches, const KZGSettings* s) {
-  return blob_batches_debug_challenges(out32, n_batches, s);
+  return batch_challenges(BLOB_BATCHES, out32, n_batches, s);
 }
 
 static C_KZG_RET verify_blob_single(bool* ok, const Blob* blob, const Bytes48* commitment_bytes, const Bytes48* proof_bytes, const KZGSettings* s,
