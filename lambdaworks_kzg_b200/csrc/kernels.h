@@ -60,6 +60,7 @@ size_t msm_ba_scratch_bytes(int n_blobs);
 int msm_ba_threads();
 int msm_ba_slots();
 int msm_ba_num_variants();
+int msm_ba_variant();
 void msm_ba_set_variant(int v);   // tuning: index into BA_VARIANTS (accumulators per thread x threads per blob), msm.cu
 // sum partials, normalise, compress.  d_aff_out (may be NULL): Montgomery affine.
 void launch_msm_finalize(void* d_out48, void* d_aff_out, const void* d_partials, int parts_per_blob, int n_blobs, cudaStream_t st);

@@ -2092,6 +2092,7 @@ long lwkzg_get_option(const char* name) {
   if (n == "verify_overlap_decode") return opts().verify_overlap_decode;
   if (n == "cell_window_bits") return opts().cell_window_bits;
   if (n == "cell_chunk_blobs") return opts().cell_chunk_blobs;
+  if (n == "msm_ba_variant") return msm_ba_variant();
   if (n == "msm_ba_threads") return msm_ba_threads();   // read-only: threads per blob of the batched-affine kernel
   if (n == "msm_ba_slots") return msm_ba_slots();       // read-only: affine accumulators per thread
   return -1;

@@ -83,6 +83,7 @@ constexpr int N_BA_VARIANTS = (int)(sizeof(BA_VARIANTS) / sizeof(BA_VARIANTS[0])
 static int g_ba_variant = 0;
 void msm_ba_set_variant(int v) { if (v >= 0 && v < N_BA_VARIANTS) g_ba_variant = v; }
 int msm_ba_num_variants() { return N_BA_VARIANTS; }
+int msm_ba_variant() { return g_ba_variant; }
 int msm_ba_threads() { return BA_VARIANTS[g_ba_variant].threads; }
 int msm_ba_slots() { return BA_VARIANTS[g_ba_variant].k; }
 size_t msm_ba_scratch_bytes(int n_blobs) {   // sized for the largest variant: 64 slots x 9 words x 128 threads
