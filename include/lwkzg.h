@@ -95,7 +95,11 @@ typedef struct {
 /* reference: src/lib.rs:709-715 (BADARGS unless n1 == 4096 && n2 == 65) */
 C_KZG_RET load_trusted_setup(KZGSettings *out, const uint8_t *g1_bytes, size_t n1,
                              const uint8_t *g2_bytes, size_t n2);
-/* reference: src/lib.rs:779-802 + src/srs.rs:25-128 (line-based text format) */
+/* reference: src/lib.rs:779-802 + src/srs.rs:25-128 (line-based text format: a header n1 / n2, then n1 G1 lines read
+ * as MONOMIAL points, then n2 G2 lines; later lines are ignored).  This is not c-kzg-4844's trusted_setup.txt, whose
+ * first G1 section is in Lagrange form: given that file, this loader reads the Lagrange points as monomial ones and,
+ * in modes 1 and 2, transforms them again -- every later result is wrong and nothing reports it.  Load c-kzg files
+ * with lwkzg_load_trusted_setup_file_ckzg (Part 2). */
 C_KZG_RET load_trusted_setup_file(KZGSettings *out, FILE *in);
 /* reference: src/lib.rs:821-829 (returns a code; c-kzg declares void) */
 C_KZG_RET free_trusted_setup(KZGSettings *s);
@@ -119,6 +123,36 @@ C_KZG_RET verify_blob_kzg_proof_batch(bool *ok, const Blob *blobs, const Bytes48
                                       const Bytes48 *proofs_bytes, size_t n, const KZGSettings *s);
 
 /* ------------------------------------------------------------------ Part 2 */
+/* c-kzg-4844 (v2) trusted setups -- the Ethereum ceremony output as c-kzg ships it (trusted_setup.txt): c-kzg's
+ * load_trusted_setup / load_trusted_setup_file signatures under an lwkzg_ prefix (a c-kzg binding reaches them with
+ * #[link_name], INTEGRATION.md 2).
+ *   Sections: 4096 G1 monomial points [tau^j]G, 4096 G1 Lagrange points [l_k(tau)]G in NATURAL order over w^k (w the
+ *   4096th root of unity of the Lagrange modes), 65 G2 monomial points [tau^i]H, compressed; exactly 4096 x 48,
+ *   4096 x 48 and 65 x 96 bytes.  precompute: 0..15, accepted as c-kzg accepts it; it changes no output (the FK20
+ *   window is the "cell_window_bits" option).
+ *   File: decimal counts 4096 and 65, then hex byte pairs -- the Lagrange points, the G2 points, the monomial points.
+ *   Whitespace (spaces, LF, CRLF) may separate tokens and byte pairs, never the two digits of a pair; anything after
+ *   the last point is ignored; anything else is malformed.  Arguments and the file are checked before the device is
+ *   touched, so those errors are C_KZG_BADARGS without a GPU.
+ *   Mode (captured at load): 0 uses the monomial section as the SRS; 1 and 2 the Lagrange section, bit-reversed, plus
+ *   the monomial section for FK20 and cell verification.  g1_values, g2_values and every later output are
+ *   byte-identical to load_trusted_setup on the monomial points of the same tau in the same mode, without its
+ *   4096-MSM Lagrange conversion.
+ *   Checks (C_KZG_BADARGS, lwkzg_last_error() names the check and the point): strict decoding as blst's (canonical x,
+ *   consistent flags, on the curve, in the subgroup -- G2 included; no point at infinity); M_0 is the generator; with
+ *   rho = SHA-256(domain || the three sections in file order) mod r, sum_k rho^k L_k = sum_j f_j M_j where f(w^k) =
+ *   rho^k; e(sum rho^i M_(i+1), Q_0) = e(sum rho^i M_i, Q_1) over i < 4095; e(M_1, Q_i) = e(M_0, Q_(i+1)) for every
+ *   i < 64.  c-kzg itself only checks that the Lagrange section is not the monomial one.
+ *   Other failures: NULL pointers C_KZG_BADARGS, allocation C_KZG_MALLOC, no usable device C_KZG_ERROR; *out is
+ *   untouched on any failure.
+ *   Parity unpinned: the section order, the natural order of the Lagrange points and the 0..15 precompute range follow
+ *   c-kzg-4844 v2's sources as recalled, not re-read; the Lagrange order agrees with consensus-specs'
+ *   bit_reversal_permutation(KZG_SETUP_G1_LAGRANGE) and is pinned by the tests against [l_k(tau)]G. */
+C_KZG_RET lwkzg_load_trusted_setup_ckzg(KZGSettings *out, const uint8_t *g1_monomial_bytes, uint64_t num_g1_monomial_bytes,
+                                        const uint8_t *g1_lagrange_bytes, uint64_t num_g1_lagrange_bytes,
+                                        const uint8_t *g2_monomial_bytes, uint64_t num_g2_monomial_bytes, uint64_t precompute);
+C_KZG_RET lwkzg_load_trusted_setup_file_ckzg(KZGSettings *out, FILE *in, uint64_t precompute);
+
 /* Additive batch API.  `status` (may be NULL) receives one C_KZG_RET per item
  * so a bad item does not poison the batch; the function's return value is
  * C_KZG_OK iff the call itself ran (per-item failures are only in `status`,
@@ -436,6 +470,11 @@ void lwkzg_debug_stage_copy(void *dst, const void *src, size_t bytes);
  * 2 = attached to the table another PROCESS built (CUDA IPC), 3 = shared with another settings object of this
  * process; -1 on error */
 int lwkzg_table_share(const KZGSettings *s);
+/* phase times of this thread's last load_trusted_setup[_file] / lwkzg_load_trusted_setup[_file]_ckzg, milliseconds
+ * (0 for a phase that did not run): decoding (CUDA events: copies + decode kernels), the c-kzg setup check (CUDA
+ * events: its kernels), the Lagrange conversion of the monomial loaders in modes 1 and 2 and the context build
+ * (digit table included; host clock, both end in a device synchronisation).  Returns 0. */
+int lwkzg_last_load_times(double *decode_ms, double *check_ms, double *convert_ms, double *build_ms);
 
 /* Options: "window_bits" (fixed-base table window c, 4..16; default 16 = 100 GiB, the fastest; shrunk
  * automatically to what free device memory allows -- lwkzg_window_bits() tells; must

@@ -50,6 +50,9 @@ def load_library() -> ctypes.CDLL:
     sig = {
         "load_trusted_setup": [sp, vp, sz, vp, sz],
         "load_trusted_setup_file": [sp, vp],
+        "lwkzg_load_trusted_setup_ckzg": [sp, vp, ctypes.c_uint64, vp, ctypes.c_uint64, vp, ctypes.c_uint64, ctypes.c_uint64],
+        "lwkzg_load_trusted_setup_file_ckzg": [sp, vp, ctypes.c_uint64],
+        "lwkzg_last_load_times": [ctypes.POINTER(ctypes.c_double)] * 4,
         "free_trusted_setup": [sp],
         "blob_to_kzg_commitment": [vp, vp, sp],
         "compute_kzg_proof": [vp, vp, vp, vp, sp],
@@ -184,8 +187,7 @@ class Settings:
             pass
 
 
-def load_trusted_setup_file(path: str) -> Settings:
-    """load_trusted_setup_file(KZGSettings*, FILE*) -- lib.rs:779-802."""
+def _load_from_file(path: str, fn: str, *extra) -> Settings:
     lib = load_library()
     libc = ctypes.CDLL(None)
     libc.fopen.restype = ctypes.c_void_p
@@ -196,11 +198,41 @@ def load_trusted_setup_file(path: str) -> Settings:
         raise FileNotFoundError(path)
     s = Settings()
     try:
-        _check(lib.load_trusted_setup_file(s.ptr, fp), "load_trusted_setup_file")
+        _check(getattr(lib, fn)(s.ptr, fp, *extra), fn)
     finally:
         libc.fclose(fp)
     s._loaded = True
     return s
+
+
+def load_trusted_setup_file(path: str) -> Settings:
+    """load_trusted_setup_file(KZGSettings*, FILE*) -- lib.rs:779-802.  Reads the reference's format (monomial G1
+    points first); a c-kzg-4844 trusted_setup.txt needs load_trusted_setup_file_ckzg."""
+    return _load_from_file(path, "load_trusted_setup_file")
+
+
+def load_trusted_setup_file_ckzg(path: str, precompute: int = 0) -> Settings:
+    """c-kzg-4844's trusted_setup.txt (4096 Lagrange G1, 65 G2, 4096 monomial G1 points), checked on the device to be
+    one powers-of-tau setup -- lwkzg_load_trusted_setup_file_ckzg."""
+    return _load_from_file(path, "lwkzg_load_trusted_setup_file_ckzg", precompute)
+
+
+def load_trusted_setup_ckzg(g1_monomial: bytes, g1_lagrange: bytes, g2_monomial: bytes, precompute: int = 0) -> Settings:
+    """c-kzg-4844 v2's load_trusted_setup(out, g1_monomial, ..., g1_lagrange, ..., g2_monomial, ..., precompute): the
+    three compressed sections as bytes -- lwkzg_load_trusted_setup_ckzg."""
+    lib = load_library()
+    s = Settings()
+    _check(lib.lwkzg_load_trusted_setup_ckzg(s.ptr, g1_monomial, len(g1_monomial), g1_lagrange, len(g1_lagrange), g2_monomial, len(g2_monomial),
+                                             precompute), "lwkzg_load_trusted_setup_ckzg")
+    s._loaded = True
+    return s
+
+
+def last_load_times() -> dict:
+    """Phase times (ms) of this thread's last trusted-setup load: decode, check, convert, build."""
+    v = [ctypes.c_double() for _ in range(4)]
+    load_library().lwkzg_last_load_times(*[ctypes.byref(x) for x in v])
+    return dict(zip(("decode_ms", "check_ms", "convert_ms", "build_ms"), (x.value for x in v)))
 
 
 def load_trusted_setup(g1_bytes: bytes, g2_bytes: bytes, n1: Optional[int] = None, n2: Optional[int] = None) -> Settings:

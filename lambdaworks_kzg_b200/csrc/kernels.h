@@ -95,8 +95,8 @@ double run_imad_peak(int variant);
 // ---- verification (verify.cu)
 struct G2PreparedDev;  // opaque: line coefficients of one G2 point
 size_t g2_prepared_bytes();
-// canonical LE limbs x.c0,x.c1,y.c0,y.c1 (48 u32) -> prepared lines; flag = 1 if not on the twist
-void launch_g2_prepare(void* d_prepared, int* d_bad, const void* d_canon_in, cudaStream_t st);
+// canonical LE limbs x.c0,x.c1,y.c0,y.c1 (48 u32) -> prepared lines; flag = 1 if not on the twist.  n points, one block each
+void launch_g2_prepare(void* d_prepared, int* d_bad, const void* d_canon_in, cudaStream_t st, int n = 1);
 // bad[i] = 1 if g2 value i (canonical limbs, 48 u32 each) is not on the twist
 void launch_g2_check(int* d_bad, const void* d_canon_in, int n, cudaStream_t st);
 // single verification: C - y*g1_0 + z*pi  vs  pi  (SURVEY App. A.7, bilinear rearrangement)
@@ -126,6 +126,8 @@ size_t batch_partials_scratch_bytes(int n_local);
 void launch_batch_final(int* d_ok, const void* d_partials288, int n_ranks, const void* d_prep0, const void* d_prep1, cudaStream_t st);
 // n_checks independent checks, one block each: d_ok[i] from the 288 bytes at d_partials288 + 288 i
 void launch_batch_final_each(int* d_ok, const void* d_partials288, int n_checks, const void* d_prep0, const void* d_prep1, cudaStream_t st);
+// the same, check i against the neighbouring prepared points d_preps[i], d_preps[i + 1] (a chain of G2 points)
+void launch_batch_final_chain(int* d_ok, const void* d_partials288, int n_checks, const void* d_preps, cudaStream_t st);
 
 // ---- many independent single-opening checks (verify_proofs.cu), one item per thread
 // d_pts[2 i] = C_i - y_i G + z_i pi_i, d_pts[2 i + 1] = -pi_i (affine Montgomery) from decoded C, pi (in G1 or infinity) and

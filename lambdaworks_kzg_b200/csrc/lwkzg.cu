@@ -40,6 +40,12 @@ using namespace lw;
 thread_local std::string tl_err;
 
 void set_err(const std::string& s) { tl_err = s; }
+// phase times of this thread's last trusted-setup load (lwkzg_last_load_times)
+struct LoadTimes { double decode_ms, check_ms, convert_ms, build_ms; };
+thread_local LoadTimes tl_load = {0, 0, 0, 0};
+double ms_since(std::chrono::steady_clock::time_point t0) {
+  return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+}
 
 #define CU_TRY(expr)                                                                      \
   do {                                                                                    \
@@ -1224,66 +1230,16 @@ bool parse_usize(const std::string& ln, size_t& v) {
   return true;
 }
 
-// Decode + validate compressed points on the device, then lay out KZGSettings
-// exactly as src/srs.rs:99-153 / src/lib.rs:724-758 do.  n1 / n2 may be
-// smaller than 4096 / 65 for the file loader (tests/trusted_setup_4.txt): the
-// arrays are always allocated full size and zero-padded so later calls stay
-// memory safe (they then fail SRS re-hydration -> C_KZG_ERROR).
-C_KZG_RET settings_from_compressed(KZGSettings* out, const uint8_t* g1_bytes, size_t n1, const uint8_t* g2_bytes, size_t n2) {
-  size_t a1 = std::max<size_t>(n1, N_POINTS), a2 = std::max<size_t>(n2, TRUSTED_SETUP_NUM_G2_POINTS);
-  void *d_in1 = nullptr, *d_in2 = nullptr, *d_c1 = nullptr, *d_c2 = nullptr;
-  int* d_st = nullptr;
-  std::vector<uint32_t> c1(n1 * 24), c2(n2 * 48);
-  std::vector<int> st(n1 + n2);
-  auto cleanup = [&]() {
-    cudaFree(d_in1); cudaFree(d_in2); cudaFree(d_c1); cudaFree(d_c2); cudaFree(d_st);
-  };
-  auto run = [&]() -> bool {
-    CU_TRY(cudaMalloc(&d_in1, std::max<size_t>(n1, 1) * 48));
-    CU_TRY(cudaMalloc(&d_in2, std::max<size_t>(n2, 1) * 96));
-    CU_TRY(cudaMalloc(&d_c1, std::max<size_t>(n1, 1) * 96));
-    CU_TRY(cudaMalloc(&d_c2, std::max<size_t>(n2, 1) * 192));
-    CU_TRY(cudaMalloc(&d_st, (n1 + n2 + 1) * sizeof(int)));
-    if (n1) CU_TRY(cudaMemcpy(d_in1, g1_bytes, n1 * 48, cudaMemcpyHostToDevice));
-    if (n2) CU_TRY(cudaMemcpy(d_in2, g2_bytes, n2 * 96, cudaMemcpyHostToDevice));
-    launch_setup_decode_g1(d_c1, d_st, d_in1, (int)n1, 0);
-    launch_setup_decode_g2(d_c2, d_st + n1, d_in2, (int)n2, 0);
-    CU_TRY(cudaDeviceSynchronize());
-    CU_TRY(cudaGetLastError());
-    if (n1) CU_TRY(cudaMemcpy(c1.data(), d_c1, n1 * 96, cudaMemcpyDeviceToHost));
-    if (n2) CU_TRY(cudaMemcpy(c2.data(), d_c2, n2 * 192, cudaMemcpyDeviceToHost));
-    CU_TRY(cudaMemcpy(st.data(), d_st, (n1 + n2) * sizeof(int), cudaMemcpyDeviceToHost));
-    return true;
-  };
-  bool ok = run();
-  cleanup();
-  if (!ok) return C_KZG_ERROR;
-  for (size_t i = 0; i < n1; i++)
-    if (st[i] != 0) { set_err("invalid G1 point in trusted setup"); return C_KZG_ERROR; }
-  for (size_t i = 0; i < n2; i++)
-    if (st[n1 + i] == 2) { set_err("invalid G2 point in trusted setup"); return C_KZG_ERROR; }
-
-  g1_t* g1 = (g1_t*)calloc(a1, sizeof(g1_t));
-  g2_t* g2 = (g2_t*)calloc(a2, sizeof(g2_t));
-  if (!g1 || !g2) { free(g1); free(g2); return C_KZG_MALLOC; }
-  for (size_t i = 0; i < n1; i++) {
-    canon_to_blst_fp(&g1[i].x, &c1[i * 24]);
-    canon_to_blst_fp(&g1[i].y, &c1[i * 24 + 12]);
-    g1[i].z.l[5] = 1;  // z = 1, most-significant-first limbs (srs.rs:131-153; also for infinity)
-  }
-  for (size_t i = n1; i < a1; i++) g1[i].z.l[5] = 1;
-  for (size_t i = 0; i < n2; i++) {
-    canon_to_blst_fp(&g2[i].x.fp[0], &c2[i * 48]);
-    canon_to_blst_fp(&g2[i].x.fp[1], &c2[i * 48 + 12]);
-    canon_to_blst_fp(&g2[i].y.fp[0], &c2[i * 48 + 24]);
-    canon_to_blst_fp(&g2[i].y.fp[1], &c2[i * 48 + 36]);
-    if (st[n1 + i] == 0) g2[i].z.fp[0].l[5] = 1;  // affine z = 1 + 0u ; infinity keeps z = 0
-  }
-  const int mode = (int)current_mode();
-  if (mode != 0 && n1 == N_POINTS) {
+// The second half of every loader: from the laid-out g1 / g2 values (ownership passes here; freed on failure) to a
+// device context in `out`.  to_lagrange: g1 holds the monomial points and the Lagrange modes convert them here.
+// mono_canon (may be NULL): the monomial points as canonical limbs (24 u32 each), kept on the device for FK20 and
+// cell verification in the Lagrange modes.  *out is written only on success.
+C_KZG_RET settings_from_points(KZGSettings* out, g1_t* g1, g2_t* g2, int mode, bool to_lagrange, const uint32_t* mono_canon) {
+  if (to_lagrange) {
     // c-kzg's load_trusted_setup stores the SRS in Lagrange form, bit-reversed
     // (the step the reference left as a TODO, lib.rs:760-770): L_i = sum_j (1/n) w_i^-j [tau^j]G,
     // computed as 4096 fixed-base MSMs over a temporary 8-bit table of the monomial points.
+    const auto t0 = std::chrono::steady_clock::now();
     Ctx* tmp = build_ctx(g1, g2, 0, 8);
     if (!tmp || !tmp->srs_valid) { if (tmp) destroy_ctx(tmp); free(g1); free(g2); set_err("Lagrange conversion failed"); return C_KZG_ERROR; }
     std::vector<uint32_t> lag((size_t)N_POINTS * 24);
@@ -1311,10 +1267,12 @@ C_KZG_RET settings_from_compressed(KZGSettings* out, const uint8_t* g1_bytes, si
       canon_to_blst_fp(&g1[i].x, &lag[i * 24]);
       canon_to_blst_fp(&g1[i].y, &lag[i * 24 + 12]);
     }
+    tl_load.convert_ms = ms_since(t0);
   }
+  const auto t1 = std::chrono::steady_clock::now();
   Ctx* c = build_ctx(g1, g2, mode);
   if (!c) { free(g1); free(g2); return C_KZG_ERROR; }
-  if (mode != 0 && n1 == N_POINTS && c->srs_valid) {
+  if (mono_canon && c->srs_valid) {
     // the Lagrange modes keep the monomial points too (c-kzg's g1_values_monomial): FK20 and cell verification need them
     bool good = [&]() -> bool {
       DeviceGuard dg(c->device);
@@ -1326,7 +1284,7 @@ C_KZG_RET settings_from_compressed(KZGSettings* out, const uint8_t* g1_bytes, si
       c->mono_owned = true;
       // on the kernel's own stream: a plain cudaMemcpy from pageable memory may return before the DMA has landed, and
       // a non-blocking stream does not wait for the legacy stream
-      CU_TRY(cudaMemcpyAsync(d_canon, c1.data(), (size_t)N_POINTS * 96, cudaMemcpyHostToDevice, c->slot[0].st));
+      CU_TRY(cudaMemcpyAsync(d_canon, mono_canon, (size_t)N_POINTS * 96, cudaMemcpyHostToDevice, c->slot[0].st));
       launch_srs_import(c->d_mono, d_canon, d_flags, d_flags + N_POINTS, N_POINTS, c->slot[0].st);
       std::vector<int> flags(N_POINTS);
       CU_TRY(cudaMemcpyAsync(flags.data(), d_flags, N_POINTS * sizeof(int), cudaMemcpyDeviceToHost, c->slot[0].st));
@@ -1340,10 +1298,92 @@ C_KZG_RET settings_from_compressed(KZGSettings* out, const uint8_t* g1_bytes, si
     }();
     if (!good) { destroy_ctx(c); free(g1); free(g2); return C_KZG_ERROR; }
   }
+  tl_load.build_ms = ms_since(t1);
   out->fs = reinterpret_cast<FFTSettings*>(c);
   out->g1_values = g1;
   out->g2_values = g2;
   return C_KZG_OK;
+}
+
+// Lay out KZGSettings.g1_values / g2_values from canonical limbs (24 / 48 u32 per point), as src/srs.rs:131-213 does:
+// u64 limbs most-significant first, z = 1 (g2: z = 0 where g2_inf[i]).  a1 / a2 >= n1 / n2 entries, zero-padded.
+bool layout_points(g1_t*& g1, g2_t*& g2, const uint32_t* c1, size_t n1, size_t a1, const uint32_t* c2, size_t n2, size_t a2, const int* g2_inf) {
+  g1 = (g1_t*)calloc(a1, sizeof(g1_t));
+  g2 = (g2_t*)calloc(a2, sizeof(g2_t));
+  if (!g1 || !g2) { free(g1); free(g2); g1 = nullptr; g2 = nullptr; return false; }
+  for (size_t i = 0; i < n1; i++) {
+    canon_to_blst_fp(&g1[i].x, &c1[i * 24]);
+    canon_to_blst_fp(&g1[i].y, &c1[i * 24 + 12]);
+  }
+  for (size_t i = 0; i < a1; i++) g1[i].z.l[5] = 1;  // also for infinity and the padding (srs.rs:131-153)
+  for (size_t i = 0; i < n2; i++) {
+    canon_to_blst_fp(&g2[i].x.fp[0], &c2[i * 48]);
+    canon_to_blst_fp(&g2[i].x.fp[1], &c2[i * 48 + 12]);
+    canon_to_blst_fp(&g2[i].y.fp[0], &c2[i * 48 + 24]);
+    canon_to_blst_fp(&g2[i].y.fp[1], &c2[i * 48 + 36]);
+    if (!(g2_inf && g2_inf[i])) g2[i].z.fp[0].l[5] = 1;  // affine z = 1 + 0u ; infinity keeps z = 0
+  }
+  return true;
+}
+
+// Decode + validate compressed points on the device, then lay out KZGSettings
+// exactly as src/srs.rs:99-153 / src/lib.rs:724-758 do.  n1 / n2 may be
+// smaller than 4096 / 65 for the file loader (tests/trusted_setup_4.txt): the
+// arrays are always allocated full size and zero-padded so later calls stay
+// memory safe (they then fail SRS re-hydration -> C_KZG_ERROR).
+C_KZG_RET settings_from_compressed(KZGSettings* out, const uint8_t* g1_bytes, size_t n1, const uint8_t* g2_bytes, size_t n2) {
+  tl_load = {0, 0, 0, 0};
+  size_t a1 = std::max<size_t>(n1, N_POINTS), a2 = std::max<size_t>(n2, TRUSTED_SETUP_NUM_G2_POINTS);
+  void *d_in1 = nullptr, *d_in2 = nullptr, *d_c1 = nullptr, *d_c2 = nullptr;
+  int* d_st = nullptr;
+  std::vector<uint32_t> c1(n1 * 24), c2(n2 * 48);
+  std::vector<int> st(n1 + n2);
+  cudaEvent_t ev[2] = {nullptr, nullptr};
+  auto cleanup = [&]() {
+    cudaFree(d_in1); cudaFree(d_in2); cudaFree(d_c1); cudaFree(d_c2); cudaFree(d_st);
+    for (cudaEvent_t e : ev)
+      if (e) cudaEventDestroy(e);
+  };
+  auto run = [&]() -> bool {
+    CU_TRY(cudaMalloc(&d_in1, std::max<size_t>(n1, 1) * 48));
+    CU_TRY(cudaMalloc(&d_in2, std::max<size_t>(n2, 1) * 96));
+    CU_TRY(cudaMalloc(&d_c1, std::max<size_t>(n1, 1) * 96));
+    CU_TRY(cudaMalloc(&d_c2, std::max<size_t>(n2, 1) * 192));
+    CU_TRY(cudaMalloc(&d_st, (n1 + n2 + 1) * sizeof(int)));
+    CU_TRY(cudaEventCreate(&ev[0]));
+    CU_TRY(cudaEventCreate(&ev[1]));
+    CU_TRY(cudaEventRecord(ev[0], 0));
+    if (n1) CU_TRY(cudaMemcpy(d_in1, g1_bytes, n1 * 48, cudaMemcpyHostToDevice));
+    if (n2) CU_TRY(cudaMemcpy(d_in2, g2_bytes, n2 * 96, cudaMemcpyHostToDevice));
+    launch_setup_decode_g1(d_c1, d_st, d_in1, (int)n1, 0);
+    launch_setup_decode_g2(d_c2, d_st + n1, d_in2, (int)n2, 0);
+    CU_TRY(cudaEventRecord(ev[1], 0));
+    CU_TRY(cudaDeviceSynchronize());
+    CU_TRY(cudaGetLastError());
+    float ms = 0;
+    CU_TRY(cudaEventElapsedTime(&ms, ev[0], ev[1]));
+    tl_load.decode_ms = ms;
+    if (n1) CU_TRY(cudaMemcpy(c1.data(), d_c1, n1 * 96, cudaMemcpyDeviceToHost));
+    if (n2) CU_TRY(cudaMemcpy(c2.data(), d_c2, n2 * 192, cudaMemcpyDeviceToHost));
+    CU_TRY(cudaMemcpy(st.data(), d_st, (n1 + n2) * sizeof(int), cudaMemcpyDeviceToHost));
+    return true;
+  };
+  bool ok = run();
+  cleanup();
+  if (!ok) return C_KZG_ERROR;
+  for (size_t i = 0; i < n1; i++)
+    if (st[i] != 0) { set_err("invalid G1 point in trusted setup"); return C_KZG_ERROR; }
+  std::vector<int> g2_inf(n2);
+  for (size_t i = 0; i < n2; i++) {
+    if (st[n1 + i] == 2) { set_err("invalid G2 point in trusted setup"); return C_KZG_ERROR; }
+    g2_inf[i] = st[n1 + i] == 1;
+  }
+  g1_t* g1;
+  g2_t* g2;
+  if (!layout_points(g1, g2, c1.data(), n1, a1, c2.data(), n2, a2, g2_inf.data())) return C_KZG_MALLOC;
+  const int mode = (int)current_mode();
+  const bool full = mode != 0 && n1 == N_POINTS;
+  return settings_from_points(out, g1, g2, mode, full, full ? c1.data() : nullptr);
 }
 
 // ------------------------------------------------------------------ verification
@@ -2135,6 +2175,269 @@ C_KZG_RET load_trusted_setup_file(KZGSettings* out, FILE* in) {
   for (size_t i = 0; i < m2; i++)
     if (!hex_line(lines[2 + m1 + i], &g2b[i * 96], 96)) { set_err("bad G2 hex line"); return C_KZG_ERROR; }
   return settings_from_compressed(out, g1b.data(), m1, g2b.data(), m2);
+}
+
+// ------------------------------------------------------------------ c-kzg-4844 trusted setups
+// The layout of c-kzg-4844 v2's trusted_setup.txt (the Ethereum ceremony output): 4096 G1 points in Lagrange form
+// (natural order: L_k = [l_k(tau)]G over w^k), 65 G2 monomial points [tau^i]H, 4096 G1 monomial points [tau^j]G.
+constexpr size_t CKZG_G1_BYTES = (size_t)N_POINTS * 48;
+constexpr size_t CKZG_G2_BYTES = (size_t)TRUSTED_SETUP_NUM_G2_POINTS * 96;
+constexpr size_t CKZG_MAX_PRECOMPUTE = 15;
+// the compressed G1 generator: a setup's first monomial point must be it
+constexpr uint8_t G1_GENERATOR_COMPRESSED[48] = {
+    0x97, 0xf1, 0xd3, 0xa7, 0x31, 0x97, 0xd7, 0x94, 0x26, 0x95, 0x63, 0x8c, 0x4f, 0xa9, 0xac, 0x0f, 0xc3, 0x68, 0x8c, 0x4f, 0x97, 0x74, 0xb9, 0x05,
+    0xa1, 0x4e, 0x3a, 0x3f, 0x17, 0x1b, 0xac, 0x58, 0x6c, 0x55, 0xe8, 0x3f, 0xf9, 0x7a, 0x1a, 0xef, 0xfb, 0x3a, 0xf0, 0x0a, 0xdb, 0x22, 0xc6, 0xbb};
+
+// c-kzg's scanf-based reader: whitespace-separated tokens -- the decimal counts 4096 and 65, then the points' bytes as
+// hex pairs (whitespace may separate pairs, never the two digits of one).  Anything after the last point is ignored.
+// A rule of its own, not the reference's line format (parse_usize / hex_line above).
+struct CkzgText {
+  const std::string& s;
+  size_t pos = 0;
+  static bool space(char ch) { return ch == ' ' || ch == '\n' || ch == '\r' || ch == '\t' || ch == '\v' || ch == '\f'; }
+  void skip() { while (pos < s.size() && space(s[pos])) pos++; }
+  bool count(size_t& v) {
+    skip();
+    const size_t p0 = pos;
+    v = 0;
+    while (pos < s.size() && s[pos] >= '0' && s[pos] <= '9' && pos - p0 < 12) v = v * 10 + (size_t)(s[pos++] - '0');
+    return pos > p0 && (pos == s.size() || space(s[pos]));
+  }
+  // 0 ok, 1 end of input, 2 not a hex pair
+  int bytes(uint8_t* out, size_t n) {
+    for (size_t i = 0; i < n; i++) {
+      skip();
+      if (pos >= s.size()) return 1;
+      if (pos + 1 >= s.size()) return hex_nibble(s[pos], out[i]) ? 1 : 2;
+      uint8_t a, b;
+      if (!hex_nibble(s[pos], a) || !hex_nibble(s[pos + 1], b)) return 2;
+      out[i] = (uint8_t)(a << 4 | b);
+      pos += 2;
+    }
+    return 0;
+  }
+};
+
+bool parse_ckzg_setup(const std::string& text, std::vector<uint8_t>& lag, std::vector<uint8_t>& g2, std::vector<uint8_t>& mono) {
+  CkzgText t{text};
+  size_t n1 = 0, n2 = 0;
+  if (!t.count(n1) || !t.count(n2)) { set_err("c-kzg trusted setup: the header is not two decimal counts"); return false; }
+  if (n1 != N_POINTS || n2 != TRUSTED_SETUP_NUM_G2_POINTS) {
+    set_err("c-kzg trusted setup: header " + std::to_string(n1) + " / " + std::to_string(n2) + ", expected 4096 / 65");
+    return false;
+  }
+  lag.assign(CKZG_G1_BYTES, 0);
+  g2.assign(CKZG_G2_BYTES, 0);
+  mono.assign(CKZG_G1_BYTES, 0);
+  struct Sec { const char* name; uint8_t* p; size_t n, each; } secs[3] = {
+      {"Lagrange G1", lag.data(), (size_t)N_POINTS, 48}, {"G2", g2.data(), (size_t)TRUSTED_SETUP_NUM_G2_POINTS, 96}, {"monomial G1", mono.data(), (size_t)N_POINTS, 48}};
+  for (const Sec& sec : secs)
+    for (size_t i = 0; i < sec.n; i++) {
+      const int r = t.bytes(sec.p + i * sec.each, sec.each);
+      if (r == 0) continue;
+      set_err(std::string("c-kzg trusted setup: ") + sec.name + " point " + std::to_string(i) + (r == 1 ? ": file truncated" : ": not hex byte pairs"));
+      return false;
+    }
+  return true;
+}
+
+// The setup check (DESIGN 2): M_0 = G; sum_k rho^k L_k = sum_j f_j M_j with f(w^k) = rho^k (Lagrange against monomial);
+// e(sum_i rho^i M_(i+1), Q_0) = e(sum_i rho^i M_i, Q_1) (the G1 points are one powers-of-tau chain); e(M_1, Q_i) =
+// e(M_0, Q_(i+1)) for i < 64 (so are the G2 points).  rho = SHA-256(domain || the three sections) mod r: the weights are
+// fixed by the file's contents, so no file can pick them.  Decoding is strict (blst's rules, G2 subgroup included).
+// Writes c_lag / c_mono / c_g2 (canonical limbs) for the layout; false with the reason in tl_err (BADARGS) or on a
+// device failure (err_code = C_KZG_ERROR).
+bool ckzg_decode_and_check(const uint8_t* mono, const uint8_t* lag, const uint8_t* g2b, std::vector<uint32_t>& c_g1, std::vector<uint32_t>& c_g2,
+                           C_KZG_RET& err_code) {
+  static const char DOMAIN_TAG[] = "LWKZG_CKZG_SETUP_CHECK_______V1_";
+  constexpr size_t DOMAIN = sizeof(DOMAIN_TAG) - 1;   // 32 bytes, no terminator
+  const int NG2 = TRUSTED_SETUP_NUM_G2_POINTS;
+  err_code = C_KZG_ERROR;
+  ScratchMem sm;
+  cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
+  struct EvFree { cudaEvent_t* e; ~EvFree() { for (int i = 0; i < 3; i++) if (e[i]) cudaEventDestroy(e[i]); } } ev_free{ev};
+  for (auto& e : ev) CU_TRY(cudaEventCreate(&e));
+  const cudaStream_t st = 0;
+  // ---- decode: [L; M] as one array of 8192 G1 points (the point vector of the Lagrange-against-monomial MSM)
+  uint8_t* d_in = (uint8_t*)sm.get(2 * CKZG_G1_BYTES + CKZG_G2_BYTES);
+  uint8_t* d_aff = (uint8_t*)sm.get((size_t)2 * N_POINTS * AFFINE_BYTES);
+  uint32_t* d_c1 = (uint32_t*)sm.get((size_t)2 * N_POINTS * 96);
+  uint32_t* d_c2 = (uint32_t*)sm.get((size_t)NG2 * 192);
+  int* d_st = (int*)sm.get((size_t)(2 * N_POINTS + NG2) * sizeof(int));
+  if (!d_in || !d_aff || !d_c1 || !d_c2 || !d_st) return false;
+  CU_TRY(cudaEventRecord(ev[0], st));
+  CU_TRY(cudaMemcpyAsync(d_in, lag, CKZG_G1_BYTES, cudaMemcpyHostToDevice, st));
+  CU_TRY(cudaMemcpyAsync(d_in + CKZG_G1_BYTES, mono, CKZG_G1_BYTES, cudaMemcpyHostToDevice, st));
+  CU_TRY(cudaMemcpyAsync(d_in + 2 * CKZG_G1_BYTES, g2b, CKZG_G2_BYTES, cudaMemcpyHostToDevice, st));
+  launch_g1_decompress(d_aff, nullptr, d_st, d_in, 2 * N_POINTS, st, true, true);
+  launch_affine_to_canon(d_c1, d_aff, 2 * N_POINTS, st);
+  launch_setup_decode_g2_strict(d_c2, d_st + 2 * N_POINTS, d_in + 2 * CKZG_G1_BYTES, NG2, st);
+  CU_TRY(cudaEventRecord(ev[1], st));
+  c_g1.resize((size_t)2 * N_POINTS * 24);
+  c_g2.resize((size_t)NG2 * 48);
+  std::vector<int> status(2 * N_POINTS + NG2);
+  CU_TRY(cudaMemcpy(c_g1.data(), d_c1, c_g1.size() * 4, cudaMemcpyDeviceToHost));
+  CU_TRY(cudaMemcpy(c_g2.data(), d_c2, c_g2.size() * 4, cudaMemcpyDeviceToHost));
+  CU_TRY(cudaMemcpy(status.data(), d_st, status.size() * sizeof(int), cudaMemcpyDeviceToHost));
+  CU_TRY(cudaGetLastError());
+  float ms = 0;
+  CU_TRY(cudaEventElapsedTime(&ms, ev[0], ev[1]));
+  tl_load.decode_ms = ms;
+  err_code = C_KZG_BADARGS;
+  for (int i = 0; i < 2 * N_POINTS; i++) {
+    const char* sec = i < N_POINTS ? "Lagrange G1" : "monomial G1";
+    const std::string where = std::string("c-kzg trusted setup: ") + sec + " point " + std::to_string(i % N_POINTS);
+    if (status[i]) { set_err(where + " is not a valid compressed G1 point (encoding, curve or subgroup)"); return false; }
+    bool inf = true;
+    for (int k = 0; k < 24; k++) inf = inf && c_g1[(size_t)i * 24 + k] == 0;
+    if (inf) { set_err(where + " is the point at infinity"); return false; }
+  }
+  static const char* G2_WHY[4] = {"", "is not a canonical compressed G2 point (flags, infinity or x >= p)", "is not on the curve", "is not in G2"};
+  for (int i = 0; i < NG2; i++) {
+    const int code = status[2 * N_POINTS + i];
+    if (code) { set_err("c-kzg trusted setup: G2 point " + std::to_string(i) + " " + G2_WHY[code & 3]); return false; }
+  }
+  // ---- check 1 (host): strict decoding makes the encoding unique, so M_0 = G iff its bytes are G's
+  if (memcmp(mono, G1_GENERATOR_COMPRESSED, 48) != 0) { set_err("c-kzg trusted setup: monomial G1 point 0 is not the generator"); return false; }
+  err_code = C_KZG_ERROR;
+
+  // ---- checks 2-4 on the device
+  const size_t msg_len = DOMAIN + 2 * CKZG_G1_BYTES + CKZG_G2_BYTES;
+  const size_t nblocks = (msg_len + 9 + 63) / 64;
+  std::vector<uint8_t> msg(nblocks * 64, 0);   // domain || Lagrange || G2 || monomial (file order), SHA-256 padding
+  memcpy(msg.data(), DOMAIN_TAG, DOMAIN);
+  memcpy(msg.data() + DOMAIN, lag, CKZG_G1_BYTES);
+  memcpy(msg.data() + DOMAIN + CKZG_G1_BYTES, g2b, CKZG_G2_BYTES);
+  memcpy(msg.data() + DOMAIN + CKZG_G1_BYTES + CKZG_G2_BYTES, mono, CKZG_G1_BYTES);
+  msg[msg_len] = 0x80;
+  for (int i = 0; i < 8; i++) msg[msg.size() - 1 - i] = (uint8_t)(((uint64_t)msg_len * 8) >> (8 * i));
+  // 64 G2-chain partials (M_0 at 0, infinity at 96, M_1 at 192: e(M_1, Q_i) = e(M_0, Q_(i+1)) in batch_final's terms)
+  std::vector<uint8_t> chain((size_t)(NG2 - 1) * 288, 0);
+  auto be48 = [](uint8_t* o, const uint32_t* le12) {
+    for (int i = 0; i < 12; i++)
+      for (int b = 0; b < 4; b++) o[44 - 4 * i + b] = (uint8_t)(le12[i] >> (24 - 8 * b));
+  };
+  const uint32_t* m0 = &c_g1[(size_t)N_POINTS * 24];
+  const uint32_t* m1 = &c_g1[(size_t)(N_POINTS + 1) * 24];
+  for (int i = 0; i < NG2 - 1; i++) {
+    uint8_t* p = &chain[(size_t)i * 288];
+    be48(p, m0); be48(p + 48, m0 + 12);
+    be48(p + 192, m1); be48(p + 240, m1 + 12);
+  }
+  uint8_t* d_msg = (uint8_t*)sm.get(msg.size());
+  uint32_t* d_rho = (uint32_t*)sm.get(32);
+  uint8_t* d_sc = (uint8_t*)sm.get((size_t)2 * N_POINTS * 32);
+  void* d_blob = sm.get(BLOB_BYTES);
+  void* d_tw = sm.get((size_t)EXT_POINTS * 32);
+  void* d_coef = sm.get((size_t)N_POINTS * 32);
+  void* d_scratch = sm.get(var_msm_scratch_bytes(2 * N_POINTS));
+  uint8_t* d_out = (uint8_t*)sm.get(96 + 288 + chain.size());   // MSM | G1-chain partial | G2-chain partials
+  void* d_prep = sm.get((size_t)NG2 * g2_prepared_bytes());
+  int* d_flags = (int*)sm.get((size_t)(NG2 + NG2) * sizeof(int));   // G2 preparation flags | verdicts
+  if (!d_msg || !d_rho || !d_sc || !d_blob || !d_tw || !d_coef || !d_scratch || !d_out || !d_prep || !d_flags) return false;
+  CU_TRY(cudaMemcpyAsync(d_msg, msg.data(), msg.size(), cudaMemcpyHostToDevice, st));
+  CU_TRY(cudaMemcpyAsync(d_out + 96 + 288, chain.data(), chain.size(), cudaMemcpyHostToDevice, st));
+  CU_TRY(cudaMemsetAsync(d_out, 0, 96 + 288, st));
+  CU_TRY(cudaEventRecord(ev[1], st));
+  launch_setup_rho(d_rho, d_msg, (int)nblocks, st);
+  launch_setup_rho_powers(d_sc, d_blob, d_rho, st);
+  // f: the inverse DFT of the values rho^k, through the cell kernels' 4096-point transform (a MODE_DENEB blob in, its
+  // coefficients out)
+  launch_cell_twiddles(d_tw, st);
+  launch_cell_poly(d_coef, nullptr, d_blob, 1, 2, d_tw, st);
+  launch_setup_neg_coef(d_sc + (size_t)N_POINTS * 32, d_coef, st);
+  // check 2: sum_k rho^k L_k - sum_j f_j M_j, one MSM over [L; M], must be infinity
+  launch_var_msm_mont(d_out, d_aff, d_sc, 2 * N_POINTS, d_scratch, st);
+  // check 3: the G1 chain, against Q_0 and Q_1
+  uint8_t* part = d_out + 96;
+  launch_var_msm_mont(part + 192, d_aff + (size_t)(N_POINTS + 1) * AFFINE_BYTES, d_sc, N_POINTS - 1, d_scratch, st);
+  launch_var_msm_mont(part, d_aff + (size_t)N_POINTS * AFFINE_BYTES, d_sc, N_POINTS - 1, d_scratch, st);
+  launch_g2_prepare(d_prep, d_flags, d_c2, st, NG2);
+  launch_batch_final(d_flags + NG2, part, 1, d_prep, (const uint8_t*)d_prep + g2_prepared_bytes(), st);
+  // check 4: the G2 chain, 64 pairing checks in one launch
+  launch_batch_final_chain(d_flags + NG2 + 1, part + 288, NG2 - 1, d_prep, st);
+  CU_TRY(cudaEventRecord(ev[2], st));
+  uint8_t lhs[96];
+  std::vector<int> flags(2 * NG2);
+  CU_TRY(cudaMemcpyAsync(lhs, d_out, 96, cudaMemcpyDeviceToHost, st));
+  CU_TRY(cudaMemcpyAsync(flags.data(), d_flags, flags.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
+  CU_TRY(cudaStreamSynchronize(st));
+  CU_TRY(cudaGetLastError());
+  CU_TRY(cudaEventElapsedTime(&ms, ev[1], ev[2]));
+  tl_load.check_ms = ms;
+  err_code = C_KZG_BADARGS;
+  for (int i = 0; i < NG2; i++)
+    if (flags[i]) { set_err("c-kzg trusted setup: G2 point " + std::to_string(i) + " is not on the curve"); return false; }
+  for (uint8_t b : lhs)
+    if (b) { set_err("c-kzg trusted setup: the Lagrange G1 section is not the Lagrange form (natural order) of the monomial G1 section"); return false; }
+  if (!flags[NG2]) { set_err("c-kzg trusted setup: the monomial G1 points are not one powers-of-tau chain over G2 points 0 and 1"); return false; }
+  for (int i = 0; i < NG2 - 1; i++)
+    if (!flags[NG2 + 1 + i]) {
+      set_err("c-kzg trusted setup: G2 point " + std::to_string(i + 1) + " does not continue the powers of tau (e(M_1, Q_" + std::to_string(i) +
+              ") != e(M_0, Q_" + std::to_string(i + 1) + "))");
+      return false;
+    }
+  return true;
+}
+
+// Both c-kzg loaders, after their argument checks.  Mode 0: the monomial section is the SRS; modes 1 and 2: the
+// Lagrange section, bit-reversed, plus the monomial section for FK20 and cell verification -- the settings a
+// monomial setup of the same tau gives through load_trusted_setup, without its conversion.
+C_KZG_RET settings_from_ckzg(KZGSettings* out, const uint8_t* mono, const uint8_t* lag, const uint8_t* g2b) {
+  tl_load = {0, 0, 0, 0};
+  const int mode = (int)current_mode();
+  std::vector<uint32_t> c_g1, c_g2;
+  C_KZG_RET code = C_KZG_ERROR;
+  if (!ckzg_decode_and_check(mono, lag, g2b, c_g1, c_g2, code)) return code;
+  const uint32_t* c_lag = c_g1.data();
+  const uint32_t* c_mono = c_g1.data() + (size_t)N_POINTS * 24;
+  std::vector<uint32_t> srs;
+  if (mode != 0) {
+    srs.resize((size_t)N_POINTS * 24);
+    for (uint32_t i = 0; i < (uint32_t)N_POINTS; i++) {
+      uint32_t k = 0;
+      for (int b = 0; b < 12; b++) k |= ((i >> b) & 1u) << (11 - b);
+      memcpy(&srs[(size_t)i * 24], &c_lag[(size_t)k * 24], 24 * sizeof(uint32_t));
+    }
+  }
+  g1_t* g1;
+  g2_t* g2;
+  if (!layout_points(g1, g2, mode != 0 ? srs.data() : c_mono, N_POINTS, N_POINTS, c_g2.data(), TRUSTED_SETUP_NUM_G2_POINTS,
+                     TRUSTED_SETUP_NUM_G2_POINTS, nullptr))
+    return C_KZG_MALLOC;
+  return settings_from_points(out, g1, g2, mode, false, mode != 0 ? c_mono : nullptr);
+}
+
+C_KZG_RET lwkzg_load_trusted_setup_ckzg(KZGSettings* out, const uint8_t* g1_monomial_bytes, uint64_t num_g1_monomial_bytes,
+                                        const uint8_t* g1_lagrange_bytes, uint64_t num_g1_lagrange_bytes, const uint8_t* g2_monomial_bytes,
+                                        uint64_t num_g2_monomial_bytes, uint64_t precompute) {
+  if (!out || !g1_monomial_bytes || !g1_lagrange_bytes || !g2_monomial_bytes) { set_err("null argument"); return C_KZG_BADARGS; }
+  if (num_g1_monomial_bytes != CKZG_G1_BYTES || num_g1_lagrange_bytes != CKZG_G1_BYTES || num_g2_monomial_bytes != CKZG_G2_BYTES) {
+    set_err("c-kzg trusted setup: the sections must be 4096 x 48, 4096 x 48 and 65 x 96 bytes");
+    return C_KZG_BADARGS;
+  }
+  if (precompute > CKZG_MAX_PRECOMPUTE) { set_err("c-kzg trusted setup: precompute must be 0..15"); return C_KZG_BADARGS; }
+  return settings_from_ckzg(out, g1_monomial_bytes, g1_lagrange_bytes, g2_monomial_bytes);
+}
+
+C_KZG_RET lwkzg_load_trusted_setup_file_ckzg(KZGSettings* out, FILE* in, uint64_t precompute) {
+  if (!out || !in) { set_err("null argument"); return C_KZG_BADARGS; }
+  if (precompute > CKZG_MAX_PRECOMPUTE) { set_err("c-kzg trusted setup: precompute must be 0..15"); return C_KZG_BADARGS; }
+  std::string contents;
+  char buf[65536];
+  size_t got;
+  while ((got = fread(buf, 1, sizeof(buf), in)) > 0) contents.append(buf, got);
+  std::vector<uint8_t> lag, g2, mono;
+  if (!parse_ckzg_setup(contents, lag, g2, mono)) return C_KZG_BADARGS;
+  return settings_from_ckzg(out, mono.data(), lag.data(), g2.data());
+}
+
+int lwkzg_last_load_times(double* decode_ms, double* check_ms, double* convert_ms, double* build_ms) {
+  if (decode_ms) *decode_ms = tl_load.decode_ms;
+  if (check_ms) *check_ms = tl_load.check_ms;
+  if (convert_ms) *convert_ms = tl_load.convert_ms;
+  if (build_ms) *build_ms = tl_load.build_ms;
+  return 0;
 }
 
 C_KZG_RET free_trusted_setup(KZGSettings* s) {

@@ -25,9 +25,12 @@ size_t g2_prepared_bytes() { return sizeof(G2Prepared); }
 
 // canonical x.c0,x.c1,y.c0,y.c1 -> prepared lines.  bad = 1 if the point is not
 // on the twist (blst_p2_to_g2_point's from_affine, src/srs.rs:215-247; the
-// all-zero encoding of infinity fails that check too).
+// all-zero encoding of infinity fails that check too).  One point per block.
 __global__ void g2_prepare_kernel(G2Prepared* __restrict__ out, int* __restrict__ bad, const uint32_t* __restrict__ canon48) {
-  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  if (threadIdx.x != 0) return;
+  out += blockIdx.x;
+  bad += blockIdx.x;
+  canon48 += (size_t)blockIdx.x * 48;
   Fp c[4];
   for (int j = 0; j < 4; j++) {
     for (int k = 0; k < 12; k++) c[j].l[k] = canon48[j * 12 + k];
@@ -271,13 +274,16 @@ __device__ __forceinline__ G1Affine affine_from_be96(const uint8_t* b) {
 
 // partials: n_ranks x (proof_lincomb, proof_z_lincomb, c_minus_y_lincomb), canonical BE affine.
 // ok = [ e(c_minus_y + proof_z, g2_0) == e(proof_lincomb, g2_1) ]   (lib.rs:679-691)
+// Block b checks the partials at b * n_ranks * 288 against prep0 + b * prep_stride, prep1 + b * prep_stride.
 __global__ void __launch_bounds__(LW_PAIR_LANES) batch_final_kernel(int* __restrict__ ok_out, const uint8_t* __restrict__ partials, int n_ranks,
-                                                          const G2Prepared* __restrict__ prep0, const G2Prepared* __restrict__ prep1) {
+                                                          const G2Prepared* __restrict__ prep0, const G2Prepared* __restrict__ prep1, int prep_stride) {
   __shared__ WarpPairingMem sh_m;
   __shared__ G1Affine sh_pts[2];
   const int lane = threadIdx.x;
   partials += (size_t)blockIdx.x * n_ranks * 288;   // one check per block (launch_batch_final_each)
   ok_out += blockIdx.x;
+  prep0 += (size_t)blockIdx.x * prep_stride;
+  prep1 += (size_t)blockIdx.x * prep_stride;
   if (lane < 2) {
     G1Xyzz acc = xyzz_inf();
     for (int r = 0; r < n_ranks; r++) {
@@ -298,8 +304,9 @@ __global__ void __launch_bounds__(LW_PAIR_LANES) batch_final_kernel(int* __restr
 }
 
 // ------------------------------------------------------------------ launchers
-void launch_g2_prepare(void* d_prepared, int* d_bad, const void* d_canon_in, cudaStream_t st) {
-  g2_prepare_kernel<<<1, 32, 0, st>>>((G2Prepared*)d_prepared, d_bad, (const uint32_t*)d_canon_in);
+void launch_g2_prepare(void* d_prepared, int* d_bad, const void* d_canon_in, cudaStream_t st, int n) {
+  if (n <= 0) return;
+  g2_prepare_kernel<<<n, 32, 0, st>>>((G2Prepared*)d_prepared, d_bad, (const uint32_t*)d_canon_in);
   count_launch();
 }
 void launch_g2_check(int* d_bad, const void* d_canon_in, int n, cudaStream_t st) {
@@ -382,12 +389,18 @@ void launch_batch_partials(void* d_partial288, const void* d_r, const void* d_c_
   cudaStreamWaitEvent(st, ev_join, 0);
 }
 void launch_batch_final(int* d_ok, const void* d_partials288, int n_ranks, const void* d_prep0, const void* d_prep1, cudaStream_t st) {
-  batch_final_kernel<<<1, LW_PAIR_LANES, 0, st>>>(d_ok, (const uint8_t*)d_partials288, n_ranks, (const G2Prepared*)d_prep0, (const G2Prepared*)d_prep1);
+  batch_final_kernel<<<1, LW_PAIR_LANES, 0, st>>>(d_ok, (const uint8_t*)d_partials288, n_ranks, (const G2Prepared*)d_prep0, (const G2Prepared*)d_prep1, 0);
   count_launch();
 }
 void launch_batch_final_each(int* d_ok, const void* d_partials288, int n_checks, const void* d_prep0, const void* d_prep1, cudaStream_t st) {
   if (n_checks <= 0) return;
-  batch_final_kernel<<<n_checks, LW_PAIR_LANES, 0, st>>>(d_ok, (const uint8_t*)d_partials288, 1, (const G2Prepared*)d_prep0, (const G2Prepared*)d_prep1);
+  batch_final_kernel<<<n_checks, LW_PAIR_LANES, 0, st>>>(d_ok, (const uint8_t*)d_partials288, 1, (const G2Prepared*)d_prep0, (const G2Prepared*)d_prep1, 0);
+  count_launch();
+}
+void launch_batch_final_chain(int* d_ok, const void* d_partials288, int n_checks, const void* d_preps, cudaStream_t st) {
+  if (n_checks <= 0) return;
+  const G2Prepared* p = (const G2Prepared*)d_preps;
+  batch_final_kernel<<<n_checks, LW_PAIR_LANES, 0, st>>>(d_ok, (const uint8_t*)d_partials288, 1, p, p + 1, 1);
   count_launch();
 }
 }  // namespace lw
